@@ -18,6 +18,13 @@ One JSON line is printed by rank 0 (see the driver contract in the task statemen
   roofline  algorithmic bytes of the dominant kernel family / its event-timed duration vs the measured HBM peak
   cpu_baseline / --impl reference   the UNMODIFIED reference (baseline/_ref, tools/install_reference.sh)
             timed on this host's cores on a bounded sample; the oracle port only if it cannot be imported
+
+--dump-outputs DIR writes what the last timed step left in its result buffer, so that two builds can be
+compared output for output on the same (seeded) inputs: DIR/<output>.npy (channels, scales, K) at K sample
+columns -- the first and last 64 (K // 2 each when fewer than 128 columns fit) and a seeded random draw of
+the others, as many as keep the dump under 64 MB -- (complex results as (..., 2) real / imaginary pairs),
+DIR/columns.npy (the K sample indices of this rank's samples) and DIR/frequencies.npy (Hz).  Tiled workloads dump the last tile a step produced.
+With several ranks every rank writes its own files, suffixed _rank<r>.
 """
 from __future__ import annotations
 
@@ -79,7 +86,13 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="N > 1: skip the strong-scaling / config 3 / config 4 entries")
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.dtype == "f64" and args.workload == "cfg2":
         args.workload = "cfg5"
     return args
@@ -332,6 +345,32 @@ class Timer:
         return ms / steps
 
 
+DUMP_BYTES = 48 << 20          # all files of one --dump-outputs call together stay under 64 MB
+DUMP_EDGE = 64                 # columns kept at either end: they see the zero padding of the convolution
+
+
+def dump_outputs(dirname, res, first, output, freqs, rank, world):
+    """--dump-outputs: K sample columns of ``res`` (channels, scales, columns), a CUDA tensor that holds
+    this rank's samples first, first + 1, ...; the columns are the same from run to run."""
+    import torch
+    nch, S, ncols = res.shape
+    parts = 2 if res.is_complex() else 1
+    item = res.element_size() // parts
+    k = max(1, min(ncols, (DUMP_BYTES // world - 8 * S) // (nch * S * parts * item + 8)))
+    e = min(DUMP_EDGE, k // 2)                            # the edge columns are reserved first, within the k
+    edge = np.r_[0:min(e, ncols), max(0, ncols - e):ncols]
+    draw = np.random.default_rng(0).integers(0, ncols, size=k - edge.size)
+    cols = np.unique(np.concatenate([edge, draw]))
+    vals = res.index_select(2, torch.from_numpy(cols).to(res.device))
+    if vals.is_complex():
+        vals = torch.view_as_real(vals)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, ("coefficients" if output == "complex" else output) + suffix + ".npy"), vals.cpu().numpy())
+    np.save(os.path.join(dirname, "columns" + suffix + ".npy"), (cols + first).astype(np.float64))
+    np.save(os.path.join(dirname, "frequencies" + suffix + ".npy"), np.asarray(freqs, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -363,13 +402,17 @@ def run_ours(args):
     tile = int(args.tile if args.tile else wl.get("tile", 0))
     out = plan.alloc_out(nch, tile if tile else n)
     torch.cuda.synchronize(dev)
+    last_tile = [0, n]                 # samples [a, b) that out[:, :, :b - a] holds after a step
+
+    def keep_range(o, a, b):
+        last_tile[:] = (a, b)
 
     def one_pass():
         if wl.get("time_shard"):
             from ghost_b200 import sharding
-            sharding.run_time_shard_tiled(plan, x_dev, rank, world, tile, out=out)
+            sharding.run_time_shard_tiled(plan, x_dev, rank, world, tile, out=out, consumer=keep_range)
         elif tile:
-            plan.execute_tiled(x_dev, tile, out=out)             # the mean kernel runs inside the step
+            plan.execute_tiled(x_dev, tile, out=out, consumer=keep_range)   # the mean kernel runs inside the step
         else:
             plan.execute(x_dev, out)
 
@@ -386,6 +429,9 @@ def run_ours(args):
     sampler.stop_flag = True
     launches = _lib.launch_count()
     gstats = plan.guard_stats()
+    if args.dump_outputs:
+        a, b = last_tile
+        dump_outputs(args.dump_outputs, out[:, :, :b - a], a, wl["output"], freqs, rank, world)
     # the same K steps again with the library's per-family event spans (they serialise the class launches):
     # what the roofline of each kernel family is computed from
     plan.profile(True)

@@ -37,6 +37,15 @@ def load_reference(path="/root/reference"):
     return ContinuousWaveletTransform, Morse, morseutils, sigtools
 
 
+def sample_columns(n, k, edge, seed=0):
+    """Sorted indices of the columns stored of a length-n output axis (it keeps every golden file under
+    1 MB): all of them when n <= k, else the first and last ``edge`` and a seeded draw of the others, k in all."""
+    if n <= k:
+        return np.arange(n)
+    inner = np.random.default_rng(seed).choice(np.arange(edge, n - edge), size=k - 2 * edge, replace=False)
+    return np.concatenate([np.arange(edge), np.sort(inner), np.arange(n - edge, n)])
+
+
 def ref_complex(CWT, Morse, sigtools, x, fs, gamma, beta, freqs_hz):
     """The reference's own wavelet_conv body (transforms.py:187-204) minus abs."""
     cwt = CWT(wavelet=Morse(gamma=gamma, beta=beta))
@@ -123,9 +132,11 @@ def main():
                                 (70000, 513), (64, 1)]):
         s = rng.standard_normal(n)
         k = rng.standard_normal(m) + 1j * rng.standard_normal(m)
+        cols = sample_columns(n, 6000, 512)
         conv[f"s_{i}"] = s
         conv[f"k_{i}"] = k
-        conv[f"y_{i}"] = sigtools.fastconv_scipy(s, k)
+        conv[f"y_{i}"] = sigtools.fastconv_scipy(s, k)[cols]
+        conv[f"cols_{i}"] = cols
     np.savez_compressed(os.path.join(GOLD, "conv.npz"), **conv)
 
     # ---- small full transforms -----------------------------------------------
@@ -156,6 +167,10 @@ def main():
     fsel = np.array([391.9891989199264, 341.2, 250.0, 97.3, 31.0, 9.7])
     W, lens = ref_complex(CWT, Morse, sigtools, x, fs, 3, 20, fsel)
     cw["d_x"], cw["d_W"], cw["d_f"], cw["d_L"], cw["d_fs"] = x, W, fsel, lens, fs
+    # the outputs keep every scale and a sample of their columns, listed in <case>_cols
+    for key, k in (("a_amp", 800), ("b_amp", 1200), ("c_amp", 600), ("d_W", 1600)):
+        cols = sample_columns(cw[key].shape[1], k, 128)
+        cw[key], cw[key[0] + "_cols"] = cw[key][:, cols], cols
     np.savez_compressed(os.path.join(GOLD, "cwt_small.npz"), **cw)
 
     # ---- sparse samples of a cfg1-sized transform -----------------------------

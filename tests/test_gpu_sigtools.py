@@ -36,7 +36,8 @@ def test_fastconv_complex_kernel_same_offset(golden_dir):
     i = 0
     while f"s_{i}" in z:
         got = sigtools.fastconv(z[f"s_{i}"], z[f"k_{i}"])
-        assert _rel(got, z[f"y_{i}"]) <= 1e-13
+        assert got.shape == z[f"s_{i}"].shape
+        assert _rel(got[z[f"cols_{i}"]], z[f"y_{i}"]) <= 1e-13      # at the columns stored of the reference's output
         i += 1
     assert i == 6
 

@@ -62,12 +62,14 @@ def test_overlap_add_same_offset(golden_dir):
     i = 0
     while f"s_{i}" in z:
         s, k, y = z[f"s_{i}"], z[f"k_{i}"], z[f"y_{i}"]
+        cols = z[f"cols_{i}"]                  # the columns stored of the reference's output
         got = orc.overlap_add_same(s, k)
-        assert np.max(np.abs(got - y)) <= 1e-13 * np.max(np.abs(y))
+        assert got.shape == s.shape
+        assert np.max(np.abs(got[cols] - y)) <= 1e-13 * np.max(np.abs(y))
         if len(s) <= 5000:          # definition by direct summation
             d = orc.direct_same(s, k) if len(k) <= len(s) else None
             if d is not None:
-                assert np.max(np.abs(d - y)) <= 1e-12 * np.max(np.abs(y))
+                assert np.max(np.abs(d[cols] - y)) <= 1e-12 * np.max(np.abs(y))
         i += 1
     assert i == 6
 
@@ -76,8 +78,8 @@ def test_transform_default(golden_dir):
     z = _load(golden_dir, "cwt_small.npz")
     amp, f, _ = orc.cwt_amplitude(z["a_x"], float(z["a_fs"]))
     assert f.tolist() == z["a_f"].tolist()
-    assert amp.shape == z["a_amp"].shape
-    assert np.max(np.abs(amp - z["a_amp"])) <= 1e-13 * np.max(z["a_amp"])
+    assert amp.shape == (len(z["a_f"]), len(z["a_x"]))
+    assert np.max(np.abs(amp[:, z["a_cols"]] - z["a_amp"])) <= 1e-13 * np.max(z["a_amp"])
 
 
 def test_transform_two_epochs_nonzero_mean(golden_dir):
@@ -86,7 +88,8 @@ def test_transform_two_epochs_nonzero_mean(golden_dir):
                                   freq_limits=[20, 300], voices_per_octave=6,
                                   timestamps=z["b_ts"])
     assert f.tolist() == z["b_f"].tolist()
-    assert np.max(np.abs(amp - z["b_amp"])) <= 1e-13 * np.max(z["b_amp"])
+    assert amp.shape == (len(z["b_f"]), len(z["b_x"]))
+    assert np.max(np.abs(amp[:, z["b_cols"]] - z["b_amp"])) <= 1e-13 * np.max(z["b_amp"])
     ep = orc.contiguous_segments(z["b_ts"], 1 / float(z["b_fs"]))
     assert ep.tolist() == [[0, 1700], [1700, 3000]]
 
@@ -96,15 +99,17 @@ def test_transform_float32_input_parallel(golden_dir):
     amp, f, _ = orc.cwt_amplitude(z["c_x"], float(z["c_fs"]), parallel=True)
     assert z["c_x"].dtype == np.float32 and amp.dtype == np.float64
     assert f.tolist() == z["c_f"].tolist()
-    assert np.max(np.abs(amp - z["c_amp"])) <= 1e-13 * np.max(z["c_amp"])
+    assert amp.shape == (len(z["c_f"]), len(z["c_x"]))
+    assert np.max(np.abs(amp[:, z["c_cols"]] - z["c_amp"])) <= 1e-13 * np.max(z["c_amp"])
 
 
 def test_complex_coefficients(golden_dir):
     z = _load(golden_dir, "cwt_small.npz")
     W, f, L = orc.cwt_complex(z["d_x"], float(z["d_fs"]), frequencies=z["d_f"])
     assert L.tolist() == z["d_L"].tolist()
+    assert W.shape == (len(z["d_f"]), len(z["d_x"]))
     for s in range(len(f)):
-        err = np.max(np.abs(W[s] - z["d_W"][s])) / np.max(np.abs(z["d_W"][s]))
+        err = np.max(np.abs(W[s, z["d_cols"]] - z["d_W"][s])) / np.max(np.abs(z["d_W"][s]))
         assert err <= 1e-13, (s, err)
 
 
