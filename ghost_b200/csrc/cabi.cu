@@ -351,6 +351,52 @@ int gcwt_pool_rows(const void* x_dev, int32_t type, int64_t n_rows, int64_t n_co
                             (cudaStream_t)stream);
 }
 
+int gcwt_band_reduce(const void* coef_dev, int32_t coef_type, int32_t coef_kind, int64_t n_channels, int64_t n_samples,
+                     int64_t scale_stride, int64_t channel_stride, int32_t n_bands, const int32_t* band_first,
+                     const int32_t* band_count, const double* weights, void* out_dev, int64_t out_band_stride,
+                     int64_t out_channel_stride, int32_t device, void* stream) {
+    if (!coef_dev || !out_dev) { set_error("band_reduce: coef/out is NULL"); return GCWT_ERR_ARG; }
+    if (coef_type != GCWT_F32 && coef_type != GCWT_F64) { set_error("band_reduce: coef_type must be GCWT_F32 or GCWT_F64"); return GCWT_ERR_ARG; }
+    if (coef_kind < GCWT_OUT_COMPLEX || coef_kind > GCWT_OUT_POWER) { set_error("band_reduce: bad coef_kind"); return GCWT_ERR_ARG; }
+    if (n_channels <= 0 || n_samples <= 0) { set_error("band_reduce: n_channels and n_samples must be positive"); return GCWT_ERR_ARG; }
+    BandTable tab;
+    int rc = band_table_build(n_bands, band_first, band_count, weights, &tab, "band_reduce");
+    if (rc) return rc;
+    if (scale_stride < n_samples || (n_channels > 1 && channel_stride < (int64_t)tab.rows * scale_stride)) {
+        set_error("band_reduce: scale_stride below n_samples, or channel_stride below the rows the bands read"); return GCWT_ERR_ARG;
+    }
+    if (out_band_stride < n_samples || (n_channels > 1 && out_channel_stride < (int64_t)n_bands * out_band_stride)) {
+        set_error("band_reduce: out_band_stride below n_samples, or out_channel_stride below n_bands rows"); return GCWT_ERR_ARG;
+    }
+    DeviceScope dev_scope(device);
+    return band_reduce_launch(coef_dev, coef_type, coef_kind, n_channels, n_samples, scale_stride, channel_stride, tab,
+                              out_dev, out_band_stride, out_channel_stride, (cudaStream_t)stream);
+}
+
+int gcwt_execute_host_bands(gcwt_plan* p, const void* x, int32_t in_type, int64_t n_channels, int64_t n_samples,
+                            int64_t x_stride, const int64_t* epoch_bounds, int32_t n_epochs, const double* means_host,
+                            int32_t n_bands, const int32_t* band_first, const int32_t* band_count, const double* weights,
+                            void* out, int64_t out_band_stride, int64_t out_channel_stride) {
+    BandTable tab;
+    int rc = band_table_build(n_bands, band_first, band_count, weights, &tab, "execute_host_bands");
+    if (rc) return rc;
+    rc = check_exec_args(p, x, in_type, n_channels, n_samples, x_stride, out);
+    if (rc) return rc;
+    if (tab.rows > p->n_scales) {
+        set_error("execute_host_bands: a band reaches scale " + std::to_string(tab.rows - 1) + " of a plan with " +
+                  std::to_string(p->n_scales) + " scales");
+        return GCWT_ERR_ARG;
+    }
+    if (out_band_stride < n_samples || (n_channels > 1 && out_channel_stride < (int64_t)n_bands * out_band_stride)) {
+        set_error("execute_host_bands: out_band_stride below n_samples, or out_channel_stride below n_bands rows"); return GCWT_ERR_ARG;
+    }
+    DeviceScope dev_scope(p->device);
+    int64_t tile_hint = 0;
+    if (const char* e = getenv("GCWT_HOST_TILE")) tile_hint = atoll(e);
+    return host_execute(p, x, in_type, n_channels, n_samples, x_stride, epoch_bounds, n_epochs, means_host, out,
+                        out_band_stride, out_channel_stride, tile_hint, 0, 0, &tab);
+}
+
 int gcwt_host_stats(const gcwt_plan* p, double* out4) {
     if (!p || !out4) { set_error("host_stats: NULL argument"); return GCWT_ERR_ARG; }
     for (int k = 0; k < 4; ++k) out4[k] = p->host.last_ms[k];

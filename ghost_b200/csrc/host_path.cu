@@ -64,11 +64,11 @@ static bool is_pinned(const void* ptr) {
     return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
 }
 
-// rows [r0, r1) of a tile: row r = (channel, scale) -> width bytes from the ring to the caller's array
+// rows [r0, r1) of a tile: row r = (channel, scale or band) -> width bytes from the ring to the caller's array
 struct RowCopy {
     const char* src; size_t src_pitch;          // ring: rows are dense (tile_alloc elements apart)
     char* dst; int64_t s_stride_b, c_stride_b;  // caller strides in bytes
-    int n_scales; size_t width; int64_t n_rows;
+    int rows_per_channel; size_t width; int64_t n_rows;
 };
 
 static void copy_rows(const RowCopy& rc, int n_threads) {
@@ -77,7 +77,7 @@ static void copy_rows(const RowCopy& rc, int n_threads) {
         for (;;) {
             const int64_t r = next.fetch_add(1);
             if (r >= rc.n_rows) break;
-            const int64_t c = r / rc.n_scales, s = r % rc.n_scales;
+            const int64_t c = r / rc.rows_per_channel, s = r % rc.rows_per_channel;
             memcpy(rc.dst + c * rc.c_stride_b + s * rc.s_stride_b, rc.src + (size_t)r * rc.src_pitch, rc.width);
         }
     };
@@ -89,15 +89,22 @@ static void copy_rows(const RowCopy& rc, int n_threads) {
 
 int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n, int64_t x_stride,
                  const int64_t* epochs, int n_epochs, const double* means_host, void* out, int64_t s_stride,
-                 int64_t c_stride, int64_t tile_hint, int64_t pool_width, int pool_mode) {
+                 int64_t c_stride, int64_t tile_hint, int64_t pool_width, int pool_mode, const BandTable* bands) {
     // pool_width > 0: `out` is a float64 array of ceil(n / pool_width) bins per row; every tile is reduced on the
-    // device (mean or max over pool_width consecutive samples) and only the bins travel to the host
+    // device (mean or max over pool_width consecutive samples) and only the bins travel to the host.
+    // bands: `out` holds (channels x bands x samples) of the plan's real type (s_stride is the band stride); every
+    // tile is band-reduced on the device into d_pool and only the band rows travel, by the same pinned-DMA /
+    // ring-and-copier routes as full-rate tiles (h_pool is the ring).  The tile geometry stays that of the
+    // full-rate path, so every coefficient summed is the one gcwt_execute_host would have written.
     gcwt_plan::HostStage& h = p->host;
     const auto t_begin = std::chrono::steady_clock::now();
     const int S = p->n_scales;
     const size_t in_el = in_type == GCWT_F32 ? 4 : 8;
     size_t out_el = p->compute_type == GCWT_F32 ? 4 : 8;
     if (p->out_kind == GCWT_OUT_COMPLEX) out_el *= 2;
+    const bool pooled = pool_width > 0, banded = bands != nullptr;
+    const int R = banded ? bands->n_bands : S;                    // rows per channel that reach `out`
+    const size_t xfer_el = banded ? (p->compute_type == GCWT_F32 ? 4 : 8) : out_el;
     int64_t one_epoch[2] = {0, n};
     if (!epochs || n_epochs <= 0) { epochs = one_epoch; n_epochs = 1; }
     for (int e = 0; e < n_epochs; ++e)
@@ -127,7 +134,6 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
         tile = std::min<int64_t>(n, (tile + 1023) / 1024 * 1024);
     }
     if (tile_hint > 0) tile = std::min<int64_t>(n, std::max<int64_t>(tile_hint, 1024));
-    const bool pooled = pool_width > 0;
     if (pooled) {
         if (p->out_kind == GCWT_OUT_COMPLEX) { set_error("execute_host: pooling needs amplitude or power output"); return GCWT_ERR_ARG; }
         if (n_epochs != 1 || epochs[0] != 0 || epochs[1] != n) {
@@ -153,18 +159,22 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
         GCWT_CUDA_OK(cudaMalloc((void**)&h.d_means, sizeof(double) * g));
         h.means_cap = g;
     }
-    if (pooled && h.pool_bytes < (size_t)g * S * bins_per_tile * sizeof(double)) {
-        const size_t need = (size_t)g * S * bins_per_tile * sizeof(double);
+    const size_t reduced_bytes = pooled ? (size_t)g * S * bins_per_tile * sizeof(double)
+                                        : banded ? (size_t)g * R * tile_alloc * xfer_el : 0;
+    if (h.pool_bytes < reduced_bytes) {
         for (int b = 0; b < 2; ++b) {
             if (h.d_pool[b]) { cudaFree(h.d_pool[b]); h.d_pool[b] = nullptr; }
             if (h.h_pool[b]) { cudaFreeHost(h.h_pool[b]); h.h_pool[b] = nullptr; }
-            GCWT_CUDA_OK(cudaMalloc((void**)&h.d_pool[b], need));
-            GCWT_CUDA_OK(cudaMallocHost((void**)&h.h_pool[b], need));
         }
-        h.pool_bytes = need;
+        h.pool_bytes = 0;
+        for (int b = 0; b < 2; ++b) {
+            GCWT_CUDA_OK(cudaMalloc(&h.d_pool[b], reduced_bytes));
+            GCWT_CUDA_OK(cudaMallocHost(&h.h_pool[b], reduced_bytes));
+        }
+        h.pool_bytes = reduced_bytes;
     }
     const bool direct = pooled || is_pinned(out);
-    if (!direct && h.ring_bytes < tile_bytes) {
+    if (!direct && !banded && h.ring_bytes < tile_bytes) {
         for (int b = 0; b < 2; ++b) {
             if (h.h_ring[b]) { cudaFreeHost(h.h_ring[b]); h.h_ring[b] = nullptr; }
             cudaError_t e = cudaMallocHost(&h.h_ring[b], tile_bytes);
@@ -187,8 +197,8 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
             const int64_t gap_end = e < n_epochs ? epochs[2 * e] : n;
             if (gap_end > pos)
                 for (int64_t c = 0; c < n_channels; ++c)
-                    for (int s = 0; s < S; ++s)
-                        memset((char*)out + ((size_t)c * c_stride + (size_t)s * s_stride + pos) * out_el, 0, (size_t)(gap_end - pos) * out_el);
+                    for (int s = 0; s < R; ++s)
+                        memset((char*)out + ((size_t)c * c_stride + (size_t)s * s_stride + pos) * xfer_el, 0, (size_t)(gap_end - pos) * xfer_el);
             if (e < n_epochs) pos = epochs[2 * e + 1];
         }
     }
@@ -199,7 +209,7 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
         for (int64_t c = 0; c < pd.gc; ++c)
             for (int s = 0; s < S; ++s)
                 memcpy((double*)out + (size_t)(pd.c0 + c) * c_stride + (size_t)s * s_stride + b0,
-                       h.h_pool[b] + ((size_t)c * S + s) * bins_per_tile, (size_t)nb * sizeof(double));
+                       (const double*)h.h_pool[b] + ((size_t)c * S + s) * bins_per_tile, (size_t)nb * sizeof(double));
     };
     Pending pend[2];
     struct Copiers {                                               // joined on every return path (an early error return
@@ -254,31 +264,44 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
                                   std::min(halo, e1 - b_end), h.d_means, h.d_out[slot], tile_alloc, (int64_t)S * tile_alloc,
                                   h.st_compute);
                 if (rc) break;
+                // ev_done follows the whole of gcwt_execute in stream order, including the accuracy guard's fp64
+                // re-computation of the failing (channel, scale) pairs (guard_resolve), so the reductions below read
+                // the corrected coefficients.  For the same reason band power is a pass of its own and not part of
+                // the fused kernels' epilogue: there it would sum values the guard then replaces.
                 GCWT_CUDA_OK(cudaEventRecord(h.ev_done[slot], h.st_compute));
                 GCWT_CUDA_OK(cudaStreamWaitEvent(h.st_copy, h.ev_done[slot], 0));
-                char* dst = (char*)out + ((size_t)c0 * c_stride + (size_t)a) * out_el;
+                char* dst = (char*)out + ((size_t)c0 * c_stride + (size_t)a) * xfer_el;
+                const void* src = h.d_out[slot];                   // what travels: the tile, or its band rows
+                void* ring = h.h_ring[slot];
+                if (banded) {
+                    rc = band_reduce_launch(h.d_out[slot], p->compute_type, p->out_kind, gc, len, tile_alloc, (int64_t)S * tile_alloc,
+                                            *bands, h.d_pool[slot], tile_alloc, (int64_t)R * tile_alloc, h.st_copy);
+                    if (rc) break;
+                    src = h.d_pool[slot];
+                    ring = h.h_pool[slot];
+                }
                 if (pooled) {
                     rc = pool_rows_launch(h.d_out[slot], p->compute_type, gc * S, len, tile_alloc, pool_width, pool_mode, 0,
-                                          h.d_pool[slot], bins_per_tile, h.st_copy);
+                                          (double*)h.d_pool[slot], bins_per_tile, h.st_copy);
                     if (rc) break;
                     GCWT_CUDA_OK(cudaMemcpyAsync(h.h_pool[slot], h.d_pool[slot], (size_t)gc * S * bins_per_tile * sizeof(double),
                                                  cudaMemcpyDeviceToHost, h.st_copy));
                     GCWT_CUDA_OK(cudaEventRecord(h.ev_out[slot], h.st_copy));
                 } else if (direct) {
                     for (int64_t c = 0; c < gc; ++c)
-                        GCWT_CUDA_OK(cudaMemcpy2DAsync(dst + (size_t)c * c_stride * out_el, (size_t)s_stride * out_el,
-                                                       (const char*)h.d_out[slot] + (size_t)c * S * tile_alloc * out_el,
-                                                       (size_t)tile_alloc * out_el, (size_t)len * out_el, (size_t)S,
+                        GCWT_CUDA_OK(cudaMemcpy2DAsync(dst + (size_t)c * c_stride * xfer_el, (size_t)s_stride * xfer_el,
+                                                       (const char*)src + (size_t)c * R * tile_alloc * xfer_el,
+                                                       (size_t)tile_alloc * xfer_el, (size_t)len * xfer_el, (size_t)R,
                                                        cudaMemcpyDeviceToHost, h.st_copy));
                     GCWT_CUDA_OK(cudaEventRecord(h.ev_out[slot], h.st_copy));
                 } else {
-                    GCWT_CUDA_OK(cudaMemcpyAsync(h.h_ring[slot], h.d_out[slot], (size_t)gc * S * tile_alloc * out_el,
+                    GCWT_CUDA_OK(cudaMemcpyAsync(ring, src, (size_t)gc * R * tile_alloc * xfer_el,
                                                  cudaMemcpyDeviceToHost, h.st_copy));
                     GCWT_CUDA_OK(cudaEventRecord(h.ev_out[slot], h.st_copy));
                     RowCopy rcp;
-                    rcp.src = (const char*)h.h_ring[slot]; rcp.src_pitch = (size_t)tile_alloc * out_el;
-                    rcp.dst = dst; rcp.s_stride_b = s_stride * (int64_t)out_el; rcp.c_stride_b = c_stride * (int64_t)out_el;
-                    rcp.n_scales = S; rcp.width = (size_t)len * out_el; rcp.n_rows = gc * S;
+                    rcp.src = (const char*)ring; rcp.src_pitch = (size_t)tile_alloc * xfer_el;
+                    rcp.dst = dst; rcp.s_stride_b = s_stride * (int64_t)xfer_el; rcp.c_stride_b = c_stride * (int64_t)xfer_el;
+                    rcp.rows_per_channel = R; rcp.width = (size_t)len * xfer_el; rcp.n_rows = gc * R;
                     cudaEvent_t ev = h.ev_out[slot];
                     const int dev = p->device;
                     copier[slot] = std::thread([rcp, ev, dev, n_threads]() {
@@ -288,7 +311,7 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
                     });
                 }
                 pend[slot].live = true; pend[slot].c0 = c0; pend[slot].gc = gc; pend[slot].a = a; pend[slot].len = len;
-                bytes_out += pooled ? (double)gc * S * ((len + pool_width - 1) / pool_width) * sizeof(double) : (double)gc * S * len * out_el;
+                bytes_out += pooled ? (double)gc * S * ((len + pool_width - 1) / pool_width) * sizeof(double) : (double)gc * R * len * xfer_el;
                 ++n_tiles;
                 slot ^= 1;
             }

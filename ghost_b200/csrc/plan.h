@@ -83,6 +83,18 @@ struct Workspace {
     size_t bytes = 0;
 };
 
+// ---- scale-averaged band power (gcwt_band_reduce, gcwt_execute_host_bands) ---------------------
+// Band b sums rows first[b] .. first[b] + count[b] - 1 with weights w[off[b] + k].  The table is passed to
+// the kernel by value (__grid_constant__), so a call needs no allocation and no host-to-device copy.
+constexpr int kMaxBands = 64;
+constexpr int kMaxBandEntries = 1024;   // sum of count[b]
+struct BandTable {
+    int32_t n_bands;
+    int32_t rows;                       // max(first[b] + count[b]): rows of a channel the bands read
+    int32_t first[kMaxBands], count[kMaxBands], off[kMaxBands];
+    double w[kMaxBandEntries];
+};
+
 }  // namespace gcwt
 
 struct gcwt_plan {
@@ -141,7 +153,7 @@ struct gcwt_plan {
         void* d_in = nullptr; size_t in_bytes = 0;           // the channel group's samples
         void* d_out[2] = {nullptr, nullptr}; size_t out_bytes = 0;   // double-buffered result tiles
         void* h_ring[2] = {nullptr, nullptr}; size_t ring_bytes = 0; // pinned bounce buffers (pageable destinations only)
-        double* d_pool[2] = {nullptr, nullptr}; double* h_pool[2] = {nullptr, nullptr}; size_t pool_bytes = 0;   // pooled tiles
+        void* d_pool[2] = {nullptr, nullptr}; void* h_pool[2] = {nullptr, nullptr}; size_t pool_bytes = 0;   // pooled / band-reduced tiles
         double* d_means = nullptr; int64_t means_cap = 0;
         cudaStream_t st_compute = nullptr, st_copy = nullptr;
         cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
@@ -178,8 +190,18 @@ int means_launch(const void* x, int in_type, int64_t n_channels, int64_t n_sampl
                  int64_t x_stride, double* d_means, double* partial, cudaStream_t st);
 int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n_samples, int64_t x_stride,
                  const int64_t* epochs, int n_epochs, const double* means_host, void* out, int64_t s_stride,
-                 int64_t c_stride, int64_t tile_hint, int64_t pool_width = 0, int pool_mode = 0);
+                 int64_t c_stride, int64_t tile_hint, int64_t pool_width = 0, int pool_mode = 0,
+                 const BandTable* bands = nullptr);
 int pool_rows_launch(const void* x_dev, int type, int64_t n_rows, int64_t n_cols, int64_t row_stride, int64_t width,
                      int mode, int square, double* out_dev, int64_t out_stride, cudaStream_t st);
+// host-side checks of a band table (NULL pointers, 1..kMaxBands bands, count >= 1, first >= 0, at most
+// kMaxBandEntries entries); `who` prefixes the error text.  Ranges against the scale count are the caller's.
+int band_table_build(int n_bands, const int32_t* first, const int32_t* count, const double* weights, BandTable* tab,
+                     const char* who);
+// out[c, b, n] = sum_k w[off_b + k] |x[c, first_b + k, n]|^2 in fp64, written as `type`; x holds elements of
+// `type` (float2 / double2 for kind GCWT_OUT_COMPLEX), strides in elements, out strides in real elements
+int band_reduce_launch(const void* x_dev, int type, int kind, int64_t n_channels, int64_t n_samples, int64_t s_stride,
+                       int64_t c_stride, const BandTable& tab, void* out_dev, int64_t out_b_stride, int64_t out_c_stride,
+                       cudaStream_t st);
 void host_stage_free(gcwt_plan* p);
 }  // namespace gcwt

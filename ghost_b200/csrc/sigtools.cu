@@ -7,9 +7,14 @@
 // All in complex128 like the reference.  They share the batched power-of-two Stockham FFT of
 // the generic CWT path; lengths that are not a power of two go through Bluestein's chirp-z
 // identity (what chirpz_dft does on the CPU) with exact integer phase reduction.
+//
+// Reductions of a result on the device, so that only the reduced array crosses the link: moments and
+// time pooling for displays, and scale-averaged band power (band_reduce_kernel).
 #include "plan.h"
 #include "common.cuh"
 #include "fft_global.cuh"
+#include <algorithm>
+#include <string>
 #include <vector>
 
 namespace gcwt {
@@ -271,6 +276,130 @@ int pool_rows_launch(const void* x_dev, int type, int64_t n_rows, int64_t n_cols
             pool_rows_kernel<double><<<grid, 256, 0, st>>>((const double*)x_dev + r0 * row_stride, row_stride, n_cols, width,
                                                            mode, square, out_dev + r0 * out_stride, out_stride, n_bins);
         count_launch();
+    }
+    GCWT_CUDA_OK(cudaGetLastError());
+    return GCWT_OK;
+}
+
+// ----------------------------------------------------------------------------- scale-averaged band power
+// Band power over time (theta, gamma, ripple envelopes) averages |W|^2 over the adjacent scales of a band.
+// One thread owns VEC consecutive samples of one (channel, band) and walks the band's rows: a pure streaming
+// read of 16-byte loads when the rows are aligned, accumulated in fp64 with explicit fma so that the vector
+// and scalar paths give the same bits.  Overlapping bands re-read their shared rows.
+__device__ __forceinline__ double mag2(float v, bool power) { const double d = v; return power ? d : d * d; }
+__device__ __forceinline__ double mag2(double v, bool power) { return power ? v : v * v; }
+__device__ __forceinline__ double mag2(float2 v, bool) { const double re = v.x, im = v.y; return fma(re, re, im * im); }
+__device__ __forceinline__ double mag2(double2 v, bool) { return fma(v.x, v.x, v.y * v.y); }
+
+template <typename In, typename Out, int VEC, bool POWER>
+__global__ void __launch_bounds__(256)
+band_reduce_kernel(const In* __restrict__ x, int64_t n, int64_t s_stride, int64_t c_stride, Out* __restrict__ out,
+                   int64_t ob_stride, int64_t oc_stride, const __grid_constant__ BandTable tab) {
+    struct alignas(sizeof(In) * VEC) InV { In v[VEC]; };
+    struct alignas(sizeof(Out) * VEC) OutV { Out v[VEC]; };
+    const int b = blockIdx.z;
+    const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
+    if (i0 >= n) return;
+    const int cnt = tab.count[b];
+    const double* w = tab.w + tab.off[b];
+    const In* row = x + (int64_t)blockIdx.y * c_stride + (int64_t)tab.first[b] * s_stride + i0;
+    Out* dst = out + (int64_t)blockIdx.y * oc_stride + (int64_t)b * ob_stride + i0;
+    double acc[VEC];
+#pragma unroll
+    for (int j = 0; j < VEC; ++j) acc[j] = 0.0;
+    if (i0 + VEC <= n) {
+#pragma unroll 4
+        for (int k = 0; k < cnt; ++k) {
+            const InV v = *reinterpret_cast<const InV*>(row + (int64_t)k * s_stride);
+            const double wk = w[k];
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) acc[j] = fma(wk, mag2(v.v[j], POWER), acc[j]);
+        }
+        OutV o;
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) o.v[j] = (Out)acc[j];
+        *reinterpret_cast<OutV*>(dst) = o;
+    } else {                                                         // the row's last, partial vector
+        const int m = (int)(n - i0);
+        for (int k = 0; k < cnt; ++k)
+#pragma unroll
+            for (int j = 0; j < VEC; ++j)
+                if (j < m) acc[j] = fma(w[k], mag2(row[(int64_t)k * s_stride + j], POWER), acc[j]);
+#pragma unroll
+        for (int j = 0; j < VEC; ++j)
+            if (j < m) dst[j] = (Out)acc[j];
+    }
+}
+
+int band_table_build(int n_bands, const int32_t* first, const int32_t* count, const double* weights, BandTable* tab,
+                     const char* who) {
+    const std::string pre = std::string(who) + ": ";
+    if (!first || !count || !weights) { set_error(pre + "band_first / band_count / weights is NULL"); return GCWT_ERR_ARG; }
+    if (n_bands < 1 || n_bands > kMaxBands) {
+        set_error(pre + "n_bands must be 1 .. " + std::to_string(kMaxBands) + " (got " + std::to_string(n_bands) + ")");
+        return GCWT_ERR_ARG;
+    }
+    tab->n_bands = n_bands;
+    tab->rows = 0;
+    int off = 0;
+    for (int b = 0; b < n_bands; ++b) {
+        if (first[b] < 0 || count[b] < 1) {
+            set_error(pre + "band " + std::to_string(b) + " needs first >= 0 and count >= 1 (got first " +
+                      std::to_string(first[b]) + ", count " + std::to_string(count[b]) + ")");
+            return GCWT_ERR_ARG;
+        }
+        if (count[b] > kMaxBandEntries - off) {
+            set_error(pre + "the bands hold more than " + std::to_string(kMaxBandEntries) + " (band, scale) entries");
+            return GCWT_ERR_ARG;
+        }
+        tab->first[b] = first[b];
+        tab->count[b] = count[b];
+        tab->off[b] = off;
+        for (int k = 0; k < count[b]; ++k) tab->w[off + k] = weights[off + k];
+        off += count[b];
+        tab->rows = std::max<int32_t>(tab->rows, (int32_t)std::min<int64_t>((int64_t)first[b] + count[b], INT32_MAX));
+    }
+    return GCWT_OK;
+}
+
+template <typename In, typename Out, int VEC>
+static void band_launch(const void* x, int kind, int64_t n_ch, int64_t n, int64_t s_stride, int64_t c_stride,
+                        const BandTable& tab, void* out, int64_t ob_stride, int64_t oc_stride, cudaStream_t st) {
+    for (int64_t c0 = 0; c0 < n_ch; c0 += 65535) {                   // gridDim.y limit
+        const int64_t rows = std::min<int64_t>(65535, n_ch - c0);
+        dim3 grid((unsigned)((n + 256 * VEC - 1) / (256 * VEC)), (unsigned)rows, (unsigned)tab.n_bands);
+        const In* xs = (const In*)x + c0 * c_stride;
+        Out* os = (Out*)out + c0 * oc_stride;
+        if (kind == GCWT_OUT_POWER)
+            band_reduce_kernel<In, Out, VEC, true><<<grid, 256, 0, st>>>(xs, n, s_stride, c_stride, os, ob_stride, oc_stride, tab);
+        else
+            band_reduce_kernel<In, Out, VEC, false><<<grid, 256, 0, st>>>(xs, n, s_stride, c_stride, os, ob_stride, oc_stride, tab);
+        count_launch();
+    }
+}
+
+// 16-byte vectors when every row of the input and of the output starts on a vector boundary, else one sample per thread
+template <typename In, typename Out>
+static void band_dispatch(const void* x, int kind, int64_t n_ch, int64_t n, int64_t s_stride, int64_t c_stride,
+                          const BandTable& tab, void* out, int64_t ob_stride, int64_t oc_stride, cudaStream_t st) {
+    constexpr int V = 16 / sizeof(In);
+    const bool vec = (uintptr_t)x % 16 == 0 && (uintptr_t)out % (sizeof(Out) * V) == 0 && s_stride % V == 0 &&
+                     c_stride % V == 0 && ob_stride % V == 0 && oc_stride % V == 0;
+    if (vec) band_launch<In, Out, V>(x, kind, n_ch, n, s_stride, c_stride, tab, out, ob_stride, oc_stride, st);
+    else band_launch<In, Out, 1>(x, kind, n_ch, n, s_stride, c_stride, tab, out, ob_stride, oc_stride, st);
+}
+
+int band_reduce_launch(const void* x_dev, int type, int kind, int64_t n_channels, int64_t n_samples, int64_t s_stride,
+                       int64_t c_stride, const BandTable& tab, void* out_dev, int64_t out_b_stride, int64_t out_c_stride,
+                       cudaStream_t st) {
+    if (n_channels <= 0 || n_samples <= 0) { set_error("band_reduce: empty input"); return GCWT_ERR_ARG; }
+    const bool cx = kind == GCWT_OUT_COMPLEX;
+    if (type == GCWT_F32) {
+        if (cx) band_dispatch<float2, float>(x_dev, kind, n_channels, n_samples, s_stride, c_stride, tab, out_dev, out_b_stride, out_c_stride, st);
+        else band_dispatch<float, float>(x_dev, kind, n_channels, n_samples, s_stride, c_stride, tab, out_dev, out_b_stride, out_c_stride, st);
+    } else {
+        if (cx) band_dispatch<double2, double>(x_dev, kind, n_channels, n_samples, s_stride, c_stride, tab, out_dev, out_b_stride, out_c_stride, st);
+        else band_dispatch<double, double>(x_dev, kind, n_channels, n_samples, s_stride, c_stride, tab, out_dev, out_b_stride, out_c_stride, st);
     }
     GCWT_CUDA_OK(cudaGetLastError());
     return GCWT_OK;

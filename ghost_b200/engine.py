@@ -12,9 +12,54 @@ import numpy as np
 
 from . import _lib
 
-__all__ = ["CwtPlan", "scale_tables", "OUT_KINDS"]
+__all__ = ["CwtPlan", "scale_tables", "band_tables", "OUT_KINDS"]
 
 OUT_KINDS = {"complex": _lib.OUT_COMPLEX, "amplitude": _lib.OUT_AMPLITUDE, "power": _lib.OUT_POWER}
+BAND_REDUCE = ("mean", "sum")
+
+
+def band_tables(frequencies, bands, reduce="mean"):
+    """Map frequency bands in Hz to the scale rows of a grid: ``(first, count, weights)`` for
+    gcwt_band_reduce / gcwt_execute_host_bands.
+
+    Band ``(lo, hi)`` holds every scale whose grid frequency f satisfies ``lo <= f <= hi``; on a monotone grid
+    that is one contiguous run of rows ``first .. first + count - 1``.  Bands keep the caller's order and may
+    overlap.  ``reduce='mean'`` weights each scale 1 / count, ``'sum'`` weights it 1."""
+    if reduce not in BAND_REDUCE:
+        raise ValueError("'band_reduce' must be 'mean' or 'sum' but got {}".format(reduce))
+    f = np.asarray(frequencies, dtype=np.float64).ravel()
+    try:
+        bands = [(float(lo), float(hi)) for lo, hi in bands]
+    except (TypeError, ValueError):
+        raise ValueError("'bands' must be a sequence of (low, high) pairs in Hz") from None
+    if not bands:
+        raise ValueError("'bands' must hold at least one (low, high) pair")
+    first, count = [], []
+    for lo, hi in bands:
+        if not (lo > 0 and hi > 0):
+            raise ValueError("band ({}, {}) Hz: limits must be positive".format(lo, hi))
+        if lo > hi:
+            raise ValueError("band ({}, {}) Hz: low limit above high limit".format(lo, hi))
+        idx = np.nonzero((f >= lo) & (f <= hi))[0]
+        if idx.size == 0:
+            grid = "the grid is empty" if f.size == 0 else "the grid spans {:.6g} .. {:.6g} Hz".format(f.min(), f.max())
+            raise ValueError("band ({}, {}) Hz holds no scale: {}".format(lo, hi, grid))
+        if idx[-1] - idx[0] + 1 != idx.size:
+            raise ValueError("band ({}, {}) Hz: the frequency grid is not monotone".format(lo, hi))
+        first.append(int(idx[0]))
+        count.append(int(idx.size))
+    count = np.asarray(count, dtype=np.int32)
+    weights = np.concatenate([np.full(c, 1.0 / c if reduce == "mean" else 1.0) for c in count])
+    return np.asarray(first, dtype=np.int32), count, np.ascontiguousarray(weights, dtype=np.float64)
+
+
+def _band_args(first, count, weights):
+    first = np.ascontiguousarray(first, dtype=np.int32)
+    count = np.ascontiguousarray(count, dtype=np.int32)
+    weights = np.ascontiguousarray(weights, dtype=np.float64)
+    if first.ndim != 1 or first.shape != count.shape or weights.shape != (int(count.sum()),):
+        raise ValueError("first and count need one entry per band and weights one per (band, scale) entry")
+    return first, count, weights
 
 
 def scale_tables(wavelet, norm_radian_freqs, lengths):
@@ -279,6 +324,66 @@ class CwtPlan:
                                            flat.stride(0), int(pool_width), _lib.POOL_MEAN if pool == "mean" else _lib.POOL_MAX,
                                            1 if square else 0, out.data_ptr(), n_bins, self.device, st))
         return out.reshape(tuple(res.shape[:-1]) + (n_bins,))
+
+    def execute_host_bands(self, x, first, count, weights, epochs=None, means=None):
+        """As :meth:`execute_host`, but every tile is reduced to scale-averaged band power on the device
+        (gcwt_execute_host_bands) and only (channels, bands, samples) of the plan's real dtype crosses the link.
+        Band b is ``sum_k weights[off_b + k] * |W[:, first[b] + k, :]|**2`` (see :func:`band_tables`); samples
+        outside the ``epochs`` are zero."""
+        first, count, weights = _band_args(first, count, weights)
+        x = np.asarray(x)
+        if x.ndim == 1:
+            x = x[None, :]
+        if x.ndim != 2:
+            raise ValueError("x must be (channels, samples)")
+        if x.dtype not in (np.float32, np.float64) or (self.dtype == np.float64 and x.dtype != np.float64):
+            x = x.astype(np.float64)
+        if x.strides[1] != x.itemsize:
+            x = np.ascontiguousarray(x)
+        n_ch, n = x.shape
+        n_b = int(first.size)
+        out = np.empty((n_ch, n_b, n), dtype=self.dtype)
+        mptr = None
+        if means is not None:
+            means = np.ascontiguousarray(means, dtype=np.float64)
+            if means.size != n_ch:
+                raise ValueError("means must hold one value per channel")
+            mptr = means.ctypes.data
+        eptr, n_ep = None, 0
+        if epochs is not None:
+            epochs = np.ascontiguousarray(epochs, dtype=np.int64).reshape(-1, 2)
+            eptr, n_ep = epochs.ctypes.data, int(epochs.shape[0])
+        in_type = _lib.F32 if x.dtype == np.float32 else _lib.F64
+        _lib.check(self.lib.gcwt_execute_host_bands(
+            self._h, x.ctypes.data, in_type, n_ch, n, x.strides[0] // x.itemsize, eptr, n_ep, mptr,
+            n_b, first.ctypes.data, count.ctypes.data, weights.ctypes.data, out.ctypes.data, n, n_b * n))
+        return out
+
+    def band_reduce(self, res, first, count, weights):
+        """Scale-averaged band power of a device-resident (channels, scales, samples) result ``res`` (a CUDA
+        tensor with unit sample stride; a window of a larger result is fine): a (channels, bands, samples) CUDA
+        tensor of ``res``'s real dtype, through gcwt_band_reduce on the current stream.  |W|^2 is re^2 + im^2
+        for a complex tensor, and for a real one the square of an amplitude or the power itself, as this
+        plan's ``output`` says."""
+        torch = _torch()
+        first, count, weights = _band_args(first, count, weights)
+        if not res.is_cuda or res.dim() != 3 or res.stride(2) != 1 or \
+                res.dtype not in (torch.float32, torch.float64, torch.complex64, torch.complex128):
+            raise ValueError("band_reduce needs a (channels, scales, samples) float / complex CUDA tensor with unit "
+                             "sample stride")
+        if int((first + count).max()) > res.shape[1]:
+            raise ValueError("a band reaches past the {} scales of the result".format(res.shape[1]))
+        n_ch, _, n = res.shape
+        cx = res.is_complex()
+        rdt = {torch.complex64: torch.float32, torch.complex128: torch.float64}.get(res.dtype, res.dtype)
+        kind = _lib.OUT_COMPLEX if cx else (_lib.OUT_POWER if self.output == "power" else _lib.OUT_AMPLITUDE)
+        out = torch.empty((n_ch, first.size, n), dtype=rdt, device=res.device)
+        st = torch.cuda.current_stream(res.device).cuda_stream
+        _lib.check(self.lib.gcwt_band_reduce(
+            res.data_ptr(), _lib.F32 if rdt == torch.float32 else _lib.F64, kind, n_ch, n, res.stride(1),
+            res.stride(0), int(first.size), first.ctypes.data, count.ctypes.data, weights.ctypes.data,
+            out.data_ptr(), n, first.size * n, res.device.index, st))
+        return out
 
     def host_stats(self):
         """{wall_ms, pinned_destination, tiles, bytes_out} of the last execute_host."""

@@ -9,7 +9,8 @@ into libghostcwt.so.
 
 Extensions (keyword-only, all optional): ``dtype`` (float64 reproduces the reference to
 1e-10; float32 is the HBM-roofline path), ``output`` ('amplitude' | 'power' | 'complex'),
-``device``, ``multichannel`` (rows of a 2-D array are channels) and ``keep_on_device``.
+``device``, ``multichannel`` (rows of a 2-D array are channels) and ``keep_on_device``; ``bands`` keeps
+only scale-averaged band power (``band_power``), reduced on the device.
 """
 from __future__ import annotations
 
@@ -91,6 +92,9 @@ class ContinuousWaveletTransform(WaveletTransform):
         self._time = None
         self._result = None          # torch tensor (C, S, N) on the device, or None
         self._host = None            # numpy view of the result, filled lazily
+        self._band_power = None      # (B, N) or (C, B, N) after transform(bands=...): the only result kept
+        self._band_frequencies = None
+        self._pooled = False         # the result was pooled over time (pool_width)
         self._multichannel = False
         self._time_auto = None       # (n, fs) when self._time is the implicit arange(n) / fs
         self._plans = {}
@@ -139,7 +143,8 @@ class ContinuousWaveletTransform(WaveletTransform):
     # ------------------------------------------------------------------ transform
     def transform(self, data, *, timestamps=None, fs=None, freq_limits=None, freqs=None,
                   voices_per_octave=None, parallel=None, verbose=None, multichannel=None,
-                  keep_on_device=None, out=None, pool_width=None, pool=None, **kwargs):
+                  keep_on_device=None, out=None, pool_width=None, pool=None, bands=None, band_reduce=None,
+                  **kwargs):
         """Continuous wavelet transform of one recording.
 
         Parameters as the reference (transforms.py:59-106): ``data`` is an ndarray with
@@ -160,8 +165,20 @@ class ContinuousWaveletTransform(WaveletTransform):
         arrays read back have ceil(samples / w) columns (float64) and ``time`` holds the bin centres --
         the link then carries kilobytes instead of every coefficient.
 
+        ``bands=[(lo, hi), ...]`` (Hz) keeps only scale-averaged band power: for every band, the mean
+        (``band_reduce='mean'``) or sum (``'sum'``) of |W|^2 over the scales whose frequency lies in
+        [lo, hi], at every sample, reduced on the device tile by tile so that only (bands x samples) per
+        channel crosses the link.  The result is ``band_power``, shaped (B, N), or (C, B, N) with
+        ``multichannel``, in the plan's dtype; ``band_frequencies`` lists each band's grid frequencies.
+        ``amplitude``, ``power`` and ``coefficients`` are then not available.
+
         Returns None; results are read from the properties.
         """
+        if bands is None:
+            if band_reduce is not None:
+                raise ValueError("'band_reduce' needs 'bands'")
+        elif out is not None or pool_width is not None or keep_on_device:
+            raise ValueError("'bands' cannot be combined with 'out', 'pool_width' or 'keep_on_device'")
         if multichannel is None:
             multichannel = False
         if multichannel:
@@ -215,6 +232,11 @@ class ContinuousWaveletTransform(WaveletTransform):
                                                        freqs=freqs, voices_per_octave=voices_per_octave),
                                  dtype=np.float64)
         self._frequencies = frequencies
+        self._band_power = self._band_frequencies = None
+        self._pooled = pool_width is not None
+        if bands is not None:
+            from ..engine import band_tables
+            b_first, b_count, b_weights = band_tables(frequencies, bands, "mean" if band_reduce is None else band_reduce)
         if frequencies.size == 0:
             # data too short for any scale: the reference ends up with a (0, N) array
             self._multichannel = bool(multichannel)
@@ -232,7 +254,14 @@ class ContinuousWaveletTransform(WaveletTransform):
         self._host = None
         self._result = None
         start_time = _time.time()
-        if pool_width is not None:
+        if bands is not None:
+            # band power only: every tile is reduced over scales on the device and (bands x samples) per channel
+            # travels to the host, epochs and zeros between them as for the full result
+            x_in = x_host if x_host.dtype == in_dtype else x_host.astype(in_dtype)
+            res = plan.execute_host_bands(x_in, b_first, b_count, b_weights, epochs=epoch_bounds)
+            self._band_power = res if multichannel else res[0]
+            self._band_frequencies = [frequencies[a:a + c] for a, c in zip(b_first, b_count)]
+        elif pool_width is not None:
             if keep_on_device or out is not None:
                 raise ValueError("'pool_width' cannot be combined with 'keep_on_device' or 'out'")
             if self._output == "complex":
@@ -281,7 +310,13 @@ class ContinuousWaveletTransform(WaveletTransform):
                 _time.time() - start_time, frequencies.size))
 
     # ------------------------------------------------------------------ results
+    def _check_full_rate(self):
+        if self._band_power is not None:
+            raise ValueError("transform(bands=...) kept only band_power; run transform without 'bands' for the "
+                             "full-rate amplitude, power or coefficients")
+
     def _materialise(self):
+        self._check_full_rate()
         if self._host is None:
             if self._result is None:
                 return None
@@ -297,6 +332,7 @@ class ContinuousWaveletTransform(WaveletTransform):
     @property
     def coefficients(self):
         """Complex coefficients (only for ``output='complex'``)."""
+        self._check_full_rate()
         if self._output != "complex":
             raise ValueError("complex coefficients need output='complex'")
         return self._materialise()
@@ -336,6 +372,46 @@ class ContinuousWaveletTransform(WaveletTransform):
     @_amplitude.setter
     def _amplitude(self, val):
         pass
+
+    @property
+    def band_power(self):
+        """Scale-averaged band power of the last ``transform(bands=...)``: (B, N), or (C, B, N) with
+        ``multichannel``; None after a full-rate transform."""
+        return self._band_power
+
+    @property
+    def band_frequencies(self):
+        """The grid frequencies (Hz) of each band of ``band_power``, one array per band."""
+        return self._band_frequencies
+
+    def scale_averaged_power(self, bands, reduce="mean"):
+        """Band power of the existing full-rate result: for every band ``(lo, hi)`` (Hz), the mean
+        (``reduce='mean'``) or sum (``'sum'``) of |W|^2 over the scales whose frequency lies in [lo, hi], at
+        every sample -- what ``transform(bands=...)`` returns.  Shape (B, N), or (C, B, N) with
+        ``multichannel``.  A device-resident result (``keep_on_device=True``) is reduced on the GPU and only the
+        bands are copied back (plan dtype); a host-resident one is reduced in numpy in float64."""
+        from ..engine import band_tables
+        self._check_full_rate()
+        if self._frequencies is None or (self._result is None and self._host is None):
+            raise ValueError("no full-rate result: call transform() first")
+        if self._pooled:
+            raise ValueError("the result was pooled over time (pool_width): band power needs the full-rate result")
+        first, count, weights = band_tables(self._frequencies, bands, reduce)
+        if self._result is not None and self._host is None:
+            res = self.last_plan.band_reduce(self._result, first, count, weights).cpu().numpy()
+        else:
+            data = self._host if self._multichannel else self._host[None]
+            res = np.empty((data.shape[0], first.size, data.shape[2]), dtype=np.float64)
+            off = 0
+            for b, (a, c) in enumerate(zip(first, count)):
+                rows = data[:, a:a + c].astype(np.complex128 if self._output == "complex" else np.float64)
+                if self._output == "complex":
+                    p = np.square(rows.real) + np.square(rows.imag)
+                else:
+                    p = rows if self._output == "power" else np.square(rows)
+                res[:, b] = np.tensordot(weights[off:off + c], p, axes=(0, 1))
+                off += c
+        return res if self._multichannel else res[0]
 
     @property
     def time(self):

@@ -157,6 +157,33 @@ int gcwt_execute_host_pooled(gcwt_plan *plan, const void *x, int32_t in_type,
                              const double *means_host, int64_t pool_width, int32_t pool_mode,
                              double *out, int64_t out_scale_stride, int64_t out_channel_stride);
 
+/* Scale-averaged band power: band power over time (theta, gamma, ripple envelopes) without the full
+ * (channels, scales, samples) result crossing the link.  Band b sums the count[b] adjacent scales starting at
+ * first[b]; its weights are weights[off_b .. off_b + count[b]) with off_b = count[0] + ... + count[b-1]
+ * (1 / count[b] for a mean).  Bands may overlap.  At most 64 bands and 1024 (band, scale) entries.
+ *
+ * gcwt_band_reduce: out[c, b, n] = sum_{k < count[b]} weights[off_b + k] * |W[c, first[b] + k, n]|^2 with fp64
+ *   accumulation, on a device array of kind coef_kind (GCWT_OUT_*: |W|^2 is the square of an amplitude, a
+ *   power as it is, re^2 + im^2 of a complex value); W[c, s, n] at coef_dev[c * channel_stride +
+ *   s * scale_stride + n] in elements of coef_type (float2 / double2 for complex) -> out_dev[c *
+ *   out_channel_stride + b * out_band_stride + n], real elements of coef_type.  Asynchronous on `stream`. */
+int gcwt_band_reduce(const void *coef_dev, int32_t coef_type, int32_t coef_kind,
+                     int64_t n_channels, int64_t n_samples, int64_t scale_stride, int64_t channel_stride,
+                     int32_t n_bands, const int32_t *band_first, const int32_t *band_count, const double *weights,
+                     void *out_dev, int64_t out_band_stride, int64_t out_channel_stride,
+                     int32_t device, void *stream);
+/* gcwt_execute_host, but every tile is band-reduced on the device and only (channels x bands x samples)
+ * travels to `out` (host, plan dtype).  Epochs as gcwt_execute_host.
+ *   out[c * out_channel_stride + b * out_band_stride + t]: float for fp32 plans, double for fp64 plans, whatever
+ *   the plan's out_kind; samples outside all epochs are zero.  The coefficients summed are those
+ *   gcwt_execute_host would have written, accuracy-guard re-computations included. */
+int gcwt_execute_host_bands(gcwt_plan *plan, const void *x, int32_t in_type,
+                            int64_t n_channels, int64_t n_samples, int64_t x_stride,
+                            const int64_t *epoch_bounds, int32_t n_epochs, const double *means_host,
+                            int32_t n_bands, const int32_t *band_first, const int32_t *band_count,
+                            const double *weights,
+                            void *out, int64_t out_band_stride, int64_t out_channel_stride);
+
 /* Diagnostics of the last gcwt_execute_host: out4 = {wall ms, 1 if `out` was pinned (direct DMA) else 0,
  * tiles, bytes copied to the host}. */
 int gcwt_host_stats(const gcwt_plan *plan, double *out4);
