@@ -9,8 +9,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# GCWT_LIB selects an experimental build of the same library (tools/build_variant.sh); never a fallback
-LIB_PATH = os.environ.get("GCWT_LIB") or os.path.join(_HERE, "libghostcwt.so")
+LIB_PATH = os.path.join(_HERE, "libghostcwt.so")
 
 F32, F64 = 0, 1
 OUT_COMPLEX, OUT_AMPLITUDE, OUT_POWER = 0, 1, 2

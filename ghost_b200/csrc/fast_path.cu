@@ -41,8 +41,8 @@ constexpr int kMaxFullScales = 64;
 constexpr double kMaxHaloFrac = 0.45;   // (L-1) / chunk must stay below this
 
 __constant__ float c_halfband[kHalfbandOdd];
-// polyphase taps for the small coarse spacings U = 2, 4, 8 (constant-bank operands of the FMAs)
-constexpr int kSmallCoef = (2 + 4 + 8) * kInterpT;
+// polyphase taps for the small coarse spacings U = 4, 8 (constant-bank operands of the FMAs)
+constexpr int kSmallCoef = (4 + 8) * kInterpT;
 __constant__ float c_interp_small[kSmallCoef];
 // wide-spacing classes: U = 4 (level 2) and U = 8 (level 3), kWideT taps
 constexpr int kWideCoef = (4 + 8) * kWideT;
@@ -272,12 +272,14 @@ int interp_taps(int log2u, int n_taps, double os, float* out) {
     return GCWT_OK;
 }
 
-static int upload_constants(const gcwt_plan* p) {
+static int upload_constants() {
+    double odd[kHalfbandOdd];
+    design_halfband(odd);
     float hb[kHalfbandOdd];
-    for (int k = 0; k < kHalfbandOdd; ++k) hb[k] = (float)p->halfband_odd[k];
+    for (int k = 0; k < kHalfbandOdd; ++k) hb[k] = (float)odd[k];
     GCWT_CUDA_OK(cudaMemcpyToSymbol(c_halfband, hb, sizeof(float) * kHalfbandOdd));
     std::vector<float> all, part;
-    for (int lu = 1; lu <= 3; ++lu) {
+    for (int lu = 2; lu <= 3; ++lu) {
         design_interpolator(lu, part, kInterpT, kInterpMinOs);
         all.insert(all.end(), part.begin(), part.end());
     }
@@ -448,7 +450,6 @@ static int guard_plan_build(gcwt_plan* p, const PlanResponses& pr, const std::ve
 
 int fast_plan_build(gcwt_plan* p) {
     design_halfband(p->halfband_odd);
-    { int rc = upload_constants(p); if (rc) return rc; }
     {
         std::vector<float2> tw(kFullN);
         for (int k = 0; k < kFullN; ++k) {
@@ -503,14 +504,14 @@ int fast_plan_build(gcwt_plan* p) {
             }
             class_geometry(fc);
             if (fc.hop <= 0) { set_error("planner: non-positive hop"); return GCWT_ERR_ARG; }
+            const int ns = (int)fc.scale_ids.size();
             if (fc.wide) {                                        // same margins on the 2x longer chunk
                 const int64_t d = int64_t(1) << level, align = std::max<int64_t>(d, 16), nc2 = 2 * fc.nc_full;
                 const int64_t lead = (int64_t)(kWideT / 2 - 1) << fc.log2u, tail = (int64_t)(kWideT / 2 + 1) << fc.log2u;
                 fc.offset2 = ((fc.lmax / 2 + lead + align - 1) / align) * align;
                 fc.hop2 = ((nc2 - (fc.lmax - 1) / 2 - tail - fc.offset2) / align) * align;
-                const int ns2 = (int)fc.scale_ids.size();
-                std::vector<float2> tab2((size_t)ns2 * 2 * kBins);
-                for (int i = 0; i < ns2; ++i) {
+                std::vector<float2> tab2((size_t)ns * 2 * kBins);
+                for (int i = 0; i < ns; ++i) {
                     const ScaleInfo& sc = p->scales[fc.scale_ids[i]];
                     const double* gsrc = pr.wide2(fc.scale_ids[i], level);
                     for (int m = 0; m < 2 * kBins; ++m) {
@@ -529,43 +530,39 @@ int fast_plan_build(gcwt_plan* p) {
                 }
                 GCWT_CUDA_OK(cudaMalloc((void**)&fc.d_table2, sizeof(float2) * tab2.size()));
                 GCWT_CUDA_OK(cudaMemcpy(fc.d_table2, tab2.data(), sizeof(float2) * tab2.size(), cudaMemcpyHostToDevice));
-            }
-            const int nb = level >= 0 ? kBins : kFullN;
-            const int ns = (int)fc.scale_ids.size();
-            std::vector<float2> tab((size_t)ns * nb);
-            for (int i = 0; i < ns; ++i) {
-                const ScaleInfo& sc = p->scales[fc.scale_ids[i]];
-                const double* gsrc = level >= 0 ? pr.level(fc.scale_ids[i], level) : pr.full(fc.scale_ids[i]);
-                for (int m = 0; m < nb; ++m) {
-                    double g = gsrc[m];
-                    if (level >= 0) {
-                        for (int j = 1; j <= level; ++j) g /= hb[(size_t)j * kBins + m];
-                        g /= (double)kChunkDec;
-                    } else {
-                        g /= (double)kFullN;
+            } else {
+                const int nb = level >= 0 ? kBins : kFullN;
+                std::vector<float2> tab((size_t)ns * nb);
+                for (int i = 0; i < ns; ++i) {
+                    const ScaleInfo& sc = p->scales[fc.scale_ids[i]];
+                    const double* gsrc = level >= 0 ? pr.level(fc.scale_ids[i], level) : pr.full(fc.scale_ids[i]);
+                    for (int m = 0; m < nb; ++m) {
+                        double g = gsrc[m];
+                        if (level >= 0) {
+                            for (int j = 1; j <= level; ++j) g /= hb[(size_t)j * kBins + m];
+                            g /= (double)kChunkDec;
+                        } else {
+                            g /= (double)kFullN;
+                        }
+                        double re = g, im = 0.0;
+                        if ((sc.L & 1) == 0) {
+                            const double ph = -M_PI * (double)m / (double)fc.nc_full;
+                            re = g * std::cos(ph);
+                            im = g * std::sin(ph);
+                        }
+                        tab[(size_t)i * nb + m] = make_float2((float)re, (float)im);
                     }
-                    double re = g, im = 0.0;
-                    if ((sc.L & 1) == 0) {
-                        const double ph = -M_PI * (double)m / (double)fc.nc_full;
-                        re = g * std::cos(ph);
-                        im = g * std::sin(ph);
-                    }
-                    tab[(size_t)i * nb + m] = make_float2((float)re, (float)im);
                 }
-            }
-            GCWT_CUDA_OK(cudaMalloc((void**)&fc.d_table, sizeof(float2) * tab.size()));
-            GCWT_CUDA_OK(cudaMemcpy(fc.d_table, tab.data(), sizeof(float2) * tab.size(), cudaMemcpyHostToDevice));
-            if (fc.interp) {
-                std::vector<float> coef;
-                // per-class taps (spacings U >= 16): fitted to the band this class really occupies
-                if (fc.wide) {
-                    design_interpolator(fc.log2u, coef, kWideT, kWideMinOs);
-                } else {
+                GCWT_CUDA_OK(cudaMalloc((void**)&fc.d_table, sizeof(float2) * tab.size()));
+                GCWT_CUDA_OK(cudaMemcpy(fc.d_table, tab.data(), sizeof(float2) * tab.size(), cudaMemcpyHostToDevice));
+                if (fc.interp) {
+                    // per-class taps (spacings U >= 16): fitted to the band this class really occupies
+                    std::vector<float> coef;
                     const double os = std::min(8.0, std::max(kInterpMinOs, 0.98 * 1024.0 / (double)wmax));
                     design_interpolator(fc.log2u, coef, kInterpT, os);
+                    GCWT_CUDA_OK(cudaMalloc((void**)&fc.d_coef, sizeof(float) * coef.size()));
+                    GCWT_CUDA_OK(cudaMemcpy(fc.d_coef, coef.data(), sizeof(float) * coef.size(), cudaMemcpyHostToDevice));
                 }
-                GCWT_CUDA_OK(cudaMalloc((void**)&fc.d_coef, sizeof(float) * coef.size()));
-                GCWT_CUDA_OK(cudaMemcpy(fc.d_coef, coef.data(), sizeof(float) * coef.size(), cudaMemcpyHostToDevice));
             }
             if (level < 0) {
                 for (int id : fc.scale_ids) fc.scale_nmu.push_back(full_extent(p, pr, id));
@@ -764,11 +761,6 @@ template <> struct out_elem<GCWT_OUT_COMPLEX> { typedef float2 type; };
 // Epilogue (kernel (3)): complex, |W| or |W|^2 of 16 register-resident outputs that lie
 // `stride` elements apart; bit k of `mask` says whether output k is owned by this chunk.
 __device__ __forceinline__ void st_pred(float* p, float v, unsigned on) {
-#ifdef GCWT_EXP_CSSTORE
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %2, 0;\n\t@q st.global.cs.f32 [%0], %1;\n\t}"
-                 :: "l"(p), "f"(v), "r"(on) : "memory");
-    return;
-#endif
     asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %2, 0;\n\t@q st.global.f32 [%0], %1;\n\t}"
                  :: "l"(p), "f"(v), "r"(on) : "memory");
 }
@@ -1118,14 +1110,13 @@ __device__ __forceinline__ void interp_rows(const float* __restrict__ pc, float*
     }
 }
 
-// Small coarse spacings (U = 2, 4, 8): thread <-> coarse interval, all U phases per thread from
-// one register window; taps come from the constant bank; U consecutive outputs leave as one
-// or two 128-bit stores (the launcher guarantees 16-byte aligned rows).
-template <int KIND, int LU>
+// Smallest coarse spacing (U = 4, level 3): thread <-> coarse interval, all U phases per thread
+// from one register window; taps come from the constant bank; the U consecutive outputs leave as
+// one 128-bit store (the launcher guarantees 16-byte aligned rows).
+template <int KIND>
 __device__ __forceinline__ void interp_rows_small(const float* __restrict__ pc, float* __restrict__ row,
                                                   int ia, int ib, int own_hi) {
-    constexpr int U = 1 << LU;
-    constexpr int COFF = (LU == 1) ? 0 : (LU == 2 ? 2 * kInterpT : 6 * kInterpT);
+    constexpr int U = 4;                                          // taps: c_interp_small[0 .. 4 kInterpT)
     for (int iota = ia + (int)threadIdx.x; iota < ib; iota += 256) {
         float w[kInterpT];
 #pragma unroll
@@ -1134,50 +1125,15 @@ __device__ __forceinline__ void interp_rows_small(const float* __restrict__ pc, 
         o[0] = w[kInterpT / 2 - 1];                               // phase 0 sits on a coarse sample
 #pragma unroll
         for (int phi = 1; phi < U; ++phi) {
-            float acc = c_interp_small[COFF + phi * kInterpT] * w[0];
+            float acc = c_interp_small[phi * kInterpT] * w[0];
 #pragma unroll
-            for (int j = 1; j < kInterpT; ++j) acc = fmaf(c_interp_small[COFF + phi * kInterpT + j], w[j], acc);
+            for (int j = 1; j < kInterpT; ++j) acc = fmaf(c_interp_small[phi * kInterpT + j], w[j], acc);
             o[phi] = (KIND == GCWT_OUT_AMPLITUDE) ? sqrt_abs_approx(acc) : fmaxf(acc, 0.f);
         }
         if (KIND == GCWT_OUT_AMPLITUDE) o[0] = sqrt_approx(o[0]);
         float* op = row + (int64_t)iota * U;
         if ((iota + 1) * U <= own_hi) {
-            if (U == 2) *(float2*)op = make_float2(o[0], o[1]);
-            else {
-#pragma unroll
-                for (int v = 0; v < U / 4; ++v) ((float4*)op)[v] = make_float4(o[4 * v], o[4 * v + 1], o[4 * v + 2], o[4 * v + 3]);
-            }
-        } else {
-#pragma unroll
-            for (int phi = 0; phi < U; ++phi) if (iota * U + phi < own_hi) op[phi] = o[phi];
-        }
-    }
-}
-
-// Wide-spacing classes (coarse spacing U = D = 4 or 8, kWideT taps): thread <-> coarse interval,
-// all U phases from one register window, taps from the constant bank, 128-bit stores.
-template <int KIND, int LU>
-__device__ __forceinline__ void interp_rows_wide(const float* __restrict__ pc, float* __restrict__ row,
-                                                 int ia, int ib, int own_hi, bool aligned) {
-    constexpr int U = 1 << LU;
-    constexpr int COFF = (LU == 2) ? 0 : 4 * kWideT;
-    for (int iota = ia + (int)threadIdx.x; iota < ib; iota += 256) {
-        float w[kWideT];
-#pragma unroll
-        for (int j = 0; j < kWideT; ++j) w[j] = pc[iota - (kWideT / 2 - 1) + j];
-        float o[U];
-        o[0] = (KIND == GCWT_OUT_AMPLITUDE) ? sqrt_approx(w[kWideT / 2 - 1]) : w[kWideT / 2 - 1];
-#pragma unroll
-        for (int phi = 1; phi < U; ++phi) {
-            float acc = c_interp_wide[COFF + phi * kWideT] * w[0];
-#pragma unroll
-            for (int j = 1; j < kWideT; ++j) acc = fmaf(c_interp_wide[COFF + phi * kWideT + j], w[j], acc);
-            o[phi] = (KIND == GCWT_OUT_AMPLITUDE) ? sqrt_abs_approx(acc) : fmaxf(acc, 0.f);
-        }
-        float* op = row + (int64_t)iota * U;
-        if (aligned && (iota + 1) * U <= own_hi) {                // rows 16-byte aligned: 128-bit stores
-#pragma unroll
-            for (int v = 0; v < U / 4; ++v) ((float4*)op)[v] = make_float4(o[4 * v], o[4 * v + 1], o[4 * v + 2], o[4 * v + 3]);
+            *(float4*)op = make_float4(o[0], o[1], o[2], o[3]);
         } else {
 #pragma unroll
             for (int phi = 0; phi < U; ++phi) if (iota * U + phi < own_hi) op[phi] = o[phi];
@@ -1191,9 +1147,11 @@ __device__ __forceinline__ void st_v8(float* p, const float* o) {
                  :: "l"(p), "f"(o[0]), "f"(o[1]), "f"(o[2]), "f"(o[3]), "f"(o[4]), "f"(o[5]), "f"(o[6]), "f"(o[7]) : "memory");
 }
 
-// The same with two adjacent coarse intervals per thread: their windows overlap in all but one sample, so the
-// 14 samples arrive as seven 64-bit shared loads (0.22 loads per output at U = 4 instead of 0.75 32-bit ones,
-// 42 % fewer shared-memory wavefronts) and the 2 U outputs leave as 256-bit stores when the rows allow it.
+// Wide-spacing classes (coarse spacing U = D = 4 or 8, kWideT taps from the constant bank): all U phases of a
+// coarse interval from one register window, two adjacent intervals per thread.  Their windows overlap in all but
+// one sample, so the 14 samples arrive as seven 64-bit shared loads (0.22 loads per output at U = 4 instead of
+// 0.75 32-bit ones with one interval per thread, 42 % fewer shared-memory wavefronts) and the 2 U outputs leave
+// as 256-bit stores when the rows allow it.
 // `align`: 0 rows unaligned (scalar stores), 1 16-byte aligned rows, 2 32-byte aligned rows.
 template <int KIND, int LU, int NI>       // NI adjacent coarse intervals per thread (ia must be a multiple of NI, NI even)
 __device__ __forceinline__ void interp_rows_wide_pairs(const float* __restrict__ pc, float* __restrict__ row,
@@ -1241,7 +1199,7 @@ __device__ __forceinline__ void interp_rows_wide_pairs(const float* __restrict__
 template <int KIND>
 __device__ __forceinline__ void interp_rows_pairs8(const float* __restrict__ pc, float* __restrict__ row,
                                                    int ia, int ib, int own_hi, int align) {
-    constexpr int U = 8, COFF = 6 * kInterpT;
+    constexpr int U = 8, COFF = 4 * kInterpT;                                   // behind the U = 4 taps
     static_assert(kInterpT == 8, "window indexing below assumes 8 taps");
     for (int iota = ia + 2 * (int)threadIdx.x; iota < ib; iota += 512) {        // ia is even
         float w[10];                                                            // pc[iota - 4 .. iota + 5]
@@ -1272,7 +1230,7 @@ __device__ __forceinline__ void interp_rows_pairs8(const float* __restrict__ pc,
 }
 
 template <int KIND, bool GUARD>
-__global__ void __launch_bounds__(256, GCWT_INTERP_CTAS)
+__global__ void __launch_bounds__(256, 2)
 fused_interp_kernel(const FusedParams prm) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* ex = (float2*)smem_raw;
@@ -1389,19 +1347,13 @@ fused_interp_kernel(const FusedParams prm) {
             const float* pcs = Pc + sl * PCS;
             float* row = out_c + (int64_t)s_ids[pair + sl] * prm.s_stride;
             if (lu == 2) {
-                interp_rows_small<KIND, 2>(pcs, row, ia, ib, own_hi);
-            } else if (lu == 1) {
-                interp_rows_small<KIND, 1>(pcs, row, ia, ib, own_hi);
+                interp_rows_small<KIND>(pcs, row, ia, ib, own_hi);
             } else {
                 switch (lu) {
-#ifdef GCWT_L4_SLIDING
-                    case 3:  interp_rows<KIND, 3, kInterpT>(pcs, row, prm.coef, c0, lu, ia, ib, own_hi); break;
-#else
                     case 3:
                         if (prm.iters == 2 && prm.units_per_chunk == 1) interp_rows_pairs8<KIND>(pcs, row, ia, ib, own_hi, 2);
                         else interp_rows<KIND, 3, kInterpT>(pcs, row, prm.coef, c0, lu, ia, ib, own_hi);
                         break;
-#endif
                     case 4:  interp_rows<KIND, 4, kInterpT>(pcs, row, prm.coef, c0, lu, ia, ib, own_hi); break;
                     case 5:  interp_rows<KIND, 5, kInterpT>(pcs, row, prm.coef, c0, lu, ia, ib, own_hi); break;
                     case 6:  interp_rows<KIND, 6, kInterpT>(pcs, row, prm.coef, c0, lu, ia, ib, own_hi); break;
@@ -1512,8 +1464,7 @@ fused_wide2_kernel(const FusedParams prm) {
 #pragma unroll
     for (int k = 0; k < 8; ++k) tw2k[k] = tw_pos(prm.twf, 2 * tid * k);        // e^{2 pi i m' k / 2048}
     float* const out_c = (float*)prm.out + c * prm.c_stride + t0;
-    const bool aligned = prm.iters != 0;                           // rows 16-byte aligned: 128-bit stores allowed
-    const int align = prm.iters;                                   // 2: 32-byte aligned rows (256-bit stores)
+    const int align = prm.iters;                                   // 1: 16-byte, 2: 32-byte aligned rows (128- / 256-bit stores)
     float2* const A = B1;
     float2* const ex = B0;
     float* const Pc = (float*)B1;
@@ -1573,15 +1524,9 @@ fused_wide2_kernel(const FusedParams prm) {
         for (int sl = 0; sl < 2 && pair + sl < prm.n_scales; ++sl) {
             const float* pcs = Pc + sl * kPcStride;
             float* row = out_c + (int64_t)s_ids[pair + sl] * prm.s_stride;
-#ifdef GCWT_WIDE_SINGLE
-            if (lu == 2) interp_rows_wide<KIND, 2>(pcs, row, ia, ib, own_hi, aligned);
-            else interp_rows_wide<KIND, 3>(pcs, row, ia, ib, own_hi, aligned);
-#else
-            (void)aligned;
             // (four intervals per thread at U = 4 measured slower: 1.99 vs 1.88 ms on level 2 of config 2)
             if (lu == 2) interp_rows_wide_pairs<KIND, 2, 2>(pcs, row, ia, ib, own_hi, align);
             else interp_rows_wide_pairs<KIND, 3, 2>(pcs, row, ia, ib, own_hi, align);
-#endif
         }
         __syncthreads();
     }
@@ -1624,18 +1569,12 @@ __device__ __forceinline__ void full_scale_loop(const FusedParams& prm, const fl
         // the issue slots, not by this latency -- staging the rows ahead of time changed nothing
         // measurable, neither with cp.async (a second LSU operation per entry) nor with a TMA bulk
         // copy + mbarrier one scale ahead (8.89 vs 8.92 ms on config 2)
-#ifdef GCWT_EXP_TABLE0
-        const float2* tab = prm.table + tid;                         // what-if: every scale reads the same (L1-hot) row
-#else
         const float2* tab = prm.table + (int64_t)s * kFullN + tid;
-#endif
         if (nmu == 2) full_prepass<2>(Yf, tab, A, tw4k);
         else if (nmu == 4) full_prepass<4>(Yf, tab, A, tw4k);
         else if (nmu == 8) full_prepass<8>(Yf, tab, A, tw4k);
         else full_prepass<16>(Yf, tab, A, tw4k);
-#ifndef GCWT_EXP_NOBAR
         __syncthreads();
-#endif
         if (MEASURE && s > 0 && tid == 0) {                          // every add for scale s - 1 came before this barrier
             atomicAdd(prm.pow + (blockIdx.x / prm.n_chunks) * prm.pow_stride + s_ids[s - 1], s_pow[(s - 1) & 1] * prm.pow_weight);
             s_pow[(s - 1) & 1] = 0.f;
@@ -1648,44 +1587,12 @@ __device__ __forceinline__ void full_scale_loop(const FusedParams& prm, const fl
         e[0] = a[0];
 #pragma unroll
         for (int k = 1; k < 16; ++k) e[k * 16] = cmul(a[k], tw[k]);
-#ifndef GCWT_EXP_NOBAR
         __syncthreads();
-#endif
         const float2* e2 = ex + g * 16 + r;
 #pragma unroll
         for (int k = 0; k < 16; ++k) a[k] = e2[k * 256];
-#ifndef GCWT_EXP_NOPASS2
         dft16<+1>(a);
-#endif
-#ifdef GCWT_EXP_NOSTORE
-        store_column<KIND>(out_c + (int64_t)s_ids[s] * prm.s_stride + rel, 256, mask & 1u, a);
-#elif defined(GCWT_EXP_HALFSTORE)
-        store_column<KIND>(out_c + (int64_t)s_ids[s] * prm.s_stride + rel, 256, mask & 0x5555u, a);     // what-if: 8 of the 16 stores
-#elif defined(GCWT_EXP_B16STORE)
-        {   // what-if: 16 stores of 2 bytes each (same requests, half the sectors)
-            unsigned short* o16 = (unsigned short*)(out_c + (int64_t)s_ids[s] * prm.s_stride) + rel;
-#pragma unroll
-            for (int k = 0; k < 16; ++k)
-                if (mask & (1u << k)) o16[k * 512] = (unsigned short)__float_as_uint(a[k].x * a[k].x + a[k].y * a[k].y);
-        }
-#elif defined(GCWT_EXP_V2STORE)
-        {   // what-if: the same bytes as 8 stores of 8 bytes (lanes consecutive): per-request or per-byte cost?
-            float2* o2 = (float2*)(out_c + (int64_t)s_ids[s] * prm.s_stride) + rel;
-#pragma unroll
-            for (int k = 0; k < 16; k += 2)
-                if (mask & (1u << k)) o2[(k >> 1) * 256] = make_float2(a[k].x * a[k].x + a[k].y * a[k].y, a[k + 1].x * a[k + 1].x + a[k + 1].y * a[k + 1].y);
-        }
-#elif defined(GCWT_EXP_STSSTORE)
-        {   // what-if: the 16 results go to shared memory instead (as a TMA bulk store would need); Yf is clobbered
-            float* stage = (float*)const_cast<float2*>(Yf);
-#pragma unroll
-            for (int k = 0; k < 16; ++k) stage[k * 256 + rel] = sqrt_approx(a[k].x * a[k].x + a[k].y * a[k].y);
-        }
-#elif defined(GCWT_EXP_L2STORE)
-        store_column<KIND>((typename out_elem<KIND>::type*)prm.out + (blockIdx.x & 255) * 4096 + rel, 256, mask, a);   // what-if: L2-resident target
-#else
         store_column<KIND>(out_c + (int64_t)s_ids[s] * prm.s_stride + rel, 256, mask, a);
-#endif
         if (MEASURE) guard_pow_add<false>(a, mask, s_pow + (s & 1));
         // no trailing barrier: the next scale's pre-pass writes A, whose readers all passed
         // the second barrier above; its pass 1 writes ex only after the next first barrier,
@@ -1761,60 +1668,21 @@ fused_full_kernel(const FusedParams prm) {
 }
 
 // ============================================================================ driver
-template <int KIND, int LP, bool GUARD>
-static void launch_banded_g(unsigned nblk, cudaStream_t st, const FusedParams& prm) {
-    static std::atomic<bool> attr_set[64];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev & 63]) {
-        cudaFuncSetAttribute(fused_banded_kernel<KIND, LP, GUARD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBandedSmem);
-        attr_set[dev & 63] = true;
-    }
-    fused_banded_kernel<KIND, LP, GUARD><<<nblk, 256, kBandedSmem, st>>>(prm);
-}
+template <int V> using IntC = std::integral_constant<int, V>;
 
-template <int KIND, int LP>
-static void launch_banded_one(unsigned nblk, cudaStream_t st, const FusedParams& prm) {
-    if (prm.pow != nullptr) launch_banded_g<KIND, LP, true>(nblk, st, prm);
-    else launch_banded_g<KIND, LP, false>(nblk, st, prm);
-}
-
-static void launch_banded(int kind, int lp, unsigned nblk, cudaStream_t st, const FusedParams& prm) {
-    if (kind == GCWT_OUT_COMPLEX) {
-        if (lp == 4) launch_banded_one<GCWT_OUT_COMPLEX, 4>(nblk, st, prm);
-        else launch_banded_one<GCWT_OUT_COMPLEX, 0>(nblk, st, prm);
-    } else if (kind == GCWT_OUT_AMPLITUDE) {
-        if (lp == 4) launch_banded_one<GCWT_OUT_AMPLITUDE, 4>(nblk, st, prm);
-        else launch_banded_one<GCWT_OUT_AMPLITUDE, 0>(nblk, st, prm);
-    } else {
-        if (lp == 4) launch_banded_one<GCWT_OUT_POWER, 4>(nblk, st, prm);
-        else launch_banded_one<GCWT_OUT_POWER, 0>(nblk, st, prm);
-    }
-}
-
-template <typename TIn, int KIND, bool GUARD>
-static void launch_full_g(unsigned nblk, cudaStream_t st, const FusedParams& prm) {
-    static std::atomic<bool> attr_set[64];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev & 63]) {
-        cudaFuncSetAttribute(fused_full_kernel<TIn, KIND, GUARD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFullSmem);
-        attr_set[dev & 63] = true;
-    }
-    fused_full_kernel<TIn, KIND, GUARD><<<nblk, 256, kFullSmem, st>>>(prm);
-}
-
-template <typename TIn, int KIND>
-static void launch_full_kind(unsigned nblk, cudaStream_t st, const FusedParams& prm, bool measure) {
-    if (measure) launch_full_g<TIn, KIND, true>(nblk, st, prm);
-    else launch_full_g<TIn, KIND, false>(nblk, st, prm);
-}
-
-template <typename TIn>
-static void launch_full(int kind, unsigned nblk, cudaStream_t st, const FusedParams& prm, bool measure) {
-    if (kind == GCWT_OUT_COMPLEX) launch_full_kind<TIn, GCWT_OUT_COMPLEX>(nblk, st, prm, measure);
-    else if (kind == GCWT_OUT_AMPLITUDE) launch_full_kind<TIn, GCWT_OUT_AMPLITUDE>(nblk, st, prm, measure);
-    else launch_full_kind<TIn, GCWT_OUT_POWER>(nblk, st, prm, measure);
+// The one place where a run-time output kind and guard flag become template arguments of the fused kernels:
+// calls f(IntC<KIND>(), std::integral_constant<bool, GUARD>()).  COMPLEX = false for the interpolating
+// kernels, which have no complex-output instance.
+template <bool COMPLEX, typename F>
+static void with_kind_guard(int kind, bool guard, const F& f) {
+    const auto with_guard = [&](auto k) {
+        if (guard) f(k, std::true_type());
+        else f(k, std::false_type());
+    };
+    if constexpr (COMPLEX)
+        if (kind == GCWT_OUT_COMPLEX) return with_guard(IntC<GCWT_OUT_COMPLEX>());
+    if (kind == GCWT_OUT_AMPLITUDE) with_guard(IntC<GCWT_OUT_AMPLITUDE>());
+    else with_guard(IntC<GCWT_OUT_POWER>());
 }
 
 struct LevelGeom { int64_t lo, hi, len, stride; float* ptr; };
@@ -1880,14 +1748,14 @@ static int fast_run(gcwt_plan* p, const TIn* x, int in_type, int64_t n_channels,
     GCWT_CUDA_OK(cudaGetLastError());
 
     // ---- fused kernels ---------------------------------------------------------------
-    // the thread <-> interval interpolators of fused_interp_kernel (U = 2, 4) write 128-bit vectors:
+    // the thread <-> interval interpolator of fused_interp_kernel at U = 4 writes 128-bit vectors:
     // rows must be 16-byte aligned, else the class falls back to the direct kernel
     const bool rows_aligned = ((uintptr_t)out % 16 == 0) && (s_stride % 4 == 0) && (c_stride % 4 == 0);
     const bool rows_aligned32 = ((uintptr_t)out % 32 == 0) && (s_stride % 8 == 0) && (c_stride % 8 == 0);
     auto uses_interp = [&](const FastClass& fc) {
         if (fc.level < 0 || !fc.interp) return false;
-        if (fc.wide && fc.d_table2) return true;                  // fused_wide2_kernel stores scalars when it must
-        return (fc.log2u >= 3 && !fc.wide) || rows_aligned;
+        if (fc.wide) return true;                                 // fused_wide2_kernel stores scalars when it must
+        return fc.log2u >= 3 || rows_aligned;
     };
     cudaStream_t full_meas_stream = nullptr;      // guard: where the measured chunks of the full-spectrum class run
     auto launch_class = [&](const FastClass& fc, cudaStream_t cs, bool own_span) -> int {
@@ -1917,7 +1785,7 @@ static int fast_run(gcwt_plan* p, const TIn* x, int in_type, int64_t n_channels,
         };
         set_guard_sampling(prm.n_chunks, fc.level >= 0 ? 8 : 16,
                            (double)(fc.level >= 0 ? (int64_t(1) << fc.level) : 1) * (double)fc.hop / (double)fc.nc_full);
-        if (fc.level >= 0 && fc.interp && fc.wide && fc.d_table2) {
+        if (fc.wide) {
             const LevelGeom& g = lv[fc.level];
             prm.src = g.ptr; prm.src_stride = g.stride; prm.src_lo = g.lo; prm.src_hi = g.hi;
             prm.log2d = fc.level;
@@ -1929,13 +1797,9 @@ static int fast_run(gcwt_plan* p, const TIn* x, int in_type, int64_t n_channels,
             prm.iters = rows_aligned32 ? 2 : (rows_aligned ? 1 : 0);   // 256-bit / 128-bit stores allowed
             const int64_t nblk = n_channels * prm.n_chunks;
             if (nblk > 0x7fffffffLL) { set_error("fast path: grid too large"); return GCWT_ERR_UNSUPPORTED; }
-            if (p->out_kind == GCWT_OUT_AMPLITUDE) {
-                if (guard) fused_wide2_kernel<GCWT_OUT_AMPLITUDE, true><<<(unsigned)nblk, 256, kWide2Smem, cs>>>(prm);
-                else fused_wide2_kernel<GCWT_OUT_AMPLITUDE, false><<<(unsigned)nblk, 256, kWide2Smem, cs>>>(prm);
-            } else {
-                if (guard) fused_wide2_kernel<GCWT_OUT_POWER, true><<<(unsigned)nblk, 256, kWide2Smem, cs>>>(prm);
-                else fused_wide2_kernel<GCWT_OUT_POWER, false><<<(unsigned)nblk, 256, kWide2Smem, cs>>>(prm);
-            }
+            with_kind_guard<false>(p->out_kind, guard, [&](auto K, auto G) {
+                fused_wide2_kernel<K, G><<<(unsigned)nblk, 256, kWide2Smem, cs>>>(prm);
+            });
         } else if (uses_interp(fc)) {
             const LevelGeom& g = lv[fc.level];
             prm.src = g.ptr; prm.src_stride = g.stride; prm.src_lo = g.lo; prm.src_hi = g.hi;
@@ -1953,13 +1817,9 @@ static int fast_run(gcwt_plan* p, const TIn* x, int in_type, int64_t n_channels,
             prm.units_per_chunk = (int)splits;
             const int64_t nblk = chunks * splits;
             if (nblk > 0x7fffffffLL) { set_error("fast path: grid too large"); return GCWT_ERR_UNSUPPORTED; }
-            if (p->out_kind == GCWT_OUT_AMPLITUDE) {
-                if (guard) fused_interp_kernel<GCWT_OUT_AMPLITUDE, true><<<(unsigned)nblk, 256, kInterpSmem, cs>>>(prm);
-                else fused_interp_kernel<GCWT_OUT_AMPLITUDE, false><<<(unsigned)nblk, 256, kInterpSmem, cs>>>(prm);
-            } else {
-                if (guard) fused_interp_kernel<GCWT_OUT_POWER, true><<<(unsigned)nblk, 256, kInterpSmem, cs>>>(prm);
-                else fused_interp_kernel<GCWT_OUT_POWER, false><<<(unsigned)nblk, 256, kInterpSmem, cs>>>(prm);
-            }
+            with_kind_guard<false>(p->out_kind, guard, [&](auto K, auto G) {
+                fused_interp_kernel<K, G><<<(unsigned)nblk, 256, kInterpSmem, cs>>>(prm);
+            });
         } else if (fc.level >= 0) {
             const LevelGeom& g = lv[fc.level];
             prm.src = g.ptr; prm.src_stride = g.stride; prm.src_lo = g.lo; prm.src_hi = g.hi;
@@ -1971,24 +1831,32 @@ static int fast_run(gcwt_plan* p, const TIn* x, int in_type, int64_t n_channels,
             prm.units_per_chunk = (blocks + prm.iters - 1) / prm.iters;
             const int64_t nblk = n_channels * prm.n_chunks * prm.units_per_chunk;
             if (nblk > 0x7fffffffLL) { set_error("fast path: grid too large"); return GCWT_ERR_UNSUPPORTED; }
-            launch_banded(p->out_kind, prm.log2p, (unsigned)nblk, cs, prm);
+            with_kind_guard<true>(p->out_kind, guard, [&](auto K, auto G) {
+                if (prm.log2p == 4) fused_banded_kernel<K, 4, G><<<(unsigned)nblk, 256, kBandedSmem, cs>>>(prm);
+                else fused_banded_kernel<K, 0, G><<<(unsigned)nblk, 256, kBandedSmem, cs>>>(prm);
+            });
         } else {
             prm.src = x; prm.src_stride = x_stride; prm.src_lo = -halo_l; prm.src_hi = n + halo_r;
             prm.log2d = 0; prm.p_cols = 16; prm.log2p = 4; prm.iters = 1; prm.units_per_chunk = 1;
             const int64_t nblk = n_channels * prm.n_chunks;
             if (nblk > 0x7fffffffLL) { set_error("fast path: grid too large"); return GCWT_ERR_UNSUPPORTED; }
+            const auto launch_full = [&](cudaStream_t fs, bool measure) {
+                with_kind_guard<true>(p->out_kind, measure, [&](auto K, auto G) {
+                    fused_full_kernel<TIn, K, G><<<(unsigned)(n_channels * prm.n_chunks), 256, kFullSmem, fs>>>(prm);
+                });
+            };
             if (!guard) {
-                launch_full<TIn>(p->out_kind, (unsigned)nblk, cs, prm, false);
+                launch_full(cs, false);
             } else {
                 // measured chunks (every guard_every-th) and the others in two launches of two kernels
                 const int64_t n_all = prm.n_chunks, n_meas = (n_all + prm.guard_every - 1) / prm.guard_every;
                 if (n_all > n_meas) {
                     prm.q_mode = 2; prm.n_chunks = n_all - n_meas;
-                    launch_full<TIn>(p->out_kind, (unsigned)(n_channels * prm.n_chunks), cs, prm, false);
+                    launch_full(cs, false);
                     count_launch();
                 }
                 prm.q_mode = prm.guard_every > 1 ? 1 : 0; prm.n_chunks = n_meas;
-                launch_full<TIn>(p->out_kind, (unsigned)(n_channels * prm.n_chunks), full_meas_stream ? full_meas_stream : cs, prm, true);
+                launch_full(full_meas_stream ? full_meas_stream : cs, true);
             }
         }
         count_launch();
@@ -2167,33 +2035,40 @@ int guard_resolve(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, 
     return GCWT_OK;
 }
 
-static std::atomic<bool> g_attr_done[64];
+// Once per device: the dynamic shared-memory limit of every fused-kernel instance fast_run can launch, and the
+// filter taps in constant memory (which is per device; the taps do not depend on the plan).
+static std::atomic<bool> g_device_ready[64];
 
-template <typename TIn>
-static int set_smem_attrs() {
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_interp_kernel<GCWT_OUT_AMPLITUDE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInterpSmem));
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_interp_kernel<GCWT_OUT_POWER, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInterpSmem));
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_wide2_kernel<GCWT_OUT_AMPLITUDE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWide2Smem));
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_wide2_kernel<GCWT_OUT_POWER, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWide2Smem));
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_interp_kernel<GCWT_OUT_AMPLITUDE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInterpSmem));
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_interp_kernel<GCWT_OUT_POWER, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInterpSmem));
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_wide2_kernel<GCWT_OUT_AMPLITUDE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWide2Smem));
-    GCWT_CUDA_OK(cudaFuncSetAttribute(fused_wide2_kernel<GCWT_OUT_POWER, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWide2Smem));
+static int prepare_device(int device) {
+    if (g_device_ready[device & 63]) return GCWT_OK;
+    cudaError_t e = cudaSuccess;
+    const auto smem = [&](auto kernel, size_t bytes) {
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    };
+    for (int kind = GCWT_OUT_COMPLEX; kind <= GCWT_OUT_POWER; ++kind)
+        for (bool guard : {false, true})
+            with_kind_guard<true>(kind, guard, [&](auto K, auto G) {
+                smem(fused_banded_kernel<K, 0, G>, kBandedSmem);
+                smem(fused_banded_kernel<K, 4, G>, kBandedSmem);
+                smem(fused_full_kernel<float, K, G>, kFullSmem);
+                smem(fused_full_kernel<double, K, G>, kFullSmem);
+                if constexpr (K != GCWT_OUT_COMPLEX) {
+                    smem(fused_interp_kernel<K, G>, kInterpSmem);
+                    smem(fused_wide2_kernel<K, G>, kWide2Smem);
+                }
+            });
+    if (e != cudaSuccess) { set_error(std::string("fused kernels: shared-memory limit: ") + cudaGetErrorString(e)); return GCWT_ERR_CUDA; }
+    int rc = upload_constants();
+    if (rc) return rc;
+    g_device_ready[device & 63] = true;
     return GCWT_OK;
 }
 
 int fast_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n_samples,
                  int64_t x_stride, int64_t halo_l, int64_t halo_r, const double* d_means, void* out,
                  int64_t s_stride, int64_t c_stride, cudaStream_t st) {
-    const int slot = (p->device & 31) * 2 + (in_type == GCWT_F32 ? 0 : 1);
-    if (!g_attr_done[slot]) {
-        int rc = in_type == GCWT_F32 ? set_smem_attrs<float>() : set_smem_attrs<double>();
-        if (rc) return rc;
-        // constant memory is per device: (re)load the filter taps
-        rc = upload_constants(p);
-        if (rc) return rc;
-        g_attr_done[slot] = true;
-    }
+    int rc = prepare_device(p->device);
+    if (rc) return rc;
     if (in_type == GCWT_F32)
         return fast_run<float>(p, (const float*)x, in_type, n_channels, n_samples, x_stride, halo_l, halo_r,
                                d_means, out, s_stride, c_stride, st);

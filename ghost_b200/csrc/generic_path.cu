@@ -308,7 +308,7 @@ static int generic_run(gcwt_plan* p, const std::vector<int>& ids, const TIn* x, 
     else nfft = std::max<int64_t>(int64_t(1) << 17, int64_t(1) << ilog2_ceil(4 * lmax));
     if (nfft > (int64_t(1) << 26)) { set_error("generic path: kernel too long"); return GCWT_ERR_UNSUPPORTED; }
     if (nfft < 16) nfft = 16;
-    if (std::is_same<T, double>::value && FourStep::usable(nfft) && !getenv("GCWT_F64_LEGACY"))
+    if (std::is_same<T, double>::value && FourStep::usable(nfft))
         return generic_run_fourstep<TIn, TOut>(p, ids, x, n_channels, n, x_stride, halo_l, halo_r, d_means, out, s_stride,
                                                c_stride, st, nfft, lmax);
     const int64_t offset = lmax / 2;

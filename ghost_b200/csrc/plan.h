@@ -10,24 +10,12 @@ namespace gcwt {
 constexpr int kBins = 256;          // spectrum bins kept per chunk by the band-limited path
 constexpr int kChunkDec = 1024;     // chunk length in decimated samples (forward FFT size)
 constexpr int kFullN = 4096;        // chunk length of the full-spectrum fused kernel
-#ifndef GCWT_MAX_CLASS
-#define GCWT_MAX_CLASS 16
-#endif
-#ifndef GCWT_INTERP_T
-#define GCWT_INTERP_T 8
-#endif
-#ifndef GCWT_WIDE_T
-#define GCWT_WIDE_T 12
-#endif
-#ifndef GCWT_INTERP_CTAS
-#define GCWT_INTERP_CTAS 2
-#endif
-constexpr int kMaxClassScales = GCWT_MAX_CLASS; // scales handled by one fused launch (shared-memory table)
+constexpr int kMaxClassScales = 16; // scales handled by one fused launch (shared-memory table)
 constexpr int kMinFastLevel = 2;    // P = kChunkDec * 2^level / kBins must be >= 16
-constexpr int kInterpT = GCWT_INTERP_T;        // taps of the polyphase interpolator (amplitude / power output)
+constexpr int kInterpT = 8;         // taps of the polyphase interpolator (amplitude / power output)
 constexpr int kInterpMinLevel = 3;  // interpolated classes: coarse spacing U = 2^(level-1) >= 4
 constexpr int kCoarse = 2048;       // coarse |W|^2 samples per chunk and scale (8 columns x 256)
-constexpr int kWideT = GCWT_WIDE_T;          // taps of the interpolator of the wide-spacing classes (U = D)
+constexpr int kWideT = 12;          // taps of the interpolator of the wide-spacing classes (U = D)
 constexpr int kWideMaxLevel = 3;    // levels 2 and 3 use U = D when their bands allow it
 constexpr double kInterpMinOs = 4.0; // |W|^2 over-sampling guaranteed on the grid U = D/2 (band <= kBins bins)
 constexpr double kWideMinOs = 2.5;   // over-sampling required of a class before it may use U = D
@@ -51,16 +39,17 @@ struct FastClass {
     std::vector<int> scale_ids;     // global scale indices, <= kMaxClassScales
     // banded: float2 [n][kBins] (response / decimator, incl. 1/kChunkDec)
     // full:   float2 [n][kFullN] (response incl. 1/kFullN)
+    // (null for wide classes, which read d_table2)
     float2* d_table = nullptr;
     int32_t* d_scale_ids = nullptr;
     // amplitude / power at level >= kInterpMinLevel: |W|^2 on a grid of spacing U = 2^log2u,
-    // then a kInterpT-tap polyphase interpolator; d_coef is float [U][kInterpT]
+    // then a kInterpT-tap polyphase interpolator; d_coef is float [U][kInterpT] (not wide classes)
     std::vector<int> scale_nmu;     // full-spectrum kernel: occupied 256-bin blocks per scale (2, 4, 8, 16)
     int32_t* d_scale_nmu = nullptr;
     bool interp = false;
     bool wide = false;              // coarse spacing U = D (4 columns), kWideT taps; else U = D/2, kInterpT taps
-    // wide classes with 16-byte aligned rows run on chunks of 2 * kChunkDec decimated samples with
-    // 2 * kBins bins kept (fused_wide2_kernel): own table [n][2 kBins] and overlap-save geometry
+    // wide classes run on chunks of 2 * kChunkDec decimated samples with 2 * kBins bins kept
+    // (fused_wide2_kernel): own table [n][2 kBins] and overlap-save geometry
     float2* d_table2 = nullptr;
     int64_t offset2 = 0, hop2 = 0;
     int log2u = 0;
