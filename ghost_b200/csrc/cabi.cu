@@ -67,6 +67,24 @@ int ensure_workspace(gcwt_plan* p, size_t bytes) {
     return GCWT_OK;
 }
 
+static int grow(void** ptr, size_t* have, size_t need, bool pinned, const char* who) {
+    if (*have >= need) return GCWT_OK;
+    if (*ptr) pinned ? cudaFreeHost(*ptr) : cudaFree(*ptr);
+    *ptr = nullptr; *have = 0;
+    const cudaError_t e = pinned ? cudaMallocHost(ptr, need) : cudaMalloc(ptr, need);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        set_error(std::string(who) + (pinned ? ": pinned" : ": device") + " allocation of " + std::to_string(need) +
+                  " bytes: " + cudaGetErrorString(e));
+        return GCWT_ERR_NOMEM;
+    }
+    *have = need;
+    return GCWT_OK;
+}
+
+int grow_device(void** ptr, size_t* have, size_t need, const char* who) { return grow(ptr, have, need, false, who); }
+int grow_pinned(void** ptr, size_t* have, size_t need, const char* who) { return grow(ptr, have, need, true, who); }
+
 int filter_response_device(int64_t L, int k_first, int n_terms, const double* terms_host, int64_t nfft,
                            int64_t first_bin, int64_t n_bins, double* out_host);
 
@@ -273,29 +291,19 @@ int gcwt_execute(gcwt_plan* p, const void* x, int32_t in_type, int64_t n_channel
     cudaStream_t st = (cudaStream_t)stream;
     const double* d_means = means;
     if (!d_means) {
-        if (p->means_cap < n_channels) {
-            if (p->d_means) cudaFree(p->d_means);
-            p->d_means = nullptr; p->means_cap = 0;
-            GCWT_CUDA_OK(cudaMalloc((void**)&p->d_means, sizeof(double) * n_channels));
-            p->means_cap = n_channels;
-        }
-        const int64_t need = (int64_t)means_blocks(n_samples) * n_channels;
-        if (p->partial_cap < need) {
-            if (p->d_partial) cudaFree(p->d_partial);
-            p->d_partial = nullptr; p->partial_cap = 0;
-            GCWT_CUDA_OK(cudaMalloc((void**)&p->d_partial, sizeof(double) * need));
-            p->partial_cap = need;
-        }
+        rc = grow_device((void**)&p->d_means, &p->means_bytes, sizeof(double) * n_channels, "execute");
+        if (rc == GCWT_OK)
+            rc = grow_device((void**)&p->d_partial, &p->partial_bytes, sizeof(double) * means_blocks(n_samples) * n_channels, "execute");
+        if (rc) return rc;
         const int sp = prof_begin(p, 0, st);
         rc = means_launch(x, in_type, n_channels, n_samples, x_stride, p->d_means, p->d_partial, st);
         prof_end(p, sp, st);
         if (rc) return rc;
         d_means = p->d_means;
     }
-    // the two drivers share one workspace: size it for the larger user up front is not
-    // needed because they run back to back on the same stream and each re-derives its
-    // layout from the base pointer; growing between them would free memory still in use,
-    // so run the generic part first only after synchronising a grown workspace.
+    // The fused kernels keep their pyramid in the plan's workspace, and the guard's fp64 re-computation lays out its
+    // own buffers there.  The generic scales reuse the workspace too, and ensure_workspace may free it to grow it, so
+    // the generic part starts only once the work queued on `st` (side streams joined) is done with it.
     if (p->compute_type == GCWT_F32 && !p->classes.empty()) {
         rc = fast_execute(p, x, in_type, n_channels, n_samples, x_stride, halo_left, halo_right, d_means,
                           out, out_scale_stride, out_channel_stride, st);
@@ -323,10 +331,8 @@ int gcwt_execute_host(gcwt_plan* p, const void* x, int32_t in_type, int64_t n_ch
     if (rc) return rc;
     if (out_scale_stride < n_samples) { set_error("execute_host: out_scale_stride smaller than n_samples"); return GCWT_ERR_ARG; }
     DeviceScope dev_scope(p->device);
-    int64_t tile_hint = 0;
-    if (const char* e = getenv("GCWT_HOST_TILE")) tile_hint = atoll(e);       // developer aid: force the time tile
     return host_execute(p, x, in_type, n_channels, n_samples, x_stride, epoch_bounds, n_epochs, means_host, out,
-                        out_scale_stride, out_channel_stride, tile_hint);
+                        out_scale_stride, out_channel_stride);
 }
 
 int gcwt_execute_host_pooled(gcwt_plan* p, const void* x, int32_t in_type, int64_t n_channels, int64_t n_samples,
@@ -337,10 +343,8 @@ int gcwt_execute_host_pooled(gcwt_plan* p, const void* x, int32_t in_type, int64
     if (pool_width < 1 || (pool_mode != GCWT_POOL_MEAN && pool_mode != GCWT_POOL_MAX)) { set_error("execute_host_pooled: bad pool_width / pool_mode"); return GCWT_ERR_ARG; }
     if (out_scale_stride < (n_samples + pool_width - 1) / pool_width) { set_error("execute_host_pooled: out_scale_stride smaller than the bin count"); return GCWT_ERR_ARG; }
     DeviceScope dev_scope(p->device);
-    int64_t tile_hint = 0;
-    if (const char* e = getenv("GCWT_HOST_TILE")) tile_hint = atoll(e);
     return host_execute(p, x, in_type, n_channels, n_samples, x_stride, nullptr, 0, means_host, out, out_scale_stride,
-                        out_channel_stride, tile_hint, pool_width, pool_mode);
+                        out_channel_stride, pool_width, pool_mode);
 }
 
 int gcwt_pool_rows(const void* x_dev, int32_t type, int64_t n_rows, int64_t n_cols, int64_t row_stride, int64_t pool_width,
@@ -391,10 +395,8 @@ int gcwt_execute_host_bands(gcwt_plan* p, const void* x, int32_t in_type, int64_
         set_error("execute_host_bands: out_band_stride below n_samples, or out_channel_stride below n_bands rows"); return GCWT_ERR_ARG;
     }
     DeviceScope dev_scope(p->device);
-    int64_t tile_hint = 0;
-    if (const char* e = getenv("GCWT_HOST_TILE")) tile_hint = atoll(e);
     return host_execute(p, x, in_type, n_channels, n_samples, x_stride, epoch_bounds, n_epochs, means_host, out,
-                        out_band_stride, out_channel_stride, tile_hint, 0, 0, &tab);
+                        out_band_stride, out_channel_stride, 0, 0, &tab);
 }
 
 int gcwt_host_stats(const gcwt_plan* p, double* out4) {

@@ -110,12 +110,12 @@ struct gcwt_plan {
     int64_t prof_launches[GCWT_PROFILE_KINDS] = {0, 0, 0, 0, 0};
     float2* d_twiddle = nullptr;            // e^{-2 pi i k / 4096}, k < 4096 (forward FFTs of the fused kernels)
     double* d_means = nullptr;              // internal per-channel means
-    int64_t means_cap = 0;
+    size_t means_bytes = 0;
     static constexpr int kSideStreams = 3;
     cudaStream_t side_stream[kSideStreams] = {nullptr, nullptr, nullptr};   // forked streams of the interpolated classes
     cudaEvent_t ev_fork = nullptr, ev_join[kSideStreams] = {nullptr, nullptr, nullptr};
     double* d_partial = nullptr;            // scratch of the mean reduction
-    int64_t partial_cap = 0;
+    size_t partial_bytes = 0;
     // accuracy guard: plan-time tables (per scale) and per-execute accumulators (per channel)
     bool guard = false;
     double guard_tol = 5e-6;
@@ -137,13 +137,13 @@ struct gcwt_plan {
     int64_t tw_fine_n = 0;
     double2* d_hcache = nullptr;            // [n_scales][nfft]
     int64_t hcache_n = 0;
-    // host-buffer path (gcwt_execute_host): persistent staging, grown on demand
+    // host-buffer path (gcwt_execute_host*): persistent staging, grown on demand
     struct HostStage {
-        void* d_in = nullptr; size_t in_bytes = 0;           // the channel group's samples
-        void* d_out[2] = {nullptr, nullptr}; size_t out_bytes = 0;   // double-buffered result tiles
-        void* h_ring[2] = {nullptr, nullptr}; size_t ring_bytes = 0; // pinned bounce buffers (pageable destinations only)
-        void* d_pool[2] = {nullptr, nullptr}; void* h_pool[2] = {nullptr, nullptr}; size_t pool_bytes = 0;   // pooled / band-reduced tiles
-        double* d_means = nullptr; int64_t means_cap = 0;
+        void* d_in = nullptr; size_t in_bytes = 0;                            // the channel group's samples
+        void* d_out[2] = {nullptr, nullptr}; size_t out_bytes[2] = {0, 0};    // double-buffered full-rate tiles
+        void* d_red[2] = {nullptr, nullptr}; size_t red_bytes[2] = {0, 0};    // reduced tiles: pooled bins or band rows
+        void* h_ring[2] = {nullptr, nullptr}; size_t ring_bytes[2] = {0, 0};  // pinned ring (pageable destinations only)
+        double* d_means = nullptr; size_t means_bytes = 0;
         cudaStream_t st_compute = nullptr, st_copy = nullptr;
         cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
         double last_ms[4] = {0, 0, 0, 0};                   // wall, h2d, tiles, bytes out (diagnostics)
@@ -152,6 +152,10 @@ struct gcwt_plan {
 
 namespace gcwt {
 int ensure_workspace(gcwt_plan* p, size_t bytes);
+// grow-on-demand buffers: when *have < need, free *ptr and allocate `need` bytes (the contents are not kept);
+// `who` prefixes the error text
+int grow_device(void** ptr, size_t* have, size_t need, const char* who);
+int grow_pinned(void** ptr, size_t* have, size_t need, const char* who);
 void count_launch(int n = 1);
 int64_t launches_so_far();
 // RAII-less profiling span: begin returns an index (or -1 when profiling is off)
@@ -179,8 +183,7 @@ int means_launch(const void* x, int in_type, int64_t n_channels, int64_t n_sampl
                  int64_t x_stride, double* d_means, double* partial, cudaStream_t st);
 int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n_samples, int64_t x_stride,
                  const int64_t* epochs, int n_epochs, const double* means_host, void* out, int64_t s_stride,
-                 int64_t c_stride, int64_t tile_hint, int64_t pool_width = 0, int pool_mode = 0,
-                 const BandTable* bands = nullptr);
+                 int64_t c_stride, int64_t pool_width = 0, int pool_mode = 0, const BandTable* bands = nullptr);
 int pool_rows_launch(const void* x_dev, int type, int64_t n_rows, int64_t n_cols, int64_t row_stride, int64_t width,
                      int mode, int square, double* out_dev, int64_t out_stride, cudaStream_t st);
 // host-side checks of a band table (NULL pointers, 1..kMaxBands bands, count >= 1, first >= 0, at most

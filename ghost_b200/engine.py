@@ -228,15 +228,11 @@ class CwtPlan:
             done += (b - a) * n_ch * self.n_scales
         return done
 
-    def execute_host(self, x, out=None, means=None, epochs=None):
-        """Host-buffer entry point (numpy in, numpy out) through gcwt_execute_host: the whole transform
-        body of the reference (global mean removal, one zero-padded convolution per epoch, zeros outside
-        the epochs; transforms.py:142-143,185,202-204) as one streamed, double-buffered call.
-
-        ``x`` (channels, samples) or (samples,); ``out`` optional (channels, scales, samples) array of the
-        plan's output dtype with unit sample stride -- pass a pinned one (e.g. the numpy view of a
-        ``torch.empty(..., pin_memory=True)``) to let the device write it by DMA; ``epochs`` optional
-        (E, 2) array of [start, stop) sample bounds.  Results larger than device memory are fine."""
+    def _host_args(self, x, means, epochs):
+        """Leading ctypes arguments of the gcwt_execute_host* entry points: ``x`` (channels, samples) or (samples,),
+        promoted to float64 unless it and the plan are float32, with unit sample stride; ``means`` one float64 per
+        channel; ``epochs`` (E, 2) int64 [start, stop) bounds.  Returns ``(n_channels, n_samples, x_args,
+        epoch_args, means_ptr)``; every pointer keeps its array alive."""
         x = np.asarray(x)
         if x.ndim == 1:
             x = x[None, :]
@@ -247,6 +243,29 @@ class CwtPlan:
         if x.strides[1] != x.itemsize:
             x = np.ascontiguousarray(x)
         n_ch, n = x.shape
+        if means is not None:
+            means = np.ascontiguousarray(means, dtype=np.float64)
+            if means.size != n_ch:
+                raise ValueError("means must hold one value per channel")
+        if epochs is not None:
+            epochs = np.ascontiguousarray(epochs, dtype=np.int64).reshape(-1, 2)
+
+        def ptr(a):
+            return None if a is None else a.ctypes.data_as(C.c_void_p)
+        in_type = _lib.F32 if x.dtype == np.float32 else _lib.F64
+        return (n_ch, n, (ptr(x), in_type, n_ch, n, x.strides[0] // x.itemsize),
+                (ptr(epochs), 0 if epochs is None else int(epochs.shape[0])), ptr(means))
+
+    def execute_host(self, x, out=None, means=None, epochs=None):
+        """Host-buffer entry point (numpy in, numpy out) through gcwt_execute_host: the whole transform
+        body of the reference (global mean removal, one zero-padded convolution per epoch, zeros outside
+        the epochs; transforms.py:142-143,185,202-204) as one streamed, double-buffered call.
+
+        ``x`` (channels, samples) or (samples,); ``out`` optional (channels, scales, samples) array of the
+        plan's output dtype with unit sample stride -- pass a pinned one (e.g. the numpy view of a
+        ``torch.empty(..., pin_memory=True)``) to let the device write it by DMA; ``epochs`` optional
+        (E, 2) array of [start, stop) sample bounds.  Results larger than device memory are fine."""
+        n_ch, n, xa, ea, mp = self._host_args(x, means, epochs)
         if self.output == "complex":
             odt = np.dtype(np.complex64 if self.dtype == np.float32 else np.complex128)
         else:
@@ -256,19 +275,7 @@ class CwtPlan:
         if out.dtype != odt or out.shape != (n_ch, self.n_scales, n) or out.strides[2] != out.itemsize \
                 or out.strides[0] % out.itemsize or out.strides[1] % out.itemsize:
             raise ValueError("out must be (channels, scales, samples) of dtype %s with unit sample stride" % odt)
-        mptr = None
-        if means is not None:
-            means = np.ascontiguousarray(means, dtype=np.float64)
-            if means.size != n_ch:
-                raise ValueError("means must hold one value per channel")
-            mptr = means.ctypes.data
-        eptr, n_ep = None, 0
-        if epochs is not None:
-            epochs = np.ascontiguousarray(epochs, dtype=np.int64).reshape(-1, 2)
-            eptr, n_ep = epochs.ctypes.data, int(epochs.shape[0])
-        in_type = _lib.F32 if x.dtype == np.float32 else _lib.F64
-        _lib.check(self.lib.gcwt_execute_host(self._h, x.ctypes.data, in_type, n_ch, n, x.strides[0] // x.itemsize,
-                                              eptr, n_ep, mptr, out.ctypes.data, out.strides[1] // out.itemsize,
+        _lib.check(self.lib.gcwt_execute_host(self._h, *xa, *ea, mp, out.ctypes.data, out.strides[1] // out.itemsize,
                                               out.strides[0] // out.itemsize))
         return out
 
@@ -283,24 +290,12 @@ class CwtPlan:
         pool_width = int(pool_width)
         if pool_width < 1:
             raise ValueError("pool_width must be a positive integer")
-        x = np.asarray(x)
-        if x.ndim == 1:
-            x = x[None, :]
-        if x.dtype not in (np.float32, np.float64) or (self.dtype == np.float64 and x.dtype != np.float64):
-            x = x.astype(np.float64)
-        if x.strides[1] != x.itemsize:
-            x = np.ascontiguousarray(x)
-        n_ch, n = x.shape
+        n_ch, n, xa, _, mp = self._host_args(x, means, None)
         n_bins = -(-n // pool_width)
         out = np.empty((n_ch, self.n_scales, n_bins), dtype=np.float64)
-        mptr = None
-        if means is not None:
-            means = np.ascontiguousarray(means, dtype=np.float64)
-            mptr = means.ctypes.data
-        in_type = _lib.F32 if x.dtype == np.float32 else _lib.F64
         _lib.check(self.lib.gcwt_execute_host_pooled(
-            self._h, x.ctypes.data, in_type, n_ch, n, x.strides[0] // x.itemsize, mptr, pool_width,
-            _lib.POOL_MEAN if pool == "mean" else _lib.POOL_MAX, out.ctypes.data, n_bins, n_bins * self.n_scales))
+            self._h, *xa, mp, pool_width, _lib.POOL_MEAN if pool == "mean" else _lib.POOL_MAX, out.ctypes.data,
+            n_bins, n_bins * self.n_scales))
         return out
 
     def pool_rows(self, res, pool_width, pool="mean", square=False):
@@ -331,32 +326,12 @@ class CwtPlan:
         Band b is ``sum_k weights[off_b + k] * |W[:, first[b] + k, :]|**2`` (see :func:`band_tables`); samples
         outside the ``epochs`` are zero."""
         first, count, weights = _band_args(first, count, weights)
-        x = np.asarray(x)
-        if x.ndim == 1:
-            x = x[None, :]
-        if x.ndim != 2:
-            raise ValueError("x must be (channels, samples)")
-        if x.dtype not in (np.float32, np.float64) or (self.dtype == np.float64 and x.dtype != np.float64):
-            x = x.astype(np.float64)
-        if x.strides[1] != x.itemsize:
-            x = np.ascontiguousarray(x)
-        n_ch, n = x.shape
+        n_ch, n, xa, ea, mp = self._host_args(x, means, epochs)
         n_b = int(first.size)
         out = np.empty((n_ch, n_b, n), dtype=self.dtype)
-        mptr = None
-        if means is not None:
-            means = np.ascontiguousarray(means, dtype=np.float64)
-            if means.size != n_ch:
-                raise ValueError("means must hold one value per channel")
-            mptr = means.ctypes.data
-        eptr, n_ep = None, 0
-        if epochs is not None:
-            epochs = np.ascontiguousarray(epochs, dtype=np.int64).reshape(-1, 2)
-            eptr, n_ep = epochs.ctypes.data, int(epochs.shape[0])
-        in_type = _lib.F32 if x.dtype == np.float32 else _lib.F64
         _lib.check(self.lib.gcwt_execute_host_bands(
-            self._h, x.ctypes.data, in_type, n_ch, n, x.strides[0] // x.itemsize, eptr, n_ep, mptr,
-            n_b, first.ctypes.data, count.ctypes.data, weights.ctypes.data, out.ctypes.data, n, n_b * n))
+            self._h, *xa, *ea, mp, n_b, first.ctypes.data, count.ctypes.data, weights.ctypes.data, out.ctypes.data,
+            n, n_b * n))
         return out
 
     def band_reduce(self, res, first, count, weights):

@@ -254,10 +254,10 @@ class ContinuousWaveletTransform(WaveletTransform):
         self._host = None
         self._result = None
         start_time = _time.time()
+        x_in = x_host if x_host.dtype == in_dtype else x_host.astype(in_dtype)
         if bands is not None:
             # band power only: every tile is reduced over scales on the device and (bands x samples) per channel
             # travels to the host, epochs and zeros between them as for the full result
-            x_in = x_host if x_host.dtype == in_dtype else x_host.astype(in_dtype)
             res = plan.execute_host_bands(x_in, b_first, b_count, b_weights, epochs=epoch_bounds)
             self._band_power = res if multichannel else res[0]
             self._band_frequencies = [frequencies[a:a + c] for a, c in zip(b_first, b_count)]
@@ -268,7 +268,6 @@ class ContinuousWaveletTransform(WaveletTransform):
                 raise ValueError("'pool_width' needs output='amplitude' or 'power'")
             if len(epoch_bounds) != 1:
                 raise ValueError("'pool_width' needs gap-free timestamps (one epoch)")
-            x_in = x_host if x_host.dtype == in_dtype else x_host.astype(in_dtype)
             res = plan.execute_host_pooled(x_in, pool_width, "mean" if pool is None else pool)
             self._host = res if multichannel else res[0]
             w = int(pool_width)
@@ -281,7 +280,6 @@ class ContinuousWaveletTransform(WaveletTransform):
             # host arrays in, host arrays out (what the reference returns, transforms.py:185,231): one
             # streamed call into the library -- tiles of the result travel to the host while the next is
             # computed, so results larger than device memory work
-            x_in = x_host if x_host.dtype == in_dtype else x_host.astype(in_dtype)
             if out is not None:
                 res = out if multichannel else out[None]
             else:
@@ -291,7 +289,7 @@ class ContinuousWaveletTransform(WaveletTransform):
         else:
             import torch
             dev = torch.device("cuda", self._device)
-            x_dev = torch.from_numpy(np.ascontiguousarray(x_host, dtype=in_dtype)).to(dev)
+            x_dev = torch.from_numpy(np.ascontiguousarray(x_in)).to(dev)
             means = plan.channel_means(x_dev)                  # global mean, transforms.py:142-143
             res = plan.alloc_out(x_dev.shape[0], x_dev.shape[1])
             covered = 0

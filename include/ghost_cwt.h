@@ -146,7 +146,9 @@ int gcwt_execute_host(gcwt_plan *plan, const void *x, int32_t in_type,
  *   (power from an amplitude array).
  * gcwt_execute_host_pooled: gcwt_execute_host (one epoch, amplitude or power plans) whose tiles are pooled
  *   on the device, so that only ceil(n_samples / pool_width) float64 bins per (channel, scale) cross the
- *   link instead of every coefficient: out[c * out_channel_stride + s * out_scale_stride + bin]. */
+ *   link instead of every coefficient: out[c * out_channel_stride + s * out_scale_stride + bin].  The bins
+ *   reach `out` as gcwt_execute_host's rows do: by DMA when `out` is pinned, through the pinned ring and host
+ *   threads when it is pageable. */
 #define GCWT_POOL_MEAN 0
 #define GCWT_POOL_MAX  1
 int gcwt_pool_rows(const void *x_dev, int32_t type, int64_t n_rows, int64_t n_cols, int64_t row_stride,

@@ -8,7 +8,7 @@ pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
 
-from ghost_b200 import ContinuousWaveletTransform, Morse, synth        # noqa: E402
+from ghost_b200 import ContinuousWaveletTransform, Morse, _lib, synth  # noqa: E402
 from ghost_b200.engine import CwtPlan, band_tables, scale_tables         # noqa: E402
 from oracle import cwt_oracle as orc                                     # noqa: E402
 
@@ -191,6 +191,40 @@ def test_bands_with_forced_time_tiles(monkeypatch):
     first, count, w = band_tables(tiled.frequencies, bands)
     full = tiled.last_plan.execute_host(X)                        # the same forced tiles, full rate
     np.testing.assert_allclose(tiled.band_power, _np_bands(full, first, count, w, "power"), rtol=1e-6, atol=0)
+
+
+@pytest.mark.parametrize("tile", [None, "7000"])
+@pytest.mark.parametrize("dest", ["pinned", "strided"])
+def test_bands_into_pinned_and_strided_destinations(dest, tile, monkeypatch):
+    """Band rows reach a pinned array by DMA and a strided pageable one through the copier threads, as
+    band_reduce of the device path's full result has them; the padding behind every row stays untouched."""
+    fs, n = 1000.0, 50000
+    X = synth.recording(2, n, fs, np.float32)
+    f = orc.frequency_grid(fs, n)
+    plan = _plan(fs, f, dtype=np.float32, output="power")
+    first, count, w = band_tables(f, EPHYS_BANDS + [(1.5, 4.0)])
+    B = first.size
+    want = plan.band_reduce(plan.execute(torch.from_numpy(X).cuda()), first, count, w).cpu().numpy()
+    if tile:
+        monkeypatch.setenv("GCWT_HOST_TILE", tile)
+    if dest == "pinned":
+        keep = torch.full((2, B, n + 5), -1.0, dtype=torch.float32).pin_memory()
+        big = keep.numpy()
+    else:
+        big = np.full((2, B + 1, n + 5), -1.0, dtype=np.float32)
+    got = big[:, :B, :n]
+    _lib.check(plan.lib.gcwt_execute_host_bands(plan._h, X.ctypes.data, _lib.F32, 2, n, n, None, 0, None, B,
+                                                first.ctypes.data, count.ctypes.data, w.ctypes.data, got.ctypes.data,
+                                                got.strides[1] // 4, got.strides[0] // 4))
+    st = plan.host_stats()
+    assert st["pinned_destination"] == (dest == "pinned") and st["tiles"] == (1 if tile is None else 8)
+    assert st["bytes_out"] == got.nbytes
+    assert np.all(big[:, :, n:] == -1.0) and np.all(big[:, B:] == -1.0)
+    if tile is None:
+        assert np.array_equal(got, want)
+    else:
+        err = _l2rel(got.astype(np.float64), want.astype(np.float64))
+        assert err.max() <= 3e-6, err.max()
 
 
 @pytest.mark.parametrize("name", ["tones", "violet"])

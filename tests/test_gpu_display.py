@@ -7,7 +7,7 @@ pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
 
-from ghost_b200 import ContinuousWaveletTransform, synth        # noqa: E402
+from ghost_b200 import ContinuousWaveletTransform, _lib, synth  # noqa: E402
 from oracle import cwt_oracle as orc                             # noqa: E402
 
 
@@ -81,6 +81,7 @@ def test_transform_pool_width_streams_only_the_bins():
         assert np.allclose(got, want, rtol=1e-6)
         st = cwt.last_plan.host_stats()
         assert st["bytes_out"] == got.nbytes and st["bytes_out"] * 250 < full.power.nbytes
+        assert not st["pinned_destination"]
         assert len(cwt.time) == got.shape[2] and abs(cwt.time[0] - 255.5 / fs) < 1e-12
     with pytest.raises(ValueError):
         ContinuousWaveletTransform(dtype=np.float32, output="complex").transform(X[0], fs=fs, pool_width=16)
@@ -99,3 +100,36 @@ def test_pooled_host_path_with_forced_time_tiles(monkeypatch):
     assert pooled.last_plan.host_stats()["tiles"] == -(-n // 6900)
     rel = np.linalg.norm(pooled.amplitude - want, axis=1) / np.linalg.norm(want, axis=1)
     assert pooled.amplitude.shape == want.shape and rel.max() <= 3e-6, rel.max()
+
+
+@pytest.mark.parametrize("tile", [None, "7000"])
+@pytest.mark.parametrize("dest", ["pinned", "strided"])
+def test_pooled_host_path_into_pinned_and_strided_destinations(dest, tile, monkeypatch):
+    """Pooled bins reach a pinned array by DMA and a strided pageable one through the copier threads, as the
+    device path's pooling of the full result has them; the padding behind every row stays untouched."""
+    fs, n, width = 1000.0, 50001, 300
+    X = synth.recording(2, n, fs, np.float32)
+    cwt = ContinuousWaveletTransform(dtype=np.float32, output="power")
+    cwt.transform(X, fs=fs, multichannel=True, freq_limits=[2.0, 300.0], keep_on_device=True)
+    plan, S, nb = cwt.last_plan, cwt.frequencies.size, -(-n // width)
+    full = plan.execute(torch.from_numpy(X).cuda())
+    if tile:
+        monkeypatch.setenv("GCWT_HOST_TILE", tile)
+    for pool, mode in (("mean", _lib.POOL_MEAN), ("max", _lib.POOL_MAX)):
+        want = plan.pool_rows(full, width, pool).cpu().numpy()
+        if dest == "pinned":
+            keep = torch.full((2, S, nb + 5), -1.0, dtype=torch.float64).pin_memory()
+            big = keep.numpy()
+        else:
+            big = np.full((2, S + 1, nb + 5), -1.0)
+        got = big[:, :S, :nb]
+        _lib.check(plan.lib.gcwt_execute_host_pooled(plan._h, X.ctypes.data, _lib.F32, 2, n, n, None, width, mode,
+                                                     got.ctypes.data, got.strides[1] // 8, got.strides[0] // 8))
+        st = plan.host_stats()
+        assert st["pinned_destination"] == (dest == "pinned") and st["tiles"] == (1 if tile is None else -(-n // 6900))
+        assert np.all(big[:, :, nb:] == -1.0) and np.all(big[:, S:] == -1.0)
+        if tile is None:
+            assert np.array_equal(got, want), pool
+        else:
+            rel = np.linalg.norm(got - want, axis=2) / np.linalg.norm(want, axis=2)
+            assert rel.max() <= 3e-6, (pool, rel.max())

@@ -101,3 +101,6 @@ def test_host_path_argument_errors():
         plan.execute_host(x, epochs=np.array([[10, 5]]))
     with pytest.raises(_lib.GcwtError, match="epoch"):
         plan.execute_host(x, epochs=np.array([[0, 3000], [2000, 5000]]))
+    x2 = np.zeros((2, 5000), dtype=np.float32)
+    with pytest.raises(ValueError, match="one value per channel"):
+        plan.execute_host_pooled(x2, 16, means=np.zeros(1))

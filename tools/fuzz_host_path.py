@@ -1,6 +1,7 @@
-"""GPU box: randomized check of the streamed host path (gcwt_execute_host and its pooled variant): random
-channel counts, lengths, epochs, forced tile lengths, pinned / pageable / strided destinations, against the
-device path executed epoch by epoch.       python tools/fuzz_host_path.py [n_cases] [seed]"""
+"""GPU box: randomized check of the streamed host path (gcwt_execute_host and its pooled and band-power
+variants): random channel counts, lengths, epochs, forced tile lengths, pinned / pageable / strided destinations
+and random bands, against the device path executed epoch by epoch (pooled in numpy, band-reduced with
+plan.band_reduce).       python tools/fuzz_host_path.py [n_cases] [seed]"""
 import os
 import sys
 import numpy as np
@@ -55,11 +56,11 @@ for case in range(n_cases):
     # device path, epoch by epoch, global mean
     xd = torch.from_numpy(X if dtype == np.float32 else X.astype(np.float64)).cuda()
     means = plan.channel_means(xd)
-    want = plan.alloc_out(nch, n)
-    want.zero_()
+    want_d = plan.alloc_out(nch, n)
+    want_d.zero_()
     for a, b in epochs:
-        plan.execute(xd, want, means=means, start=int(a), stop=int(b))
-    want = want.cpu().numpy()
+        plan.execute(xd, want_d, means=means, start=int(a), stop=int(b))
+    want = want_d.cpu().numpy()
     num = np.linalg.norm((got - want).reshape(nch, S, -1), axis=2)
     den = np.linalg.norm(want.reshape(nch, S, -1), axis=2)
     err = float((num / den).max())
@@ -83,8 +84,23 @@ for case in range(n_cases):
         # per row, relative to the row's largest bin (tiles round differently at the 1e-7 level of the row's scale)
         perr = float(np.max(np.max(np.abs(pooled - ref), axis=2) / (np.max(np.abs(ref), axis=2) + 1e-300)))
         ok = ok and perr <= (1e-5 if dtype == np.float32 else 1e-11)
-    print("case %2d %s %s %s ch=%d n=%d epochs=%d S=%d tile=%d tiles=%d dest=%s err=%.2e pooled=%.1e" % (
-        case, "ok " if ok else "BAD", np.dtype(dtype).name, output, nch, n, n_ep, S, tile, tiles, dest, err, perr), flush=True)
+    # band power: random (possibly overlapping) bands, same epochs and tiles; the gap columns of want_d are zero
+    n_b = int(rng.integers(1, 7))
+    first = rng.integers(0, S, n_b).astype(np.int32)
+    count = np.array([rng.integers(1, S - f + 1) for f in first], dtype=np.int32)
+    weights = rng.uniform(0.1, 2.0, int(count.sum()))
+    got_b = plan.execute_host_bands(X if dtype == np.float32 else X.astype(np.float64), first, count, weights, epochs=epochs)
+    want_b = plan.band_reduce(want_d, first, count, weights).cpu().numpy()
+    berr = float(np.max(np.linalg.norm(got_b - want_b, axis=2) / np.linalg.norm(want_b, axis=2)))
+    pos = 0
+    for a, b in epochs:
+        gaps_ok = gaps_ok and bool(np.all(got_b[:, :, pos:a] == 0))
+        pos = b
+    gaps_ok = gaps_ok and bool(np.all(got_b[:, :, pos:] == 0))
+    ok = ok and gaps_ok and berr <= (1.2e-5 if dtype == np.float32 else 1e-11)
+    print("case %2d %s %s %s ch=%d n=%d epochs=%d S=%d tile=%d tiles=%d dest=%s err=%.2e pooled=%.1e bands=%d %.1e" % (
+        case, "ok " if ok else "BAD", np.dtype(dtype).name, output, nch, n, n_ep, S, tile, tiles, dest, err, perr, n_b,
+        berr), flush=True)
     if not ok:
         fails.append(case)
     plan.close()
