@@ -25,7 +25,7 @@ EXPORTS = (
     "gcwt_morse_kernel", "gcwt_profile_enable", "gcwt_profile_read",
     "gcwt_fastconv", "gcwt_dft", "gcwt_analytic_signal", "gcwt_moments", "gcwt_interp_taps",
     "gcwt_guard_stats", "gcwt_host_stats", "gcwt_pool_rows", "gcwt_execute_host_pooled",
-    "gcwt_band_reduce", "gcwt_execute_host_bands",
+    "gcwt_band_reduce", "gcwt_execute_host_bands", "gcwt_event_reduce", "gcwt_execute_host_events",
 )
 
 
@@ -80,6 +80,9 @@ def load():
     lib.gcwt_execute_host_pooled.argtypes = [vp, vp, i32, i64, i64, i64, vp, i64, i32, vp, i64, i64]
     lib.gcwt_band_reduce.argtypes = [vp, i32, i32, i64, i64, i64, i64, i32, vp, vp, vp, vp, i64, i64, i32, vp]
     lib.gcwt_execute_host_bands.argtypes = [vp, vp, i32, i64, i64, i64, vp, i32, vp, i32, vp, vp, vp, vp, i64, i64]
+    lib.gcwt_event_reduce.argtypes = [vp, i32, i32, i64, i32, i64, i64, i64, i64, vp, i64, i64, i64, vp, vp, i64, i64,
+                                      i32, vp]
+    lib.gcwt_execute_host_events.argtypes = [vp, vp, i32, i64, i64, i64, vp, i32, vp, vp, i64, i64, i64, vp, vp, i64, i64]
     lib.gcwt_filter_response.argtypes = [i64, i32, i32, dp, i64, i64, i64, dp, i32]
     lib.gcwt_morse_kernel.argtypes = [i64, i32, i32, dp, dp, i32]
     lib.gcwt_fastconv.argtypes = [dp, i32, i64, dp, i32, i64, dp, i32]

@@ -399,6 +399,51 @@ int gcwt_execute_host_bands(gcwt_plan* p, const void* x, int32_t in_type, int64_
                         out_band_stride, out_channel_stride, 0, 0, &tab);
 }
 
+int gcwt_event_reduce(const void* coef_dev, int32_t coef_type, int32_t coef_kind, int64_t n_channels, int32_t n_scales,
+                      int64_t n_samples, int64_t scale_stride, int64_t channel_stride, int64_t sample0,
+                      const int64_t* events_dev, int64_t n_events, int64_t lag_first, int64_t n_lags,
+                      double* acc_power_dev, double* acc_phase_dev, int64_t acc_scale_stride,
+                      int64_t acc_channel_stride, int32_t device, void* stream) {
+    if (!coef_dev || !events_dev || !acc_power_dev) { set_error("event_reduce: coef/events/acc_power is NULL"); return GCWT_ERR_ARG; }
+    if (coef_type != GCWT_F32 && coef_type != GCWT_F64) { set_error("event_reduce: coef_type must be GCWT_F32 or GCWT_F64"); return GCWT_ERR_ARG; }
+    if (coef_kind < GCWT_OUT_COMPLEX || coef_kind > GCWT_OUT_POWER) { set_error("event_reduce: bad coef_kind"); return GCWT_ERR_ARG; }
+    if (acc_phase_dev && coef_kind != GCWT_OUT_COMPLEX) { set_error("event_reduce: a phase accumulator needs complex coefficients"); return GCWT_ERR_ARG; }
+    if (n_channels <= 0 || n_scales <= 0 || n_samples <= 0 || n_events <= 0 || n_lags <= 0) {
+        set_error("event_reduce: n_channels, n_scales, n_samples, n_events and n_lags must be positive"); return GCWT_ERR_ARG;
+    }
+    if (n_scales > 65535) { set_error("event_reduce: at most 65535 scales"); return GCWT_ERR_ARG; }
+    if (scale_stride < n_samples || (n_channels > 1 && channel_stride < (int64_t)n_scales * scale_stride)) {
+        set_error("event_reduce: scale_stride below n_samples, or channel_stride below n_scales rows"); return GCWT_ERR_ARG;
+    }
+    if (acc_scale_stride < n_lags || (n_channels > 1 && acc_channel_stride < (int64_t)n_scales * acc_scale_stride)) {
+        set_error("event_reduce: acc_scale_stride below n_lags, or acc_channel_stride below n_scales rows"); return GCWT_ERR_ARG;
+    }
+    if (acc_phase_dev && (uintptr_t)acc_phase_dev % 16) { set_error("event_reduce: acc_phase must be 16-byte aligned"); return GCWT_ERR_ARG; }
+    DeviceScope dev_scope(device);
+    return event_reduce_launch(coef_dev, coef_type, coef_kind, n_channels, n_scales, n_samples, scale_stride, channel_stride,
+                               sample0, events_dev, n_events, lag_first, n_lags, acc_power_dev, (double2*)acc_phase_dev,
+                               acc_scale_stride, acc_channel_stride, (cudaStream_t)stream);
+}
+
+int gcwt_execute_host_events(gcwt_plan* p, const void* x, int32_t in_type, int64_t n_channels, int64_t n_samples,
+                             int64_t x_stride, const int64_t* epoch_bounds, int32_t n_epochs, const double* means_host,
+                             const int64_t* events, int64_t n_events, int64_t lag_first, int64_t n_lags, double* power_out,
+                             double* phase_out, int64_t out_scale_stride, int64_t out_channel_stride) {
+    if (!events) { set_error("execute_host_events: events is NULL"); return GCWT_ERR_ARG; }
+    if (n_events <= 0 || n_lags <= 0) { set_error("execute_host_events: n_events and n_lags must be positive"); return GCWT_ERR_ARG; }
+    int rc = check_event_args(n_samples, epoch_bounds, n_epochs, events, n_events, lag_first, n_lags);
+    if (rc) return rc;
+    rc = check_exec_args(p, x, in_type, n_channels, n_samples, x_stride, power_out);
+    if (rc) return rc;
+    if (phase_out && p->out_kind != GCWT_OUT_COMPLEX) { set_error("execute_host_events: phase_out needs a complex plan"); return GCWT_ERR_ARG; }
+    if (out_scale_stride < n_lags || (n_channels > 1 && out_channel_stride < (int64_t)p->n_scales * out_scale_stride)) {
+        set_error("execute_host_events: out_scale_stride below n_lags, or out_channel_stride below n_scales rows"); return GCWT_ERR_ARG;
+    }
+    DeviceScope dev_scope(p->device);
+    return host_execute_events(p, x, in_type, n_channels, n_samples, x_stride, epoch_bounds, n_epochs, means_host, events,
+                               n_events, lag_first, n_lags, power_out, phase_out, out_scale_stride, out_channel_stride);
+}
+
 int gcwt_host_stats(const gcwt_plan* p, double* out4) {
     if (!p || !out4) { set_error("host_stats: NULL argument"); return GCWT_ERR_ARG; }
     for (int k = 0; k < 4; ++k) out4[k] = p->host.last_ms[k];

@@ -13,6 +13,8 @@
 //     one cudaMemcpy2DAsync per channel of a tile;
 //   pageable destination (a plain numpy array): tiles land in a plan-owned pinned ring by DMA and a few
 //     host threads copy the rows out (which also first-touches the caller's pages in parallel).
+// Event-locked averages (host_execute_events) use the same tiles but send nothing per tile: each tile is added into
+// a device accumulator of (channels x scales x lags) and only that crosses the link, once per channel group.
 //
 // Epochs (transforms.py:202-204): every epoch is a zero-padded convolution of its own; samples outside
 // all epochs are zero.  The mean is the channel's mean over ALL samples (transforms.py:142-143).
@@ -41,6 +43,8 @@ void host_stage_free(gcwt_plan* p) {
         if (h.ev_out[b]) cudaEventDestroy(h.ev_out[b]);
     }
     if (h.d_means) cudaFree(h.d_means);
+    if (h.d_acc) cudaFree(h.d_acc);
+    if (h.d_events) cudaFree(h.d_events);
     if (h.st_compute) cudaStreamDestroy(h.st_compute);
     if (h.st_copy) cudaStreamDestroy(h.st_copy);
     h = gcwt_plan::HostStage();
@@ -126,6 +130,41 @@ static int grow_staging(gcwt_plan::HostStage& h, size_t in_bytes, size_t tile_by
     return rc;
 }
 
+// the compute and copy streams and the two slots' events, created on a plan's first host call
+static int ensure_streams(gcwt_plan::HostStage& h) {
+    if (h.st_compute) return GCWT_OK;
+    GCWT_CUDA_OK(cudaStreamCreateWithFlags(&h.st_compute, cudaStreamNonBlocking));
+    GCWT_CUDA_OK(cudaStreamCreateWithFlags(&h.st_copy, cudaStreamNonBlocking));
+    for (int b = 0; b < 2; ++b) {
+        GCWT_CUDA_OK(cudaEventCreateWithFlags(&h.ev_done[b], cudaEventDisableTiming));
+        GCWT_CUDA_OK(cudaEventCreateWithFlags(&h.ev_out[b], cudaEventDisableTiming));
+    }
+    return GCWT_OK;
+}
+
+// upload channels [c0, c0 + gc) of x into d_in and put their means into d_means, on the compute stream
+static int load_group(gcwt_plan* p, const void* x, int in_type, int64_t n, int64_t x_stride, const double* means_host,
+                      int64_t c0, int64_t gc) {
+    gcwt_plan::HostStage& h = p->host;
+    const size_t in_el = in_type == GCWT_F32 ? 4 : 8;
+    // the previous group's tiles may still be copying out, but nothing reads d_in any more: every execute of
+    // that group has completed (gcwt_execute waits, or we wait here)
+    GCWT_CUDA_OK(cudaStreamSynchronize(h.st_compute));
+    GCWT_CUDA_OK(cudaMemcpy2DAsync(h.d_in, (size_t)n * in_el, (const char*)x + (size_t)c0 * x_stride * in_el, (size_t)x_stride * in_el,
+                                   (size_t)n * in_el, (size_t)gc, cudaMemcpyHostToDevice, h.st_compute));
+    if (means_host) {
+        GCWT_CUDA_OK(cudaMemcpyAsync(h.d_means, means_host + c0, sizeof(double) * gc, cudaMemcpyHostToDevice, h.st_compute));
+        return GCWT_OK;
+    }
+    const size_t need = sizeof(double) * means_blocks(n) * gc;
+    if (p->partial_bytes < need) {
+        GCWT_CUDA_OK(cudaStreamSynchronize(h.st_compute));
+        const int r = grow_device((void**)&p->d_partial, &p->partial_bytes, need, "execute_host");
+        if (r) return r;
+    }
+    return means_launch(h.d_in, in_type, gc, n, n, h.d_means, p->d_partial, h.st_compute);
+}
+
 // zero the columns outside the epochs (the reference starts from np.zeros, transforms.py:185)
 static void zero_gaps(char* out, const int64_t* epochs, int n_epochs, int64_t n, int64_t n_channels, int R,
                       int64_t s_stride, int64_t c_stride, size_t el) {
@@ -166,14 +205,8 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
             return GCWT_ERR_UNSUPPORTED;
         }
     }
-    if (!h.st_compute) {
-        GCWT_CUDA_OK(cudaStreamCreateWithFlags(&h.st_compute, cudaStreamNonBlocking));
-        GCWT_CUDA_OK(cudaStreamCreateWithFlags(&h.st_copy, cudaStreamNonBlocking));
-        for (int b = 0; b < 2; ++b) {
-            GCWT_CUDA_OK(cudaEventCreateWithFlags(&h.ev_done[b], cudaEventDisableTiming));
-            GCWT_CUDA_OK(cudaEventCreateWithFlags(&h.ev_out[b], cudaEventDisableTiming));
-        }
-    }
+    rc = ensure_streams(h);
+    if (rc) return rc;
     const TileGeometry geo = tile_geometry(p, n_channels, n, out_el, pool_width);
     const int64_t tile_alloc = (geo.tile + 3) & ~int64_t(3);      // rows of a tile stay 16-byte aligned
 
@@ -215,25 +248,6 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
         else if (copier[b].joinable()) copier[b].join();
         live[b] = false;
         return GCWT_OK;
-    };
-    // the group's samples and means
-    auto load_group = [&](int64_t c0, int64_t gc) -> int {
-        // the previous group's tiles may still be copying out, but nothing reads d_in any more: every execute of
-        // that group has completed (gcwt_execute waits, or we wait here)
-        GCWT_CUDA_OK(cudaStreamSynchronize(h.st_compute));
-        GCWT_CUDA_OK(cudaMemcpy2DAsync(h.d_in, (size_t)n * in_el, (const char*)x + (size_t)c0 * x_stride * in_el, (size_t)x_stride * in_el,
-                                       (size_t)n * in_el, (size_t)gc, cudaMemcpyHostToDevice, h.st_compute));
-        if (means_host) {
-            GCWT_CUDA_OK(cudaMemcpyAsync(h.d_means, means_host + c0, sizeof(double) * gc, cudaMemcpyHostToDevice, h.st_compute));
-            return GCWT_OK;
-        }
-        const size_t need = sizeof(double) * means_blocks(n) * gc;
-        if (p->partial_bytes < need) {
-            GCWT_CUDA_OK(cudaStreamSynchronize(h.st_compute));
-            const int r = grow_device((void**)&p->d_partial, &p->partial_bytes, need, "execute_host");
-            if (r) return r;
-        }
-        return means_launch(h.d_in, in_type, gc, n, n, h.d_means, p->d_partial, h.st_compute);
     };
     // one tile: compute it into d_out[b], reduce it if this call asks for a reduction, and send its rows to `out`
     auto run_tile = [&](int b, int64_t c0, int64_t gc, int64_t a, int64_t len, int64_t halo_l, int64_t halo_r) -> int {
@@ -285,7 +299,7 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
     double bytes_out = 0;
     for (int64_t c0 = 0; c0 < n_channels && rc == GCWT_OK; c0 += geo.g) {
         const int64_t gc = std::min<int64_t>(geo.g, n_channels - c0);
-        rc = load_group(c0, gc);
+        rc = load_group(p, x, in_type, n, x_stride, means_host, c0, gc);
         for (int e = 0; e < n_epochs && rc == GCWT_OK; ++e) {
             const int64_t e0 = epochs[2 * e], e1 = epochs[2 * e + 1];
             for (int64_t a = e0; a < e1 && rc == GCWT_OK; a += geo.tile) {
@@ -307,6 +321,140 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
     cudaStreamSynchronize(h.st_compute);
     h.last_ms[0] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     h.last_ms[1] = pinned ? 1.0 : 0.0;
+    h.last_ms[2] = (double)n_tiles;
+    h.last_ms[3] = bytes_out;
+    return rc;
+}
+
+int check_event_args(int64_t n, const int64_t* epochs, int n_epochs, const int64_t* events, int64_t n_events,
+                     int64_t lag_first, int64_t n_lags) {
+    int64_t one_epoch[2] = {0, n};
+    if (!epochs || n_epochs <= 0) { epochs = one_epoch; n_epochs = 1; }
+    const int rc = check_epochs(epochs, n_epochs, n);
+    if (rc) return rc;
+    for (int64_t i = 0; i < n_events; ++i) {
+        if (i > 0 && events[i] < events[i - 1]) {
+            set_error("execute_host_events: events must be ascending (event " + std::to_string(i) + " at sample " +
+                      std::to_string(events[i]) + " follows sample " + std::to_string(events[i - 1]) + ")");
+            return GCWT_ERR_ARG;
+        }
+        int64_t w0 = 0, w1 = 0;
+        bool inside = !__builtin_add_overflow(events[i], lag_first, &w0) && !__builtin_add_overflow(w0, n_lags, &w1);
+        if (inside) {                                              // the last epoch that starts at or before w0
+            int lo = 0, hi = n_epochs;
+            while (lo < hi) {
+                const int mid = (lo + hi) / 2;
+                if (epochs[2 * mid] <= w0) lo = mid + 1; else hi = mid;
+            }
+            inside = lo > 0 && w1 <= epochs[2 * (lo - 1) + 1];
+        }
+        if (!inside) {
+            set_error("execute_host_events: the window of event " + std::to_string(i) + " (sample " +
+                      std::to_string(events[i]) + ") does not lie inside one epoch");
+            return GCWT_ERR_ARG;
+        }
+    }
+    return GCWT_OK;
+}
+
+int host_execute_events(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n, int64_t x_stride,
+                        const int64_t* epochs, int n_epochs, const double* means_host, const int64_t* events,
+                        int64_t n_events, int64_t lag_first, int64_t n_lags, double* power_out, double* phase_out,
+                        int64_t os_stride, int64_t oc_stride) {
+    // The tiles are those of gcwt_execute_host, but no tile travels.  After a tile's ev_done the copy stream adds
+    // the tile's part of every window that meets it into a per-group fp64 accumulator (event_reduce_kernel), and
+    // ev_out[b] keeps the next tile of slot b from overwriting d_out[b] before that reduction has read it.  After the
+    // group's last tile the accumulator travels once, through the pinned ring, and the host divides by n_events.
+    gcwt_plan::HostStage& h = p->host;
+    const auto t_begin = std::chrono::steady_clock::now();
+    const int S = p->n_scales;
+    const size_t in_el = in_type == GCWT_F32 ? 4 : 8;
+    const size_t real_el = p->compute_type == GCWT_F32 ? 4 : 8;
+    const size_t out_el = p->out_kind == GCWT_OUT_COMPLEX ? 2 * real_el : real_el;
+    int64_t one_epoch[2] = {0, n};
+    if (!epochs || n_epochs <= 0) { epochs = one_epoch; n_epochs = 1; }
+    int rc = ensure_streams(h);
+    if (rc) return rc;
+    const TileGeometry geo = tile_geometry(p, n_channels, n, out_el, 0);
+    const int64_t tile_alloc = (geo.tile + 3) & ~int64_t(3);      // rows of a tile stay 16-byte aligned
+
+    // a group's accumulator: gc x S x n_lags power sums, then as many double2 phase sums on a 16-byte boundary
+    const bool phase = phase_out != nullptr;
+    auto power_cells = [&](int64_t gc) { return (gc * S * n_lags + 1) & ~int64_t(1); };
+    auto acc_bytes = [&](int64_t gc) {
+        return sizeof(double) * (size_t)power_cells(gc) + (phase ? sizeof(double2) * (size_t)(gc * S * n_lags) : 0);
+    };
+    rc = grow_staging(h, (size_t)geo.g * n * in_el, (size_t)geo.g * S * tile_alloc * out_el, 0, 0, geo.g);
+    if (rc == GCWT_OK) rc = grow_device((void**)&h.d_acc, &h.acc_bytes, acc_bytes(geo.g), "execute_host_events");
+    if (rc == GCWT_OK) rc = grow_device((void**)&h.d_events, &h.events_bytes, sizeof(int64_t) * n_events, "execute_host_events");
+    if (rc == GCWT_OK) rc = grow_pinned(&h.h_ring[0], &h.ring_bytes[0], acc_bytes(geo.g), "execute_host_events");
+    if (rc) return rc;
+    GCWT_CUDA_OK(cudaMemcpyAsync(h.d_events, events, sizeof(int64_t) * n_events, cudaMemcpyHostToDevice, h.st_copy));
+
+    // one tile: compute it into d_out[b] and add its part of every window that meets it
+    auto run_tile = [&](int b, int64_t gc, int64_t a, int64_t len, int64_t halo_l, int64_t halo_r) -> int {
+        GCWT_CUDA_OK(cudaStreamWaitEvent(h.st_compute, h.ev_out[b], 0));
+        int r = gcwt_execute(p, (const char*)h.d_in + (size_t)a * in_el, in_type, gc, len, n, halo_l, halo_r, h.d_means,
+                             h.d_out[b], tile_alloc, (int64_t)S * tile_alloc, h.st_compute);
+        if (r) return r;
+        // ev_done follows the accuracy guard's re-computation, so the sums read the corrected coefficients
+        GCWT_CUDA_OK(cudaEventRecord(h.ev_done[b], h.st_compute));
+        GCWT_CUDA_OK(cudaStreamWaitEvent(h.st_copy, h.ev_done[b], 0));
+        // the events whose windows start in (a - n_lags, a + len): a host-side binary search over ascending events
+        const int64_t* lo = std::partition_point(events, events + n_events,
+                                                 [&](int64_t e) { return e + lag_first <= a - n_lags; });
+        const int64_t* hi = std::partition_point(lo, events + n_events, [&](int64_t e) { return e + lag_first < a + len; });
+        double* acc = h.d_acc;
+        r = event_reduce_launch(h.d_out[b], p->compute_type, p->out_kind, gc, S, len, tile_alloc, (int64_t)S * tile_alloc,
+                                a, h.d_events + (lo - events), hi - lo, lag_first, n_lags, acc,
+                                phase ? (double2*)(acc + power_cells(gc)) : nullptr, n_lags, (int64_t)S * n_lags, h.st_copy);
+        if (r) return r;
+        GCWT_CUDA_OK(cudaEventRecord(h.ev_out[b], h.st_copy));
+        return GCWT_OK;
+    };
+    // the group's means: one D2H of its accumulator, then sum / n_events into the caller's arrays
+    auto drain_group = [&](int64_t c0, int64_t gc) -> int {
+        GCWT_CUDA_OK(cudaMemcpyAsync(h.h_ring[0], h.d_acc, acc_bytes(gc), cudaMemcpyDeviceToHost, h.st_copy));
+        GCWT_CUDA_OK(cudaStreamSynchronize(h.st_copy));
+        const double* sums = (const double*)h.h_ring[0];
+        const double* phase_sums = sums + power_cells(gc);
+        const double cnt = (double)n_events;
+        for (int64_t c = 0; c < gc; ++c)
+            for (int s = 0; s < S; ++s) {
+                const int64_t row = c * S + s, o = (c0 + c) * oc_stride + (int64_t)s * os_stride;
+                for (int64_t l = 0; l < n_lags; ++l) power_out[o + l] = sums[row * n_lags + l] / cnt;
+                if (phase)
+                    for (int64_t l = 0; l < 2 * n_lags; ++l) phase_out[2 * o + l] = phase_sums[2 * row * n_lags + l] / cnt;
+            }
+        return GCWT_OK;
+    };
+
+    int slot = 0;
+    int64_t n_tiles = 0;
+    double bytes_out = 0;
+    for (int64_t c0 = 0; c0 < n_channels && rc == GCWT_OK; c0 += geo.g) {
+        const int64_t gc = std::min<int64_t>(geo.g, n_channels - c0);
+        rc = load_group(p, x, in_type, n, x_stride, means_host, c0, gc);
+        if (rc == GCWT_OK) {
+            const cudaError_t e = cudaMemsetAsync(h.d_acc, 0, acc_bytes(gc), h.st_copy);
+            if (e != cudaSuccess) { set_error(std::string("execute_host_events: ") + cudaGetErrorString(e)); rc = GCWT_ERR_CUDA; }
+        }
+        for (int e = 0; e < n_epochs && rc == GCWT_OK; ++e) {
+            const int64_t e0 = epochs[2 * e], e1 = epochs[2 * e + 1];
+            for (int64_t a = e0; a < e1 && rc == GCWT_OK; a += geo.tile) {
+                const int64_t len = std::min(e1, a + geo.tile) - a;
+                rc = run_tile(slot, gc, a, len, std::min(geo.halo, a - e0), std::min(geo.halo, e1 - a - len));
+                ++n_tiles;
+                slot ^= 1;
+            }
+        }
+        if (rc == GCWT_OK) rc = drain_group(c0, gc);
+        if (rc == GCWT_OK) bytes_out += (double)gc * S * n_lags * (sizeof(double) + (phase ? sizeof(double2) : 0));
+    }
+    cudaStreamSynchronize(h.st_copy);
+    cudaStreamSynchronize(h.st_compute);
+    h.last_ms[0] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    h.last_ms[1] = 0.0;                                            // the means reach the caller from the pinned ring
     h.last_ms[2] = (double)n_tiles;
     h.last_ms[3] = bytes_out;
     return rc;

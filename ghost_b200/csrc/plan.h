@@ -144,6 +144,8 @@ struct gcwt_plan {
         void* d_red[2] = {nullptr, nullptr}; size_t red_bytes[2] = {0, 0};    // reduced tiles: pooled bins or band rows
         void* h_ring[2] = {nullptr, nullptr}; size_t ring_bytes[2] = {0, 0};  // pinned ring (pageable destinations only)
         double* d_means = nullptr; size_t means_bytes = 0;
+        double* d_acc = nullptr; size_t acc_bytes = 0;                         // event sums of a channel group
+        int64_t* d_events = nullptr; size_t events_bytes = 0;                  // the event samples of a call
         cudaStream_t st_compute = nullptr, st_copy = nullptr;
         cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
         double last_ms[4] = {0, 0, 0, 0};                   // wall, h2d, tiles, bytes out (diagnostics)
@@ -195,5 +197,21 @@ int band_table_build(int n_bands, const int32_t* first, const int32_t* count, co
 int band_reduce_launch(const void* x_dev, int type, int kind, int64_t n_channels, int64_t n_samples, int64_t s_stride,
                        int64_t c_stride, const BandTable& tab, void* out_dev, int64_t out_b_stride, int64_t out_c_stride,
                        cudaStream_t st);
+// acc_power[c, s, l] += sum_e |x[c, s, events[e] + lag_first + l - sample0]|^2 and, when acc_phase is not NULL
+// (complex kinds only), acc_phase[c, s, l] += sum_e W / |W|, in fp64, over the events whose sample lies inside
+// [0, n_samples); x strides in elements of `type` (float2 / double2 for complex), acc strides in elements
+int event_reduce_launch(const void* x_dev, int type, int kind, int64_t n_channels, int n_scales, int64_t n_samples,
+                        int64_t s_stride, int64_t c_stride, int64_t sample0, const int64_t* events_dev, int64_t n_events,
+                        int64_t lag_first, int64_t n_lags, double* acc_power, double2* acc_phase, int64_t as_stride,
+                        int64_t ac_stride, cudaStream_t st);
+// host-side checks of gcwt_execute_host_events, run before any device work: the epochs as gcwt_execute_host checks
+// them, events ascending, and every window [e + lag_first, e + lag_first + n_lags) inside one epoch
+int check_event_args(int64_t n_samples, const int64_t* epochs, int n_epochs, const int64_t* events, int64_t n_events,
+                     int64_t lag_first, int64_t n_lags);
+// the events' arguments have passed check_event_args
+int host_execute_events(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n_samples,
+                        int64_t x_stride, const int64_t* epochs, int n_epochs, const double* means_host,
+                        const int64_t* events, int64_t n_events, int64_t lag_first, int64_t n_lags, double* power_out,
+                        double* phase_out, int64_t out_s_stride, int64_t out_c_stride);
 void host_stage_free(gcwt_plan* p);
 }  // namespace gcwt

@@ -9,7 +9,8 @@
 // identity (what chirpz_dft does on the CPU) with exact integer phase reduction.
 //
 // Reductions of a result on the device, so that only the reduced array crosses the link: moments and
-// time pooling for displays, and scale-averaged band power (band_reduce_kernel).
+// time pooling for displays, scale-averaged band power (band_reduce_kernel) and event-locked power and phase
+// (event_reduce_kernel).
 #include "plan.h"
 #include "common.cuh"
 #include "fft_global.cuh"
@@ -401,6 +402,87 @@ int band_reduce_launch(const void* x_dev, int type, int kind, int64_t n_channels
         if (cx) band_dispatch<double2, double>(x_dev, kind, n_channels, n_samples, s_stride, c_stride, tab, out_dev, out_b_stride, out_c_stride, st);
         else band_dispatch<double, double>(x_dev, kind, n_channels, n_samples, s_stride, c_stride, tab, out_dev, out_b_stride, out_c_stride, st);
     }
+    GCWT_CUDA_OK(cudaGetLastError());
+    return GCWT_OK;
+}
+
+// ----------------------------------------------------------------------------- event-locked power and phase
+// The mean spectrogram around a set of events (stimuli, ripple peaks, trial starts) and the inter-trial phase
+// coherence.  A block owns lags [256 x, 256 x + 256) of one (channel, scale); each thread owns one lag and walks
+// the events in the order given, so a warp's loads are 32 consecutive samples of the row and every sum has one
+// fixed order: no atomics, the same bits on every run.  Events whose sample falls outside the tile
+// [sample0, sample0 + n) are skipped, so a caller can drive a result tile by tile into the same accumulator.
+__device__ __forceinline__ double2 unit_phase(double2 v) {
+    const double m2 = fma(v.x, v.x, v.y * v.y);
+    if (!(m2 > 0.0)) return make_double2(0.0, 0.0);                 // |W| = 0 counts, adds nothing
+    const double r = rsqrt(m2);                                     // 1 / |W| within 1 ulp, no division slow path
+    return make_double2(v.x * r, v.y * r);
+}
+__device__ __forceinline__ double2 unit_phase(float2 v) { return unit_phase(make_double2(v.x, v.y)); }
+
+template <typename In, bool POWER, bool PHASE>
+__global__ void __launch_bounds__(256)
+event_reduce_kernel(const In* __restrict__ x, int64_t n, int64_t s_stride, int64_t c_stride, int64_t sample0,
+                    const int64_t* __restrict__ events, int64_t n_events, int64_t lag_first, int64_t n_lags,
+                    double* __restrict__ acc_power, double2* __restrict__ acc_phase, int64_t as_stride,
+                    int64_t ac_stride) {
+    const int64_t lag = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (lag >= n_lags) return;
+    const In* row = x + (int64_t)blockIdx.z * c_stride + (int64_t)blockIdx.y * s_stride;
+    const int64_t shift = lag_first + lag - sample0;
+    double p = 0.0, re = 0.0, im = 0.0;
+#pragma unroll 4
+    for (int64_t e = 0; e < n_events; ++e) {
+        const int64_t t = __ldg(events + e) + shift;
+        if (t < 0 || t >= n) continue;
+        const In v = row[t];
+        p += mag2(v, POWER);
+        if constexpr (PHASE) {
+            const double2 u = unit_phase(v);
+            re += u.x;
+            im += u.y;
+        }
+    }
+    const int64_t o = (int64_t)blockIdx.z * ac_stride + (int64_t)blockIdx.y * as_stride + lag;
+    acc_power[o] += p;
+    if constexpr (PHASE) {
+        const double2 a = acc_phase[o];
+        acc_phase[o] = make_double2(a.x + re, a.y + im);
+    }
+}
+
+template <typename In, bool POWER, bool PHASE>
+static void event_launch(const void* x, int64_t n_ch, int n_scales, int64_t n, int64_t s_stride, int64_t c_stride,
+                         int64_t sample0, const int64_t* events, int64_t n_events, int64_t lag_first, int64_t n_lags,
+                         double* acc_power, double2* acc_phase, int64_t as_stride, int64_t ac_stride, cudaStream_t st) {
+    for (int64_t c0 = 0; c0 < n_ch; c0 += 65535) {                   // gridDim.z limit
+        const int64_t rows = std::min<int64_t>(65535, n_ch - c0);
+        dim3 grid((unsigned)((n_lags + 255) / 256), (unsigned)n_scales, (unsigned)rows);
+        event_reduce_kernel<In, POWER, PHASE><<<grid, 256, 0, st>>>(
+            (const In*)x + c0 * c_stride, n, s_stride, c_stride, sample0, events, n_events, lag_first, n_lags,
+            acc_power + c0 * ac_stride, PHASE ? acc_phase + c0 * ac_stride : nullptr, as_stride, ac_stride);
+        count_launch();
+    }
+}
+
+int event_reduce_launch(const void* x_dev, int type, int kind, int64_t n_channels, int n_scales, int64_t n_samples,
+                        int64_t s_stride, int64_t c_stride, int64_t sample0, const int64_t* events_dev, int64_t n_events,
+                        int64_t lag_first, int64_t n_lags, double* acc_power, double2* acc_phase, int64_t as_stride,
+                        int64_t ac_stride, cudaStream_t st) {
+    if (n_events == 0) return GCWT_OK;
+    const bool f32 = type == GCWT_F32;
+#define GCWT_EVENTS(In, POWER, PHASE)                                                                                 \
+    event_launch<In, POWER, PHASE>(x_dev, n_channels, n_scales, n_samples, s_stride, c_stride, sample0, events_dev, \
+                                   n_events, lag_first, n_lags, acc_power, acc_phase, as_stride, ac_stride, st)
+    if (kind == GCWT_OUT_COMPLEX) {
+        if (acc_phase) { if (f32) GCWT_EVENTS(float2, false, true); else GCWT_EVENTS(double2, false, true); }
+        else { if (f32) GCWT_EVENTS(float2, false, false); else GCWT_EVENTS(double2, false, false); }
+    } else if (kind == GCWT_OUT_POWER) {
+        if (f32) GCWT_EVENTS(float, true, false); else GCWT_EVENTS(double, true, false);
+    } else {
+        if (f32) GCWT_EVENTS(float, false, false); else GCWT_EVENTS(double, false, false);
+    }
+#undef GCWT_EVENTS
     GCWT_CUDA_OK(cudaGetLastError());
     return GCWT_OK;
 }

@@ -12,7 +12,7 @@ import numpy as np
 
 from . import _lib
 
-__all__ = ["CwtPlan", "scale_tables", "band_tables", "OUT_KINDS"]
+__all__ = ["CwtPlan", "scale_tables", "band_tables", "event_windows", "OUT_KINDS"]
 
 OUT_KINDS = {"complex": _lib.OUT_COMPLEX, "amplitude": _lib.OUT_AMPLITUDE, "power": _lib.OUT_POWER}
 BAND_REDUCE = ("mean", "sum")
@@ -51,6 +51,45 @@ def band_tables(frequencies, bands, reduce="mean"):
     count = np.asarray(count, dtype=np.int32)
     weights = np.concatenate([np.full(c, 1.0 / c if reduce == "mean" else 1.0) for c in count])
     return np.asarray(first, dtype=np.int32), count, np.ascontiguousarray(weights, dtype=np.float64)
+
+
+def event_windows(time, events_s, window_s, epoch_bounds, fs):
+    """Map events in seconds to sample indices for gcwt_execute_host_events / gcwt_event_reduce: ``(samples,
+    kept_mask, lag_first, n_lags)``.
+
+    Each event goes to its nearest timestamp of ``time``; one more than half a sample period from every timestamp
+    (inside a gap) is dropped.  ``window_s = (t_pre, t_post)`` gives ``lag_first = round(t_pre * fs)`` and ``n_lags =
+    round(t_post * fs) - lag_first + 1``.  An event whose window ``[sample + lag_first, sample + lag_first + n_lags)``
+    leaves its epoch (``epoch_bounds``: (E, 2) [start, stop) sample indices) is dropped as well.  ``samples`` holds
+    the kept events' indices in the caller's order, ``kept_mask`` one flag per given event."""
+    try:
+        t_pre, t_post = (float(v) for v in window_s)
+    except (TypeError, ValueError):
+        raise ValueError("'event_window' must be a (t_pre, t_post) pair in seconds") from None
+    fs = float(fs)
+    lag_first = int(round(t_pre * fs))
+    n_lags = int(round(t_post * fs)) - lag_first + 1
+    if n_lags < 1:
+        raise ValueError("event window ({}, {}) s holds no sample at {} Hz".format(t_pre, t_post, fs))
+    t = np.asarray(time, dtype=np.float64).ravel()
+    ev = np.asarray(events_s, dtype=np.float64).ravel()
+    if ev.size == 0:
+        raise ValueError("'events' is empty")
+    if not np.all(np.isfinite(ev)):
+        raise ValueError("'events' must be finite times in seconds")
+    # nearest timestamp: the one at or after the event, or the one before it
+    hi = np.clip(np.searchsorted(t, ev), 0, t.size - 1)
+    lo = np.clip(hi - 1, 0, t.size - 1)
+    idx = np.where(np.abs(t[lo] - ev) <= np.abs(t[hi] - ev), lo, hi)
+    kept = np.abs(t[idx] - ev) <= 0.5 / fs * (1 + 1e-9)        # an event midway between two samples is kept
+    bounds = np.asarray(epoch_bounds, dtype=np.int64).reshape(-1, 2)
+    w0 = idx + lag_first
+    ep = np.clip(np.searchsorted(bounds[:, 0], w0, side="right") - 1, 0, None)
+    kept &= (w0 >= bounds[ep, 0]) & (w0 + n_lags <= bounds[ep, 1])
+    if not kept.any():
+        raise ValueError("no event has its whole window ({}, {}) s inside one epoch of the recording".format(
+            t_pre, t_post))
+    return idx[kept].astype(np.int64), kept, lag_first, n_lags
 
 
 def _band_args(first, count, weights):
@@ -359,6 +398,62 @@ class CwtPlan:
             res.stride(0), int(first.size), first.ctypes.data, count.ctypes.data, weights.ctypes.data,
             out.data_ptr(), n, first.size * n, res.device.index, st))
         return out
+
+    def execute_host_events(self, x, events, lag_first, n_lags, epochs=None, means=None):
+        """As :meth:`execute_host`, but every tile is reduced on the device to event-locked sums
+        (gcwt_execute_host_events) and only the means cross the link: ``(power, phase)``, power (channels, scales,
+        n_lags) float64 = mean over events of |W(c, s, e + lag_first + l)|**2, phase the same shape complex128 = mean
+        of W / |W| for complex plans (its modulus is the inter-trial phase coherence), else None.  ``events`` are
+        ascending sample indices whose windows each lie inside one epoch."""
+        n_ch, n, xa, ea, mp = self._host_args(x, means, epochs)
+        ev = np.ascontiguousarray(events, dtype=np.int64).ravel()
+        L = int(n_lags)
+        power = np.empty((n_ch, self.n_scales, L), dtype=np.float64)
+        phase = np.empty((n_ch, self.n_scales, L), dtype=np.complex128) if self.output == "complex" else None
+        _lib.check(self.lib.gcwt_execute_host_events(
+            self._h, *xa, *ea, mp, ev.ctypes.data, ev.size, int(lag_first), L, power.ctypes.data,
+            None if phase is None else phase.ctypes.data, L, self.n_scales * L))
+        return power, phase
+
+    def event_reduce(self, res, events, lag_first, n_lags, *, sample0=0, power=None, phase=None):
+        """Event-locked sums of a device-resident (channels, scales, samples) result ``res`` (a CUDA tensor with unit
+        sample stride, possibly one tile of a longer result starting at sample ``sample0``), through
+        gcwt_event_reduce on the current stream: adds |W(c, s, e + lag_first + l)|**2 into ``power`` (float64) and,
+        for a complex ``res``, W / |W| into ``phase`` (complex128), both (channels, scales, n_lags) CUDA tensors,
+        allocated as zeros when not given.  Only the event samples inside the tile contribute, so tiles can be added
+        into the same accumulators one after another.  Returns ``(power, phase or None)``: sums, not means."""
+        torch = _torch()
+        if not res.is_cuda or res.dim() != 3 or res.stride(2) != 1 or \
+                res.dtype not in (torch.float32, torch.float64, torch.complex64, torch.complex128):
+            raise ValueError("event_reduce needs a (channels, scales, samples) float / complex CUDA tensor with unit "
+                             "sample stride")
+        n_ch, S, n = res.shape
+        L = int(n_lags)
+        cx = res.is_complex()
+        if isinstance(events, torch.Tensor):
+            ev = events.to(device=res.device, dtype=torch.int64).contiguous().view(-1)
+        else:
+            ev = torch.from_numpy(np.ascontiguousarray(events, dtype=np.int64).ravel()).to(res.device)
+        if power is None:
+            power = torch.zeros((n_ch, S, L), dtype=torch.float64, device=res.device)
+        if cx and phase is None:
+            phase = torch.zeros((n_ch, S, L), dtype=torch.complex128, device=res.device)
+        if power.dtype != torch.float64 or power.shape != (n_ch, S, L) or power.stride(2) != 1 or not power.is_cuda:
+            raise ValueError("power must be a float64 (channels, scales, n_lags) CUDA tensor with unit lag stride")
+        if phase is not None:
+            if not cx:
+                raise ValueError("phase needs a complex result")
+            if phase.dtype != torch.complex128 or phase.shape != (n_ch, S, L) or phase.stride() != power.stride() \
+                    or not phase.is_cuda:
+                raise ValueError("phase must be a complex128 CUDA tensor of power's shape and strides")
+        rdt = {torch.complex64: torch.float32, torch.complex128: torch.float64}.get(res.dtype, res.dtype)
+        kind = _lib.OUT_COMPLEX if cx else (_lib.OUT_POWER if self.output == "power" else _lib.OUT_AMPLITUDE)
+        st = torch.cuda.current_stream(res.device).cuda_stream
+        _lib.check(self.lib.gcwt_event_reduce(
+            res.data_ptr(), _lib.F32 if rdt == torch.float32 else _lib.F64, kind, n_ch, S, n, res.stride(1),
+            res.stride(0), int(sample0), ev.data_ptr(), ev.numel(), int(lag_first), L, power.data_ptr(),
+            None if phase is None else phase.data_ptr(), power.stride(1), power.stride(0), res.device.index, st))
+        return power, phase
 
     def host_stats(self):
         """{wall_ms, pinned_destination, tiles, bytes_out} of the last execute_host."""

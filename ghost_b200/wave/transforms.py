@@ -10,7 +10,8 @@ into libghostcwt.so.
 Extensions (keyword-only, all optional): ``dtype`` (float64 reproduces the reference to
 1e-10; float32 is the HBM-roofline path), ``output`` ('amplitude' | 'power' | 'complex'),
 ``device``, ``multichannel`` (rows of a 2-D array are channels) and ``keep_on_device``; ``bands`` keeps
-only scale-averaged band power (``band_power``), reduced on the device.
+only scale-averaged band power (``band_power``), reduced on the device; ``events`` / ``event_window`` keep only
+event-locked power and inter-trial phase coherence (``event_power``, ``itc``), reduced on the device.
 """
 from __future__ import annotations
 
@@ -94,6 +95,11 @@ class ContinuousWaveletTransform(WaveletTransform):
         self._host = None            # numpy view of the result, filled lazily
         self._band_power = None      # (B, N) or (C, B, N) after transform(bands=...): the only result kept
         self._band_frequencies = None
+        self._event_power = None     # (S, L) or (C, S, L) after transform(events=...): the only result kept
+        self._event_phase = None
+        self._event_lags = None
+        self._events_used = None
+        self._epoch_bounds = None
         self._pooled = False         # the result was pooled over time (pool_width)
         self._multichannel = False
         self._time_auto = None       # (n, fs) when self._time is the implicit arange(n) / fs
@@ -144,7 +150,7 @@ class ContinuousWaveletTransform(WaveletTransform):
     def transform(self, data, *, timestamps=None, fs=None, freq_limits=None, freqs=None,
                   voices_per_octave=None, parallel=None, verbose=None, multichannel=None,
                   keep_on_device=None, out=None, pool_width=None, pool=None, bands=None, band_reduce=None,
-                  **kwargs):
+                  events=None, event_window=None, **kwargs):
         """Continuous wavelet transform of one recording.
 
         Parameters as the reference (transforms.py:59-106): ``data`` is an ndarray with
@@ -172,8 +178,21 @@ class ContinuousWaveletTransform(WaveletTransform):
         ``multichannel``, in the plan's dtype; ``band_frequencies`` lists each band's grid frequencies.
         ``amplitude``, ``power`` and ``coefficients`` are then not available.
 
+        ``events=[t, ...]`` (seconds on the ``time`` axis) with ``event_window=(t_pre, t_post)`` (seconds, t_pre may
+        be negative) keeps only event-locked averages, reduced on the device tile by tile so that only (scales x lags)
+        per channel crosses the link: ``event_power`` = mean over events of |W|^2 at every lag, ``event_phase`` = mean
+        of W / |W| (output='complex' only, else None) and ``itc`` = its modulus, the inter-trial phase coherence;
+        shaped (S, L), or (C, S, L) with ``multichannel``, float64 / complex128; ``event_lags`` holds the lags in
+        seconds.  Each event is taken at its nearest sample; events in a gap, and events whose window leaves their
+        epoch, are dropped (with a warning), and ``events_used`` lists the event times averaged.  ``amplitude``,
+        ``power`` and ``coefficients`` are then not available.
+
         Returns None; results are read from the properties.
         """
+        if (events is None) != (event_window is None):
+            raise ValueError("'events' and 'event_window' go together")
+        if events is not None and (bands is not None or pool_width is not None or out is not None or keep_on_device):
+            raise ValueError("'events' cannot be combined with 'bands', 'pool_width', 'out' or 'keep_on_device'")
         if bands is None:
             if band_reduce is not None:
                 raise ValueError("'band_reduce' needs 'bands'")
@@ -233,10 +252,18 @@ class ContinuousWaveletTransform(WaveletTransform):
                                  dtype=np.float64)
         self._frequencies = frequencies
         self._band_power = self._band_frequencies = None
+        self._event_power = self._event_phase = self._event_lags = self._events_used = None
+        self._epoch_bounds = epoch_bounds
         self._pooled = pool_width is not None
         if bands is not None:
             from ..engine import band_tables
             b_first, b_count, b_weights = band_tables(frequencies, bands, "mean" if band_reduce is None else band_reduce)
+        if events is not None:
+            from ..engine import event_windows
+            ev_samples, ev_kept, lag_first, n_lags = event_windows(self._time, events, event_window, epoch_bounds, fs)
+            if not ev_kept.all():
+                logging.warning("events: kept {} of {}; the others lie in a gap or their window leaves the "
+                                "recording's epoch".format(int(ev_kept.sum()), ev_kept.size))
         if frequencies.size == 0:
             # data too short for any scale: the reference ends up with a (0, N) array
             self._multichannel = bool(multichannel)
@@ -255,7 +282,16 @@ class ContinuousWaveletTransform(WaveletTransform):
         self._result = None
         start_time = _time.time()
         x_in = x_host if x_host.dtype == in_dtype else x_host.astype(in_dtype)
-        if bands is not None:
+        if events is not None:
+            # event-locked averages only: every tile is added into (scales x lags) sums per channel on the device
+            # and only those cross the link, once per channel group
+            power, phase = plan.execute_host_events(x_in, np.sort(ev_samples), lag_first, n_lags, epochs=epoch_bounds)
+            self._event_power = power if multichannel else power[0]
+            if phase is not None:
+                self._event_phase = phase if multichannel else phase[0]
+            self._event_lags = (lag_first + np.arange(n_lags)) / float(fs)
+            self._events_used = np.asarray(events, dtype=np.float64).ravel()[ev_kept]
+        elif bands is not None:
             # band power only: every tile is reduced over scales on the device and (bands x samples) per channel
             # travels to the host, epochs and zeros between them as for the full result
             res = plan.execute_host_bands(x_in, b_first, b_count, b_weights, epochs=epoch_bounds)
@@ -312,6 +348,9 @@ class ContinuousWaveletTransform(WaveletTransform):
         if self._band_power is not None:
             raise ValueError("transform(bands=...) kept only band_power; run transform without 'bands' for the "
                              "full-rate amplitude, power or coefficients")
+        if self._event_power is not None:
+            raise ValueError("transform(events=...) kept only the event-locked averages; run transform without "
+                             "'events' for the full-rate amplitude, power or coefficients")
 
     def _materialise(self):
         self._check_full_rate()
@@ -410,6 +449,72 @@ class ContinuousWaveletTransform(WaveletTransform):
                 res[:, b] = np.tensordot(weights[off:off + c], p, axes=(0, 1))
                 off += c
         return res if self._multichannel else res[0]
+
+    @property
+    def event_power(self):
+        """Mean |W|^2 over the events of the last ``transform(events=...)`` at every (scale, lag): (S, L), or
+        (C, S, L) with ``multichannel``, float64; None after any other transform."""
+        return self._event_power
+
+    @property
+    def event_phase(self):
+        """Mean of W / |W| over the events (complex128, shaped as ``event_power``); output='complex' only."""
+        return self._event_phase
+
+    @property
+    def itc(self):
+        """Inter-trial phase coherence |mean W / |W||: 1 where the phase is locked to the events, about
+        1 / sqrt(n_events) where it is not.  Needs output='complex'; None otherwise."""
+        return None if self._event_phase is None else np.abs(self._event_phase)
+
+    @property
+    def event_lags(self):
+        """The lags of ``event_power``'s last axis, in seconds relative to the events."""
+        return self._event_lags
+
+    @property
+    def events_used(self):
+        """The event times (seconds, as given) that ``event_power`` averages."""
+        return self._events_used
+
+    def event_average(self, events, event_window):
+        """Event-locked averages of the existing full-rate result: ``(power, phase)`` as ``transform(events=...,
+        event_window=...)`` computes them (``phase`` None unless output='complex'), shaped (S, L), or (C, S, L) with
+        ``multichannel``.  Events map to samples as there (engine.event_windows).  A device-resident result
+        (``keep_on_device=True``) is reduced on the GPU and only the means are copied back; a host-resident one is
+        reduced in numpy in float64."""
+        from ..engine import event_windows
+        self._check_full_rate()
+        if self._frequencies is None or (self._result is None and self._host is None):
+            raise ValueError("no full-rate result: call transform() first")
+        if self._pooled:
+            raise ValueError("the result was pooled over time (pool_width): event averages need the full-rate result")
+        samples, _, lag_first, n_lags = event_windows(self._time, events, event_window, self._epoch_bounds, self._fs)
+        cx = self._output == "complex"
+        if self._result is not None and self._host is None:
+            power, phase = self.last_plan.event_reduce(self._result, samples, lag_first, n_lags)
+            power = (power / samples.size).cpu().numpy()
+            phase = None if phase is None else (phase / samples.size).cpu().numpy()
+        else:
+            data = self._host if self._multichannel else self._host[None]
+            power = np.zeros(data.shape[:2] + (n_lags,))
+            phase = np.zeros(power.shape, dtype=np.complex128) if cx else None
+            for s in samples:
+                w = data[:, :, s + lag_first:s + lag_first + n_lags]
+                if cx:
+                    w = w.astype(np.complex128)
+                    power += np.square(w.real) + np.square(w.imag)
+                    m = np.abs(w)
+                    phase += np.where(m > 0, w / np.where(m > 0, m, 1.0), 0.0)
+                else:
+                    w = w.astype(np.float64)
+                    power += w if self._output == "power" else np.square(w)
+            power /= samples.size
+            if cx:
+                phase /= samples.size
+        if self._multichannel:
+            return power, phase
+        return power[0], None if phase is None else phase[0]
 
     @property
     def time(self):

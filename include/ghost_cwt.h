@@ -186,6 +186,40 @@ int gcwt_execute_host_bands(gcwt_plan *plan, const void *x, int32_t in_type,
                             const double *weights,
                             void *out, int64_t out_band_stride, int64_t out_channel_stride);
 
+/* Event-locked averages: the mean spectrogram around a set of events (stimuli, ripple peaks, spikes, trial starts)
+ * and the inter-trial phase coherence, without the full (channels, scales, samples) result crossing the link.
+ * Events are sample indices; event e covers the n_lags samples e + lag_first + l, l = 0 .. n_lags - 1 (lag_first
+ * may be negative).  |W|^2 follows the kind as in gcwt_band_reduce; the phase term is W / |W| (0 where |W| = 0, and
+ * still counted).  Sums are fp64 and in one fixed order: the same bits on every run.
+ *
+ * gcwt_event_reduce: ADDS, for every event whose sample e + lag_first + l lies in the tile
+ *   [sample0, sample0 + n_samples), |W[c, s, e + lag_first + l - sample0]|^2 to acc_power_dev[c * acc_channel_stride +
+ *   s * acc_scale_stride + l] (double) and, when acc_phase_dev is not NULL (complex coefficients only), W / |W| to
+ *   acc_phase_dev at the same index (double2, 16-byte aligned); W[c, s, t] at coef_dev[c * channel_stride +
+ *   s * scale_stride + t] in elements of coef_type (float2 / double2 for complex).  Events in any order, duplicates
+ *   count twice.  A caller can drive a result tile by tile into one accumulator; the means are sums / n_events.
+ *   Asynchronous on `stream`; at most 65535 scales.
+ * gcwt_execute_host_events: gcwt_execute_host (epochs, means) whose tiles are reduced on the device; writes MEANS over
+ *   the n_events events: power_out[c * out_channel_stride + s * out_scale_stride + l] (host double) and, for complex
+ *   plans, phase_out at the same index (host complex double, re/im interleaved; NULL skips the phase).  Events must
+ *   ascend and each window must lie inside one epoch; otherwise GCWT_ERR_ARG names the event, before any device work.
+ *   The coefficients summed are those gcwt_execute_host would have written, accuracy-guard re-computations included.
+ *   gcwt_host_stats reports bytes_out = the bytes of the means, and 0 for a pinned destination (they arrive through
+ *   the plan's pinned ring). */
+int gcwt_event_reduce(const void *coef_dev, int32_t coef_type, int32_t coef_kind,
+                      int64_t n_channels, int32_t n_scales, int64_t n_samples,
+                      int64_t scale_stride, int64_t channel_stride, int64_t sample0,
+                      const int64_t *events_dev, int64_t n_events, int64_t lag_first, int64_t n_lags,
+                      double *acc_power_dev, double *acc_phase_dev,
+                      int64_t acc_scale_stride, int64_t acc_channel_stride,
+                      int32_t device, void *stream);
+int gcwt_execute_host_events(gcwt_plan *plan, const void *x, int32_t in_type,
+                             int64_t n_channels, int64_t n_samples, int64_t x_stride,
+                             const int64_t *epoch_bounds, int32_t n_epochs, const double *means_host,
+                             const int64_t *events_host, int64_t n_events, int64_t lag_first, int64_t n_lags,
+                             double *power_out, double *phase_out,
+                             int64_t out_scale_stride, int64_t out_channel_stride);
+
 /* Diagnostics of the last gcwt_execute_host: out4 = {wall ms, 1 if `out` was pinned (direct DMA) else 0,
  * tiles, bytes copied to the host}. */
 int gcwt_host_stats(const gcwt_plan *plan, double *out4);
