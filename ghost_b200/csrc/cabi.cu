@@ -115,6 +115,18 @@ static int check_exec_args(const gcwt_plan* plan, const void* x, int in_type, in
     return GCWT_OK;
 }
 
+// the checks both device reductions make on their coefficients: non-NULL pointers, type, kind and positive sizes;
+// the error texts name the entry point (`who`), its pointers (`ptrs`) and its sizes (`sizes`)
+static int check_coef_args(const char* who, bool ptrs_ok, const char* ptrs, int type, int kind, bool sizes_ok, const char* sizes) {
+    const std::string msg = !ptrs_ok ? std::string(ptrs) + " is NULL"
+                          : type != GCWT_F32 && type != GCWT_F64 ? "coef_type must be GCWT_F32 or GCWT_F64"
+                          : kind < GCWT_OUT_COMPLEX || kind > GCWT_OUT_POWER ? "bad coef_kind"
+                          : !sizes_ok ? std::string(sizes) + " must be positive" : "";
+    if (msg.empty()) return GCWT_OK;
+    set_error(std::string(who) + ": " + msg);
+    return GCWT_ERR_ARG;
+}
+
 }  // namespace gcwt
 
 using namespace gcwt;
@@ -359,12 +371,10 @@ int gcwt_band_reduce(const void* coef_dev, int32_t coef_type, int32_t coef_kind,
                      int64_t scale_stride, int64_t channel_stride, int32_t n_bands, const int32_t* band_first,
                      const int32_t* band_count, const double* weights, void* out_dev, int64_t out_band_stride,
                      int64_t out_channel_stride, int32_t device, void* stream) {
-    if (!coef_dev || !out_dev) { set_error("band_reduce: coef/out is NULL"); return GCWT_ERR_ARG; }
-    if (coef_type != GCWT_F32 && coef_type != GCWT_F64) { set_error("band_reduce: coef_type must be GCWT_F32 or GCWT_F64"); return GCWT_ERR_ARG; }
-    if (coef_kind < GCWT_OUT_COMPLEX || coef_kind > GCWT_OUT_POWER) { set_error("band_reduce: bad coef_kind"); return GCWT_ERR_ARG; }
-    if (n_channels <= 0 || n_samples <= 0) { set_error("band_reduce: n_channels and n_samples must be positive"); return GCWT_ERR_ARG; }
     BandTable tab;
-    int rc = band_table_build(n_bands, band_first, band_count, weights, &tab, "band_reduce");
+    int rc = check_coef_args("band_reduce", coef_dev && out_dev, "coef/out", coef_type, coef_kind,
+                             n_channels > 0 && n_samples > 0, "n_channels and n_samples");
+    if (rc == GCWT_OK) rc = band_table_build(n_bands, band_first, band_count, weights, &tab, "band_reduce");
     if (rc) return rc;
     if (scale_stride < n_samples || (n_channels > 1 && channel_stride < (int64_t)tab.rows * scale_stride)) {
         set_error("band_reduce: scale_stride below n_samples, or channel_stride below the rows the bands read"); return GCWT_ERR_ARG;
@@ -404,13 +414,11 @@ int gcwt_event_reduce(const void* coef_dev, int32_t coef_type, int32_t coef_kind
                       const int64_t* events_dev, int64_t n_events, int64_t lag_first, int64_t n_lags,
                       double* acc_power_dev, double* acc_phase_dev, int64_t acc_scale_stride,
                       int64_t acc_channel_stride, int32_t device, void* stream) {
-    if (!coef_dev || !events_dev || !acc_power_dev) { set_error("event_reduce: coef/events/acc_power is NULL"); return GCWT_ERR_ARG; }
-    if (coef_type != GCWT_F32 && coef_type != GCWT_F64) { set_error("event_reduce: coef_type must be GCWT_F32 or GCWT_F64"); return GCWT_ERR_ARG; }
-    if (coef_kind < GCWT_OUT_COMPLEX || coef_kind > GCWT_OUT_POWER) { set_error("event_reduce: bad coef_kind"); return GCWT_ERR_ARG; }
+    const int rc = check_coef_args("event_reduce", coef_dev && events_dev && acc_power_dev, "coef/events/acc_power", coef_type,
+                                   coef_kind, n_channels > 0 && n_scales > 0 && n_samples > 0 && n_events > 0 && n_lags > 0,
+                                   "n_channels, n_scales, n_samples, n_events and n_lags");
+    if (rc) return rc;
     if (acc_phase_dev && coef_kind != GCWT_OUT_COMPLEX) { set_error("event_reduce: a phase accumulator needs complex coefficients"); return GCWT_ERR_ARG; }
-    if (n_channels <= 0 || n_scales <= 0 || n_samples <= 0 || n_events <= 0 || n_lags <= 0) {
-        set_error("event_reduce: n_channels, n_scales, n_samples, n_events and n_lags must be positive"); return GCWT_ERR_ARG;
-    }
     if (n_scales > 65535) { set_error("event_reduce: at most 65535 scales"); return GCWT_ERR_ARG; }
     if (scale_stride < n_samples || (n_channels > 1 && channel_stride < (int64_t)n_scales * scale_stride)) {
         set_error("event_reduce: scale_stride below n_samples, or channel_stride below n_scales rows"); return GCWT_ERR_ARG;

@@ -7,14 +7,15 @@
 // Results larger than device memory (config 3: 295 GB per GPU) therefore work, the device holds one
 // channel group's samples plus two tiles, and the link -- not the kernels -- sets the pace.
 //
+// One walk (walk_tiles) computes the tiles of every host call; its output decides what happens to each tile.
 // What travels is the tile itself (full rate) or its reduction on the device (pooled bins or band power), and
-// every output takes the same route:
+// every such output takes the same route (Streamed):
 //   pinned destination (cudaHostAlloc / cudaHostRegister / torch pin_memory): rows are written by DMA,
 //     one cudaMemcpy2DAsync per channel of a tile;
 //   pageable destination (a plain numpy array): tiles land in a plan-owned pinned ring by DMA and a few
 //     host threads copy the rows out (which also first-touches the caller's pages in parallel).
-// Event-locked averages (host_execute_events) use the same tiles but send nothing per tile: each tile is added into
-// a device accumulator of (channels x scales x lags) and only that crosses the link, once per channel group.
+// Event-locked averages (EventSums) send nothing per tile: each tile is added into a device accumulator of
+// (channels x scales x lags) and only that crosses the link, once per channel group.
 //
 // Epochs (transforms.py:202-204): every epoch is a zero-padded convolution of its own; samples outside
 // all epochs are zero.  The mean is the channel's mean over ALL samples (transforms.py:142-143).
@@ -90,8 +91,8 @@ static int check_epochs(const int64_t* epochs, int n_epochs, int64_t n) {
 }
 
 // a tile is a group of g channels x all scales x a stretch of `tile` samples, computed with `halo` real samples
-// on each side where its epoch has them
-struct TileGeometry { int64_t g, tile, halo; };
+// on each side where its epoch has them; on the device its rows lie `alloc` elements apart
+struct TileGeometry { int64_t g, tile, halo, alloc; };
 
 static TileGeometry tile_geometry(const gcwt_plan* p, int64_t n_channels, int64_t n, size_t out_el, int64_t pool_width) {
     const int S = p->n_scales;
@@ -113,21 +114,8 @@ static TileGeometry tile_geometry(const gcwt_plan* p, int64_t n_channels, int64_
     }
     if (pool_width > 0 && t.tile < n)                             // tiles end on bin boundaries
         t.tile = std::max<int64_t>(pool_width, t.tile / pool_width * pool_width);
+    t.alloc = (t.tile + 3) & ~int64_t(3);                         // rows of a tile stay 16-byte aligned
     return t;
-}
-
-// staging of one call: full-rate tiles of `tile_bytes`, reduced tiles of `red_bytes` and a pinned ring of
-// `ring_bytes` per slot (0: not needed by this call); buffers only grow
-static int grow_staging(gcwt_plan::HostStage& h, size_t in_bytes, size_t tile_bytes, size_t red_bytes, size_t ring_bytes,
-                        int64_t g) {
-    int rc = grow_device(&h.d_in, &h.in_bytes, in_bytes, "execute_host");
-    for (int b = 0; b < 2 && rc == GCWT_OK; ++b) {
-        rc = grow_device(&h.d_out[b], &h.out_bytes[b], tile_bytes, "execute_host");
-        if (rc == GCWT_OK) rc = grow_device(&h.d_red[b], &h.red_bytes[b], red_bytes, "execute_host");
-        if (rc == GCWT_OK) rc = grow_pinned(&h.h_ring[b], &h.ring_bytes[b], ring_bytes, "execute_host");
-    }
-    if (rc == GCWT_OK) rc = grow_device((void**)&h.d_means, &h.means_bytes, sizeof(double) * g, "execute_host");
-    return rc;
 }
 
 // the compute and copy streams and the two slots' events, created on a plan's first host call
@@ -179,95 +167,145 @@ static void zero_gaps(char* out, const int64_t* epochs, int n_epochs, int64_t n,
     }
 }
 
-int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n, int64_t x_stride,
-                 const int64_t* epochs, int n_epochs, const double* means_host, void* out, int64_t s_stride,
-                 int64_t c_stride, int64_t pool_width, int pool_mode, const BandTable* bands) {
-    // pool_width > 0: `out` is a float64 array of ceil(n / pool_width) bins per row; every tile is reduced on the
-    // device (mean or max over pool_width consecutive samples) and only the bins travel to the host.
-    // bands: `out` holds (channels x bands x samples) of the plan's real type (s_stride is the band stride); every
-    // tile is band-reduced on the device and only the band rows travel.  The tile geometry stays that of the
-    // full-rate path, so every coefficient summed is the one gcwt_execute_host would have written.
+// The tiles of one host call: channel groups of geo.g channels, each epoch of a group, tiles of geo.tile samples in
+// an epoch, alternating between the slots d_out[0] and d_out[1].  Out says what the call makes of them: prepare(geo,
+// epochs, n_epochs) sets up its buffers; slot_free(b) does what must happen before d_out[b] is overwritten;
+// group_begin / group_end(c0, gc) frame the tiles of channels [c0, c0 + gc); tile(b, c0, gc, a, len) works on the
+// tile of samples [a, a + len) in d_out[b], on the copy stream; pinned and bytes_out go to host_stats.
+template <class Out>
+static int walk_tiles(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n, int64_t x_stride,
+                      const int64_t* epochs, int n_epochs, const double* means_host, int64_t pool_width, Out& out) {
     gcwt_plan::HostStage& h = p->host;
     const auto t_begin = std::chrono::steady_clock::now();
     const int S = p->n_scales;
     const size_t in_el = in_type == GCWT_F32 ? 4 : 8;
     const size_t real_el = p->compute_type == GCWT_F32 ? 4 : 8;
     const size_t out_el = p->out_kind == GCWT_OUT_COMPLEX ? 2 * real_el : real_el;
-    const bool pooled = pool_width > 0, reduced = pooled || bands;
     int64_t one_epoch[2] = {0, n};
     if (!epochs || n_epochs <= 0) { epochs = one_epoch; n_epochs = 1; }
     int rc = check_epochs(epochs, n_epochs, n);
-    if (rc) return rc;
-    if (pooled) {
-        if (p->out_kind == GCWT_OUT_COMPLEX) { set_error("execute_host: pooling needs amplitude or power output"); return GCWT_ERR_ARG; }
-        if (n_epochs != 1 || epochs[0] != 0 || epochs[1] != n) {
-            set_error("execute_host: pooling across epoch gaps is not supported (pool the full-rate result instead)");
-            return GCWT_ERR_UNSUPPORTED;
-        }
-    }
-    rc = ensure_streams(h);
+    if (rc == GCWT_OK) rc = ensure_streams(h);
     if (rc) return rc;
     const TileGeometry geo = tile_geometry(p, n_channels, n, out_el, pool_width);
-    const int64_t tile_alloc = (geo.tile + 3) & ~int64_t(3);      // rows of a tile stay 16-byte aligned
+    rc = grow_device(&h.d_in, &h.in_bytes, (size_t)geo.g * n * in_el, "execute_host");
+    for (int b = 0; b < 2 && rc == GCWT_OK; ++b)
+        rc = grow_device(&h.d_out[b], &h.out_bytes[b], (size_t)geo.g * S * geo.alloc * out_el, "execute_host");
+    if (rc == GCWT_OK) rc = grow_device((void**)&h.d_means, &h.means_bytes, sizeof(double) * geo.g, "execute_host");
+    if (rc == GCWT_OK) rc = out.prepare(geo, epochs, n_epochs);
+    if (rc) return rc;
 
+    auto run_tile = [&](int b, int64_t c0, int64_t gc, int64_t a, int64_t len, int64_t halo_l, int64_t halo_r) -> int {
+        int r = out.slot_free(b);
+        if (r) return r;
+        r = gcwt_execute(p, (const char*)h.d_in + (size_t)a * in_el, in_type, gc, len, n, halo_l, halo_r, h.d_means,
+                         h.d_out[b], geo.alloc, (int64_t)S * geo.alloc, h.st_compute);
+        if (r) return r;
+        // ev_done follows the whole of gcwt_execute in stream order, including the accuracy guard's fp64 re-computation
+        // of the failing (channel, scale) pairs (guard_resolve), so the reductions on the copy stream read the corrected
+        // coefficients.  For the same reason band power and event sums are passes of their own and not part of the
+        // fused kernels' epilogue: there they would sum values the guard then replaces.
+        GCWT_CUDA_OK(cudaEventRecord(h.ev_done[b], h.st_compute));
+        GCWT_CUDA_OK(cudaStreamWaitEvent(h.st_copy, h.ev_done[b], 0));
+        return out.tile(b, c0, gc, a, len);
+    };
+
+    int slot = 0;
+    int64_t n_tiles = 0;
+    for (int64_t c0 = 0; c0 < n_channels && rc == GCWT_OK; c0 += geo.g) {
+        const int64_t gc = std::min<int64_t>(geo.g, n_channels - c0);
+        rc = load_group(p, x, in_type, n, x_stride, means_host, c0, gc);
+        if (rc == GCWT_OK) rc = out.group_begin(c0, gc);
+        for (int e = 0; e < n_epochs && rc == GCWT_OK; ++e) {
+            const int64_t e0 = epochs[2 * e], e1 = epochs[2 * e + 1];
+            for (int64_t a = e0; a < e1 && rc == GCWT_OK; a += geo.tile) {
+                const int64_t len = std::min(e1, a + geo.tile) - a;
+                rc = run_tile(slot, c0, gc, a, len, std::min(geo.halo, a - e0), std::min(geo.halo, e1 - a - len));
+                if (rc) break;
+                ++n_tiles;
+                slot ^= 1;
+            }
+        }
+        if (rc == GCWT_OK) rc = out.group_end(c0, gc);
+    }
+    for (int b = 0; b < 2; ++b) {                                  // the last tiles have left both slots
+        const int r = out.slot_free(b);
+        if (rc == GCWT_OK) rc = r;
+    }
+    cudaStreamSynchronize(h.st_copy);
+    cudaStreamSynchronize(h.st_compute);
+    h.last_ms[0] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    h.last_ms[1] = out.pinned ? 1.0 : 0.0;
+    h.last_ms[2] = (double)n_tiles;
+    h.last_ms[3] = out.bytes_out;
+    return rc;
+}
+
+// Full-rate, pooled or band-power tiles, sent to the caller's array `out`.
+// pool_width > 0: `out` is a float64 array of ceil(n / pool_width) bins per row; every tile is reduced on the device
+// (mean or max over pool_width consecutive samples) and only the bins travel to the host.
+// bands: `out` holds (channels x bands x samples) of the plan's real type (s_stride is the band stride); every tile
+// is band-reduced on the device and only the band rows travel.  The tile geometry stays that of the full-rate path,
+// so every coefficient summed is the one gcwt_execute_host would have written.
+struct Streamed {
+    gcwt_plan* p; int64_t n_channels, n; char* out; int64_t s_stride, c_stride, pool_width; int pool_mode;
+    const BandTable* bands;
+    gcwt_plan::HostStage& h = p->host;
+    const int S = p->n_scales;
+    const bool reduced = pool_width > 0 || bands;
+    const bool pinned = is_pinned(out);
+    double bytes_out = 0;
     // What reaches `out`: R rows per channel of `el`-byte elements.  A tile of `len` samples that starts at sample
     // a fills width(len) columns of them from column col(a); on the device its rows are staged `pitch` elements apart.
     const int R = bands ? bands->n_bands : S;
-    const size_t el = bands ? real_el : pooled ? sizeof(double) : out_el;
-    const int64_t pitch = pooled ? (geo.tile + pool_width - 1) / pool_width : tile_alloc;
-    auto col = [&](int64_t a) { return pooled ? a / pool_width : a; };
-    auto width = [&](int64_t len) { return pooled ? (len + pool_width - 1) / pool_width : len; };
-    // the optional reduction of the full-rate tile in slot b into d_red[b], on the copy stream
-    auto reduce = [&](int b, int64_t gc, int64_t len) -> int {
-        if (pooled)
-            return pool_rows_launch(h.d_out[b], p->compute_type, gc * S, len, tile_alloc, pool_width, pool_mode, 0,
-                                    (double*)h.d_red[b], pitch, h.st_copy);
-        return band_reduce_launch(h.d_out[b], p->compute_type, p->out_kind, gc, len, tile_alloc, (int64_t)S * tile_alloc,
-                                  *bands, h.d_red[b], pitch, (int64_t)R * pitch, h.st_copy);
-    };
-
-    const bool pinned = is_pinned(out);
-    const size_t stage_bytes = (size_t)geo.g * R * pitch * el;
-    rc = grow_staging(h, (size_t)geo.g * n * in_el, (size_t)geo.g * S * tile_alloc * out_el, reduced ? stage_bytes : 0,
-                      pinned ? 0 : stage_bytes, geo.g);
-    if (rc) return rc;
-    // copier threads of the pageable path (measured on a 16-core host, 6.9 GB per call: 8 threads 34 GB/s, see DESIGN.md)
-    int n_threads = (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency() > 2 ? std::thread::hardware_concurrency() - 2 : 1u));
-    if (const char* e = getenv("GCWT_HOST_THREADS")) n_threads = std::max(1, atoi(e));
-    zero_gaps((char*)out, epochs, n_epochs, n, n_channels, R, s_stride, c_stride, el);
-
+    const size_t real_el = p->compute_type == GCWT_F32 ? 4 : 8;
+    const size_t el = bands ? real_el : pool_width > 0 ? sizeof(double) : p->out_kind == GCWT_OUT_COMPLEX ? 2 * real_el : real_el;
+    int64_t pitch = 0, alloc = 0;
+    int n_threads = 1;
     bool live[2] = {false, false};
-    struct Copiers {                                               // joined on every return path (an early error return
-        std::thread t[2];                                          // must not destroy a running thread)
-        ~Copiers() { for (auto& th : t) if (th.joinable()) th.join(); }
-        std::thread& operator[](int i) { return t[i]; }
-    } copier;
-    auto finish = [&](int b) -> int {                              // tile in slot b has reached the caller's array
+    std::thread copier[2];
+
+    // the copiers are joined on every return path: an early error return must not destroy a running thread
+    ~Streamed() { for (auto& t : copier) if (t.joinable()) t.join(); }
+    int64_t col(int64_t a) const { return pool_width > 0 ? a / pool_width : a; }
+    int64_t width(int64_t len) const { return pool_width > 0 ? (len + pool_width - 1) / pool_width : len; }
+
+    int prepare(const TileGeometry& geo, const int64_t* epochs, int n_epochs) {
+        alloc = geo.alloc;
+        pitch = pool_width > 0 ? (geo.tile + pool_width - 1) / pool_width : geo.alloc;
+        const size_t stage_bytes = (size_t)geo.g * R * pitch * el;
+        int rc = GCWT_OK;
+        for (int b = 0; b < 2 && rc == GCWT_OK; ++b) {
+            rc = grow_device(&h.d_red[b], &h.red_bytes[b], reduced ? stage_bytes : 0, "execute_host");
+            if (rc == GCWT_OK) rc = grow_pinned(&h.h_ring[b], &h.ring_bytes[b], pinned ? 0 : stage_bytes, "execute_host");
+        }
+        if (rc) return rc;
+        // copier threads of the pageable path (measured on a 16-core host, 6.9 GB per call: 8 threads 34 GB/s, see DESIGN.md)
+        n_threads = (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency() > 2 ? std::thread::hardware_concurrency() - 2 : 1u));
+        if (const char* e = getenv("GCWT_HOST_THREADS")) n_threads = std::max(1, atoi(e));
+        zero_gaps(out, epochs, n_epochs, n, n_channels, R, s_stride, c_stride, el);
+        return GCWT_OK;
+    }
+    int slot_free(int b) {                                         // tile in slot b has reached the caller's array
         if (!live[b]) return GCWT_OK;
         if (pinned) GCWT_CUDA_OK(cudaEventSynchronize(h.ev_out[b]));
         else if (copier[b].joinable()) copier[b].join();
         live[b] = false;
         return GCWT_OK;
-    };
-    // one tile: compute it into d_out[b], reduce it if this call asks for a reduction, and send its rows to `out`
-    auto run_tile = [&](int b, int64_t c0, int64_t gc, int64_t a, int64_t len, int64_t halo_l, int64_t halo_r) -> int {
-        int r = finish(b);                                         // the slot's previous tile has left its buffers
+    }
+    int group_begin(int64_t, int64_t) { return GCWT_OK; }
+    int group_end(int64_t, int64_t) { return GCWT_OK; }
+    // reduce the tile if this call asks for a reduction, and send its rows to `out`
+    int tile(int b, int64_t c0, int64_t gc, int64_t a, int64_t len) {
+        int r = GCWT_OK;
+        if (pool_width > 0)
+            r = pool_rows_launch(h.d_out[b], p->compute_type, gc * S, len, alloc, pool_width, pool_mode, 0,
+                                 (double*)h.d_red[b], pitch, h.st_copy);
+        else if (bands)
+            r = band_reduce_launch(h.d_out[b], p->compute_type, p->out_kind, gc, len, alloc, (int64_t)S * alloc, *bands,
+                                   h.d_red[b], pitch, (int64_t)R * pitch, h.st_copy);
         if (r) return r;
-        r = gcwt_execute(p, (const char*)h.d_in + (size_t)a * in_el, in_type, gc, len, n, halo_l, halo_r, h.d_means,
-                         h.d_out[b], tile_alloc, (int64_t)S * tile_alloc, h.st_compute);
-        if (r) return r;
-        // ev_done follows the whole of gcwt_execute in stream order, including the accuracy guard's fp64
-        // re-computation of the failing (channel, scale) pairs (guard_resolve), so the reductions read the
-        // corrected coefficients.  For the same reason band power is a pass of its own and not part of the
-        // fused kernels' epilogue: there it would sum values the guard then replaces.
-        GCWT_CUDA_OK(cudaEventRecord(h.ev_done[b], h.st_compute));
-        GCWT_CUDA_OK(cudaStreamWaitEvent(h.st_copy, h.ev_done[b], 0));
-        if (reduced) {
-            r = reduce(b, gc, len);
-            if (r) return r;
-        }
         const char* src = (const char*)(reduced ? h.d_red[b] : h.d_out[b]);
-        char* dst = (char*)out + ((size_t)c0 * c_stride + (size_t)col(a)) * el;
+        char* dst = out + ((size_t)c0 * c_stride + (size_t)col(a)) * el;
         const size_t row_bytes = (size_t)width(len) * el;
         if (pinned) {
             for (int64_t c = 0; c < gc; ++c)
@@ -278,52 +316,34 @@ int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, i
         } else {
             GCWT_CUDA_OK(cudaMemcpyAsync(h.h_ring[b], src, (size_t)gc * R * pitch * el, cudaMemcpyDeviceToHost, h.st_copy));
             GCWT_CUDA_OK(cudaEventRecord(h.ev_out[b], h.st_copy));
-            RowCopy rcp;
-            rcp.src = (const char*)h.h_ring[b]; rcp.src_pitch = (size_t)pitch * el;
-            rcp.dst = dst; rcp.s_stride_b = s_stride * (int64_t)el; rcp.c_stride_b = c_stride * (int64_t)el;
-            rcp.rows_per_channel = R; rcp.width = row_bytes; rcp.n_rows = gc * R;
+            const RowCopy rcp{(const char*)h.h_ring[b], (size_t)pitch * el, dst, s_stride * (int64_t)el,
+                              c_stride * (int64_t)el, R, row_bytes, gc * R};
             cudaEvent_t ev = h.ev_out[b];
-            const int dev = p->device;
-            copier[b] = std::thread([rcp, ev, dev, n_threads]() {
+            const int dev = p->device, nt = n_threads;
+            copier[b] = std::thread([rcp, ev, dev, nt]() {
                 cudaSetDevice(dev);
                 cudaEventSynchronize(ev);
-                copy_rows(rcp, n_threads);
+                copy_rows(rcp, nt);
             });
         }
         live[b] = true;
+        bytes_out += (double)gc * R * row_bytes;
         return GCWT_OK;
-    };
+    }
+};
 
-    int slot = 0;
-    int64_t n_tiles = 0;
-    double bytes_out = 0;
-    for (int64_t c0 = 0; c0 < n_channels && rc == GCWT_OK; c0 += geo.g) {
-        const int64_t gc = std::min<int64_t>(geo.g, n_channels - c0);
-        rc = load_group(p, x, in_type, n, x_stride, means_host, c0, gc);
-        for (int e = 0; e < n_epochs && rc == GCWT_OK; ++e) {
-            const int64_t e0 = epochs[2 * e], e1 = epochs[2 * e + 1];
-            for (int64_t a = e0; a < e1 && rc == GCWT_OK; a += geo.tile) {
-                const int64_t len = std::min(e1, a + geo.tile) - a;
-                rc = run_tile(slot, c0, gc, a, len, std::min(geo.halo, a - e0), std::min(geo.halo, e1 - a - len));
-                if (rc) break;
-                bytes_out += (double)gc * R * width(len) * el;
-                ++n_tiles;
-                slot ^= 1;
-            }
+int host_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n, int64_t x_stride,
+                 const int64_t* epochs, int n_epochs, const double* means_host, void* out, int64_t s_stride,
+                 int64_t c_stride, int64_t pool_width, int pool_mode, const BandTable* bands) {
+    if (pool_width > 0) {
+        if (p->out_kind == GCWT_OUT_COMPLEX) { set_error("execute_host: pooling needs amplitude or power output"); return GCWT_ERR_ARG; }
+        if (epochs && n_epochs > 0 && (n_epochs != 1 || epochs[0] != 0 || epochs[1] != n)) {
+            set_error("execute_host: pooling across epoch gaps is not supported (pool the full-rate result instead)");
+            return GCWT_ERR_UNSUPPORTED;
         }
     }
-    for (int b = 0; b < 2; ++b) {
-        const int r2 = finish(b);
-        if (rc == GCWT_OK) rc = r2;
-        if (copier[b].joinable()) copier[b].join();
-    }
-    cudaStreamSynchronize(h.st_copy);
-    cudaStreamSynchronize(h.st_compute);
-    h.last_ms[0] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
-    h.last_ms[1] = pinned ? 1.0 : 0.0;
-    h.last_ms[2] = (double)n_tiles;
-    h.last_ms[3] = bytes_out;
-    return rc;
+    Streamed s{p, n_channels, n, (char*)out, s_stride, c_stride, pool_width, pool_mode, bands};
+    return walk_tiles(p, x, in_type, n_channels, n, x_stride, epochs, n_epochs, means_host, pool_width, s);
 }
 
 int check_event_args(int64_t n, const int64_t* epochs, int n_epochs, const int64_t* events, int64_t n_events,
@@ -357,63 +377,59 @@ int check_event_args(int64_t n, const int64_t* epochs, int n_epochs, const int64
     return GCWT_OK;
 }
 
-int host_execute_events(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n, int64_t x_stride,
-                        const int64_t* epochs, int n_epochs, const double* means_host, const int64_t* events,
-                        int64_t n_events, int64_t lag_first, int64_t n_lags, double* power_out, double* phase_out,
-                        int64_t os_stride, int64_t oc_stride) {
-    // The tiles are those of gcwt_execute_host, but no tile travels.  After a tile's ev_done the copy stream adds
-    // the tile's part of every window that meets it into a per-group fp64 accumulator (event_reduce_kernel), and
-    // ev_out[b] keeps the next tile of slot b from overwriting d_out[b] before that reduction has read it.  After the
-    // group's last tile the accumulator travels once, through the pinned ring, and the host divides by n_events.
+// Event-locked sums: no tile travels.  After a tile's ev_done the copy stream adds the tile's part of every window that
+// meets it into a per-group fp64 accumulator (event_reduce_kernel), and ev_out[b] keeps the next tile of slot b from
+// overwriting d_out[b] before that reduction has read it.  After the group's last tile the accumulator travels once,
+// through the pinned ring, and the host divides by n_events.  The events have passed check_event_args.
+struct EventSums {
+    gcwt_plan* p; const int64_t* events; int64_t n_events, lag_first, n_lags; double* power_out; double* phase_out;
+    int64_t os_stride, oc_stride;
     gcwt_plan::HostStage& h = p->host;
-    const auto t_begin = std::chrono::steady_clock::now();
     const int S = p->n_scales;
-    const size_t in_el = in_type == GCWT_F32 ? 4 : 8;
-    const size_t real_el = p->compute_type == GCWT_F32 ? 4 : 8;
-    const size_t out_el = p->out_kind == GCWT_OUT_COMPLEX ? 2 * real_el : real_el;
-    int64_t one_epoch[2] = {0, n};
-    if (!epochs || n_epochs <= 0) { epochs = one_epoch; n_epochs = 1; }
-    int rc = ensure_streams(h);
-    if (rc) return rc;
-    const TileGeometry geo = tile_geometry(p, n_channels, n, out_el, 0);
-    const int64_t tile_alloc = (geo.tile + 3) & ~int64_t(3);      // rows of a tile stay 16-byte aligned
+    static constexpr bool pinned = false;                          // the means reach the caller from the pinned ring
+    double bytes_out = 0;
+    int64_t alloc = 0;
 
     // a group's accumulator: gc x S x n_lags power sums, then as many double2 phase sums on a 16-byte boundary
-    const bool phase = phase_out != nullptr;
-    auto power_cells = [&](int64_t gc) { return (gc * S * n_lags + 1) & ~int64_t(1); };
-    auto acc_bytes = [&](int64_t gc) {
-        return sizeof(double) * (size_t)power_cells(gc) + (phase ? sizeof(double2) * (size_t)(gc * S * n_lags) : 0);
-    };
-    rc = grow_staging(h, (size_t)geo.g * n * in_el, (size_t)geo.g * S * tile_alloc * out_el, 0, 0, geo.g);
-    if (rc == GCWT_OK) rc = grow_device((void**)&h.d_acc, &h.acc_bytes, acc_bytes(geo.g), "execute_host_events");
-    if (rc == GCWT_OK) rc = grow_device((void**)&h.d_events, &h.events_bytes, sizeof(int64_t) * n_events, "execute_host_events");
-    if (rc == GCWT_OK) rc = grow_pinned(&h.h_ring[0], &h.ring_bytes[0], acc_bytes(geo.g), "execute_host_events");
-    if (rc) return rc;
-    GCWT_CUDA_OK(cudaMemcpyAsync(h.d_events, events, sizeof(int64_t) * n_events, cudaMemcpyHostToDevice, h.st_copy));
+    int64_t power_cells(int64_t gc) const { return (gc * S * n_lags + 1) & ~int64_t(1); }
+    size_t acc_bytes(int64_t gc) const {
+        return sizeof(double) * (size_t)power_cells(gc) + (phase_out ? sizeof(double2) * (size_t)(gc * S * n_lags) : 0);
+    }
 
-    // one tile: compute it into d_out[b] and add its part of every window that meets it
-    auto run_tile = [&](int b, int64_t gc, int64_t a, int64_t len, int64_t halo_l, int64_t halo_r) -> int {
+    int prepare(const TileGeometry& geo, const int64_t*, int) {
+        alloc = geo.alloc;
+        int rc = grow_device((void**)&h.d_acc, &h.acc_bytes, acc_bytes(geo.g), "execute_host_events");
+        if (rc == GCWT_OK) rc = grow_device((void**)&h.d_events, &h.events_bytes, sizeof(int64_t) * n_events, "execute_host_events");
+        if (rc == GCWT_OK) rc = grow_pinned(&h.h_ring[0], &h.ring_bytes[0], acc_bytes(geo.g), "execute_host_events");
+        if (rc) return rc;
+        GCWT_CUDA_OK(cudaMemcpyAsync(h.d_events, events, sizeof(int64_t) * n_events, cudaMemcpyHostToDevice, h.st_copy));
+        return GCWT_OK;
+    }
+    int slot_free(int b) {                                         // on the device: the host never waits per tile
         GCWT_CUDA_OK(cudaStreamWaitEvent(h.st_compute, h.ev_out[b], 0));
-        int r = gcwt_execute(p, (const char*)h.d_in + (size_t)a * in_el, in_type, gc, len, n, halo_l, halo_r, h.d_means,
-                             h.d_out[b], tile_alloc, (int64_t)S * tile_alloc, h.st_compute);
-        if (r) return r;
-        // ev_done follows the accuracy guard's re-computation, so the sums read the corrected coefficients
-        GCWT_CUDA_OK(cudaEventRecord(h.ev_done[b], h.st_compute));
-        GCWT_CUDA_OK(cudaStreamWaitEvent(h.st_copy, h.ev_done[b], 0));
+        return GCWT_OK;
+    }
+    int group_begin(int64_t, int64_t gc) {
+        const cudaError_t e = cudaMemsetAsync(h.d_acc, 0, acc_bytes(gc), h.st_copy);
+        if (e != cudaSuccess) { set_error(std::string("execute_host_events: ") + cudaGetErrorString(e)); return GCWT_ERR_CUDA; }
+        return GCWT_OK;
+    }
+    // add the tile's part of every window that meets it
+    int tile(int b, int64_t, int64_t gc, int64_t a, int64_t len) {
         // the events whose windows start in (a - n_lags, a + len): a host-side binary search over ascending events
         const int64_t* lo = std::partition_point(events, events + n_events,
                                                  [&](int64_t e) { return e + lag_first <= a - n_lags; });
         const int64_t* hi = std::partition_point(lo, events + n_events, [&](int64_t e) { return e + lag_first < a + len; });
-        double* acc = h.d_acc;
-        r = event_reduce_launch(h.d_out[b], p->compute_type, p->out_kind, gc, S, len, tile_alloc, (int64_t)S * tile_alloc,
-                                a, h.d_events + (lo - events), hi - lo, lag_first, n_lags, acc,
-                                phase ? (double2*)(acc + power_cells(gc)) : nullptr, n_lags, (int64_t)S * n_lags, h.st_copy);
+        const int r = event_reduce_launch(h.d_out[b], p->compute_type, p->out_kind, gc, S, len, alloc, (int64_t)S * alloc,
+                                          a, h.d_events + (lo - events), hi - lo, lag_first, n_lags, h.d_acc,
+                                          phase_out ? (double2*)(h.d_acc + power_cells(gc)) : nullptr, n_lags,
+                                          (int64_t)S * n_lags, h.st_copy);
         if (r) return r;
         GCWT_CUDA_OK(cudaEventRecord(h.ev_out[b], h.st_copy));
         return GCWT_OK;
-    };
+    }
     // the group's means: one D2H of its accumulator, then sum / n_events into the caller's arrays
-    auto drain_group = [&](int64_t c0, int64_t gc) -> int {
+    int group_end(int64_t c0, int64_t gc) {
         GCWT_CUDA_OK(cudaMemcpyAsync(h.h_ring[0], h.d_acc, acc_bytes(gc), cudaMemcpyDeviceToHost, h.st_copy));
         GCWT_CUDA_OK(cudaStreamSynchronize(h.st_copy));
         const double* sums = (const double*)h.h_ring[0];
@@ -423,41 +439,20 @@ int host_execute_events(gcwt_plan* p, const void* x, int in_type, int64_t n_chan
             for (int s = 0; s < S; ++s) {
                 const int64_t row = c * S + s, o = (c0 + c) * oc_stride + (int64_t)s * os_stride;
                 for (int64_t l = 0; l < n_lags; ++l) power_out[o + l] = sums[row * n_lags + l] / cnt;
-                if (phase)
+                if (phase_out)
                     for (int64_t l = 0; l < 2 * n_lags; ++l) phase_out[2 * o + l] = phase_sums[2 * row * n_lags + l] / cnt;
             }
+        bytes_out += (double)gc * S * n_lags * (sizeof(double) + (phase_out ? sizeof(double2) : 0));
         return GCWT_OK;
-    };
-
-    int slot = 0;
-    int64_t n_tiles = 0;
-    double bytes_out = 0;
-    for (int64_t c0 = 0; c0 < n_channels && rc == GCWT_OK; c0 += geo.g) {
-        const int64_t gc = std::min<int64_t>(geo.g, n_channels - c0);
-        rc = load_group(p, x, in_type, n, x_stride, means_host, c0, gc);
-        if (rc == GCWT_OK) {
-            const cudaError_t e = cudaMemsetAsync(h.d_acc, 0, acc_bytes(gc), h.st_copy);
-            if (e != cudaSuccess) { set_error(std::string("execute_host_events: ") + cudaGetErrorString(e)); rc = GCWT_ERR_CUDA; }
-        }
-        for (int e = 0; e < n_epochs && rc == GCWT_OK; ++e) {
-            const int64_t e0 = epochs[2 * e], e1 = epochs[2 * e + 1];
-            for (int64_t a = e0; a < e1 && rc == GCWT_OK; a += geo.tile) {
-                const int64_t len = std::min(e1, a + geo.tile) - a;
-                rc = run_tile(slot, gc, a, len, std::min(geo.halo, a - e0), std::min(geo.halo, e1 - a - len));
-                ++n_tiles;
-                slot ^= 1;
-            }
-        }
-        if (rc == GCWT_OK) rc = drain_group(c0, gc);
-        if (rc == GCWT_OK) bytes_out += (double)gc * S * n_lags * (sizeof(double) + (phase ? sizeof(double2) : 0));
     }
-    cudaStreamSynchronize(h.st_copy);
-    cudaStreamSynchronize(h.st_compute);
-    h.last_ms[0] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
-    h.last_ms[1] = 0.0;                                            // the means reach the caller from the pinned ring
-    h.last_ms[2] = (double)n_tiles;
-    h.last_ms[3] = bytes_out;
-    return rc;
+};
+
+int host_execute_events(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n, int64_t x_stride,
+                        const int64_t* epochs, int n_epochs, const double* means_host, const int64_t* events,
+                        int64_t n_events, int64_t lag_first, int64_t n_lags, double* power_out, double* phase_out,
+                        int64_t os_stride, int64_t oc_stride) {
+    EventSums s{p, events, n_events, lag_first, n_lags, power_out, phase_out, os_stride, oc_stride};
+    return walk_tiles(p, x, in_type, n_channels, n, x_stride, epochs, n_epochs, means_host, 0, s);
 }
 
 }  // namespace gcwt

@@ -373,6 +373,18 @@ class CwtPlan:
             n, n_b * n))
         return out
 
+    def _device_coef_args(self, res, who):
+        """Checks a device-resident (channels, scales, samples) result; returns its real dtype, type code, kind (a
+        real ``res`` holds this plan's ``output``) and the current stream of its device."""
+        torch = _torch()
+        if not res.is_cuda or res.dim() != 3 or res.stride(2) != 1 or \
+                res.dtype not in (torch.float32, torch.float64, torch.complex64, torch.complex128):
+            raise ValueError(who + " needs a (channels, scales, samples) float / complex CUDA tensor with unit "
+                             "sample stride")
+        rdt = {torch.complex64: torch.float32, torch.complex128: torch.float64}.get(res.dtype, res.dtype)
+        kind = _lib.OUT_COMPLEX if res.is_complex() else (_lib.OUT_POWER if self.output == "power" else _lib.OUT_AMPLITUDE)
+        return rdt, _lib.F32 if rdt == torch.float32 else _lib.F64, kind, torch.cuda.current_stream(res.device).cuda_stream
+
     def band_reduce(self, res, first, count, weights):
         """Scale-averaged band power of a device-resident (channels, scales, samples) result ``res`` (a CUDA
         tensor with unit sample stride; a window of a larger result is fine): a (channels, bands, samples) CUDA
@@ -381,22 +393,14 @@ class CwtPlan:
         plan's ``output`` says."""
         torch = _torch()
         first, count, weights = _band_args(first, count, weights)
-        if not res.is_cuda or res.dim() != 3 or res.stride(2) != 1 or \
-                res.dtype not in (torch.float32, torch.float64, torch.complex64, torch.complex128):
-            raise ValueError("band_reduce needs a (channels, scales, samples) float / complex CUDA tensor with unit "
-                             "sample stride")
+        rdt, code, kind, st = self._device_coef_args(res, "band_reduce")
         if int((first + count).max()) > res.shape[1]:
             raise ValueError("a band reaches past the {} scales of the result".format(res.shape[1]))
         n_ch, _, n = res.shape
-        cx = res.is_complex()
-        rdt = {torch.complex64: torch.float32, torch.complex128: torch.float64}.get(res.dtype, res.dtype)
-        kind = _lib.OUT_COMPLEX if cx else (_lib.OUT_POWER if self.output == "power" else _lib.OUT_AMPLITUDE)
         out = torch.empty((n_ch, first.size, n), dtype=rdt, device=res.device)
-        st = torch.cuda.current_stream(res.device).cuda_stream
         _lib.check(self.lib.gcwt_band_reduce(
-            res.data_ptr(), _lib.F32 if rdt == torch.float32 else _lib.F64, kind, n_ch, n, res.stride(1),
-            res.stride(0), int(first.size), first.ctypes.data, count.ctypes.data, weights.ctypes.data,
-            out.data_ptr(), n, first.size * n, res.device.index, st))
+            res.data_ptr(), code, kind, n_ch, n, res.stride(1), res.stride(0), int(first.size), first.ctypes.data,
+            count.ctypes.data, weights.ctypes.data, out.data_ptr(), n, first.size * n, res.device.index, st))
         return out
 
     def execute_host_events(self, x, events, lag_first, n_lags, epochs=None, means=None):
@@ -423,10 +427,7 @@ class CwtPlan:
         allocated as zeros when not given.  Only the event samples inside the tile contribute, so tiles can be added
         into the same accumulators one after another.  Returns ``(power, phase or None)``: sums, not means."""
         torch = _torch()
-        if not res.is_cuda or res.dim() != 3 or res.stride(2) != 1 or \
-                res.dtype not in (torch.float32, torch.float64, torch.complex64, torch.complex128):
-            raise ValueError("event_reduce needs a (channels, scales, samples) float / complex CUDA tensor with unit "
-                             "sample stride")
+        _, code, kind, st = self._device_coef_args(res, "event_reduce")
         n_ch, S, n = res.shape
         L = int(n_lags)
         cx = res.is_complex()
@@ -446,13 +447,10 @@ class CwtPlan:
             if phase.dtype != torch.complex128 or phase.shape != (n_ch, S, L) or phase.stride() != power.stride() \
                     or not phase.is_cuda:
                 raise ValueError("phase must be a complex128 CUDA tensor of power's shape and strides")
-        rdt = {torch.complex64: torch.float32, torch.complex128: torch.float64}.get(res.dtype, res.dtype)
-        kind = _lib.OUT_COMPLEX if cx else (_lib.OUT_POWER if self.output == "power" else _lib.OUT_AMPLITUDE)
-        st = torch.cuda.current_stream(res.device).cuda_stream
         _lib.check(self.lib.gcwt_event_reduce(
-            res.data_ptr(), _lib.F32 if rdt == torch.float32 else _lib.F64, kind, n_ch, S, n, res.stride(1),
-            res.stride(0), int(sample0), ev.data_ptr(), ev.numel(), int(lag_first), L, power.data_ptr(),
-            None if phase is None else phase.data_ptr(), power.stride(1), power.stride(0), res.device.index, st))
+            res.data_ptr(), code, kind, n_ch, S, n, res.stride(1), res.stride(0), int(sample0), ev.data_ptr(),
+            ev.numel(), int(lag_first), L, power.data_ptr(), None if phase is None else phase.data_ptr(),
+            power.stride(1), power.stride(0), res.device.index, st))
         return power, phase
 
     def host_stats(self):

@@ -352,6 +352,21 @@ class ContinuousWaveletTransform(WaveletTransform):
             raise ValueError("transform(events=...) kept only the event-locked averages; run transform without "
                              "'events' for the full-rate amplitude, power or coefficients")
 
+    def _check_full_rate_result(self, needs):
+        self._check_full_rate()
+        if self._frequencies is None or (self._result is None and self._host is None):
+            raise ValueError("no full-rate result: call transform() first")
+        if self._pooled:
+            raise ValueError("the result was pooled over time (pool_width): {} the full-rate result".format(needs))
+
+    def _host_power(self, block):
+        """|W|^2 in float64 of a block of the host-resident result by output kind, as mag2 in sigtools.cu reads it."""
+        if self._output == "complex":
+            block = block.astype(np.complex128)
+            return np.square(block.real) + np.square(block.imag)
+        block = block.astype(np.float64)
+        return block if self._output == "power" else np.square(block)
+
     def _materialise(self):
         self._check_full_rate()
         if self._host is None:
@@ -428,11 +443,7 @@ class ContinuousWaveletTransform(WaveletTransform):
         ``multichannel``.  A device-resident result (``keep_on_device=True``) is reduced on the GPU and only the
         bands are copied back (plan dtype); a host-resident one is reduced in numpy in float64."""
         from ..engine import band_tables
-        self._check_full_rate()
-        if self._frequencies is None or (self._result is None and self._host is None):
-            raise ValueError("no full-rate result: call transform() first")
-        if self._pooled:
-            raise ValueError("the result was pooled over time (pool_width): band power needs the full-rate result")
+        self._check_full_rate_result("band power needs")
         first, count, weights = band_tables(self._frequencies, bands, reduce)
         if self._result is not None and self._host is None:
             res = self.last_plan.band_reduce(self._result, first, count, weights).cpu().numpy()
@@ -441,12 +452,7 @@ class ContinuousWaveletTransform(WaveletTransform):
             res = np.empty((data.shape[0], first.size, data.shape[2]), dtype=np.float64)
             off = 0
             for b, (a, c) in enumerate(zip(first, count)):
-                rows = data[:, a:a + c].astype(np.complex128 if self._output == "complex" else np.float64)
-                if self._output == "complex":
-                    p = np.square(rows.real) + np.square(rows.imag)
-                else:
-                    p = rows if self._output == "power" else np.square(rows)
-                res[:, b] = np.tensordot(weights[off:off + c], p, axes=(0, 1))
+                res[:, b] = np.tensordot(weights[off:off + c], self._host_power(data[:, a:a + c]), axes=(0, 1))
                 off += c
         return res if self._multichannel else res[0]
 
@@ -484,11 +490,7 @@ class ContinuousWaveletTransform(WaveletTransform):
         (``keep_on_device=True``) is reduced on the GPU and only the means are copied back; a host-resident one is
         reduced in numpy in float64."""
         from ..engine import event_windows
-        self._check_full_rate()
-        if self._frequencies is None or (self._result is None and self._host is None):
-            raise ValueError("no full-rate result: call transform() first")
-        if self._pooled:
-            raise ValueError("the result was pooled over time (pool_width): event averages need the full-rate result")
+        self._check_full_rate_result("event averages need")
         samples, _, lag_first, n_lags = event_windows(self._time, events, event_window, self._epoch_bounds, self._fs)
         cx = self._output == "complex"
         if self._result is not None and self._host is None:
@@ -501,14 +503,11 @@ class ContinuousWaveletTransform(WaveletTransform):
             phase = np.zeros(power.shape, dtype=np.complex128) if cx else None
             for s in samples:
                 w = data[:, :, s + lag_first:s + lag_first + n_lags]
+                power += self._host_power(w)
                 if cx:
                     w = w.astype(np.complex128)
-                    power += np.square(w.real) + np.square(w.imag)
                     m = np.abs(w)
                     phase += np.where(m > 0, w / np.where(m > 0, m, 1.0), 0.0)
-                else:
-                    w = w.astype(np.float64)
-                    power += w if self._output == "power" else np.square(w)
             power /= samples.size
             if cx:
                 phase /= samples.size

@@ -1,7 +1,8 @@
-"""GPU box: randomized check of the streamed host path (gcwt_execute_host and its pooled and band-power
-variants): random channel counts, lengths, epochs, forced tile lengths, pinned / pageable / strided destinations
-and random bands, against the device path executed epoch by epoch (pooled in numpy, band-reduced with
-plan.band_reduce).       python tools/fuzz_host_path.py [n_cases] [seed]"""
+"""GPU box: randomized check of the streamed host path (gcwt_execute_host and its pooled, band-power and event-locked
+variants): random channel counts, lengths, epochs, forced tile lengths, pinned / pageable / strided destinations,
+random bands and random events, against the device path executed epoch by epoch (pooled in numpy, band-reduced with
+plan.band_reduce) and, for the events, plan.event_reduce of the full-rate host result (the same tiles).
+       python tools/fuzz_host_path.py [n_cases] [seed]"""
 import os
 import sys
 import numpy as np
@@ -98,9 +99,35 @@ for case in range(n_cases):
         pos = b
     gaps_ok = gaps_ok and bool(np.all(got_b[:, :, pos:] == 0))
     ok = ok and gaps_ok and berr <= (1.2e-5 if dtype == np.float32 else 1e-11)
-    print("case %2d %s %s %s ch=%d n=%d epochs=%d S=%d tile=%d tiles=%d dest=%s err=%.2e pooled=%.1e bands=%d %.1e" % (
-        case, "ok " if ok else "BAD", np.dtype(dtype).name, output, nch, n, n_ep, S, tile, tiles, dest, err, perr, n_b,
-        berr), flush=True)
+    # event-locked means: ascending events with duplicates, windows of n_lags lags from lag_first (often negative)
+    # inside every epoch, some across the forced tile boundaries.  The reference sums the same windows of `got`
+    # (the same tiles, so the same coefficients): only the grouping of the fp64 sums differs.
+    n_lags = int(rng.integers(1, min(400, n_min) + 1))
+    lag_first = int(rng.integers(-n_lags - 50, 50))
+    ev = []
+    for a, b in epochs:                                              # window starts w0 in [a, b - n_lags]
+        ev += (rng.integers(a, b - n_lags + 1, int(rng.integers(1, 6))) - lag_first).tolist()
+        bounds_t = np.arange(a + max(tile, 1024), b, max(tile, 1024)) if tile else []
+        for t in bounds_t[:3]:                                       # windows that straddle a tile boundary
+            lo, hi = max(a, t - n_lags + 1), min(b - n_lags, t - 1)
+            if n_lags > 1 and lo <= hi:
+                ev.append(int(rng.integers(lo, hi + 1)) - lag_first)
+    ev = np.sort(np.array(ev + list(rng.choice(ev, int(rng.integers(1, 4)))), dtype=np.int64))
+    Xin = X if dtype == np.float32 else X.astype(np.float64)
+    got_p, got_ph = plan.execute_host_events(Xin, ev, lag_first, n_lags, epochs=epochs)
+    ref_p, ref_ph = plan.event_reduce(torch.from_numpy(np.ascontiguousarray(got)).cuda(), ev, lag_first, n_lags)
+    ref_p = ref_p.cpu().numpy() / ev.size
+    eerr = float(np.max(np.abs(got_p - ref_p) / np.maximum(np.abs(ref_p), 1e-300)))
+    pherr = 0.0
+    if output == "complex":
+        pherr = float(np.max(np.abs(got_ph - ref_ph.cpu().numpy() / ev.size)))
+    else:
+        ok = ok and got_ph is None and ref_ph is None
+    ok = ok and eerr <= 1e-12 and pherr <= 1e-12
+    print("case %2d %s %s %s ch=%d n=%d epochs=%d S=%d tile=%d tiles=%d dest=%s err=%.2e pooled=%.1e bands=%d %.1e "
+          "events=%d lags=%d%+d %.1e %.1e" % (
+              case, "ok " if ok else "BAD", np.dtype(dtype).name, output, nch, n, n_ep, S, tile, tiles, dest, err, perr,
+              n_b, berr, ev.size, n_lags, lag_first, eerr, pherr), flush=True)
     if not ok:
         fails.append(case)
     plan.close()
