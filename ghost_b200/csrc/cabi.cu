@@ -159,6 +159,8 @@ int gcwt_plan_create(gcwt_plan** out, const gcwt_plan_desc* d) {
     }
     if (d->device < 0 || d->device >= ndev) { set_error("plan_create: bad device ordinal"); return GCWT_ERR_ARG; }
     DeviceScope dev_scope(d->device);
+    int rc = prepare_device(d->device);
+    if (rc) return rc;
 
     gcwt_plan* p = new (std::nothrow) gcwt_plan();
     if (!p) { set_error("out of host memory"); return GCWT_ERR_NOMEM; }
@@ -188,7 +190,6 @@ int gcwt_plan_create(gcwt_plan** out, const gcwt_plan_desc* d) {
     }
     p->terms.assign(d->terms, d->terms + off);
 
-    int rc = GCWT_OK;
     {
         cudaError_t e = cudaMalloc((void**)&p->d_scales, sizeof(ScaleInfo) * p->n_scales);
         if (e == cudaSuccess) e = cudaMalloc((void**)&p->d_terms, sizeof(double) * p->terms.size());

@@ -4,6 +4,7 @@
 #include <stdint.h>
 #include <math.h>
 #include <string>
+#include <type_traits>
 #include "../../include/ghost_cwt.h"
 
 namespace gcwt {
@@ -146,5 +147,18 @@ template <int SIGN, typename C> struct small_dft<8, SIGN, C>  { static __device_
 template <int SIGN, typename C> struct small_dft<16, SIGN, C> { static __device__ __forceinline__ void run(C* a) { dft16<SIGN>(a); } };
 
 static inline int ilog2_ceil(int64_t v) { int l = 0; while ((int64_t(1) << l) < v) ++l; return l; }
+
+// ---------------------------------------------------------------- output kind
+template <int V> using IntC = std::integral_constant<int, V>;
+
+// The run-time output kind as a template argument: calls f(IntC<KIND>()), where any kind other than complex and
+// amplitude is power.  COMPLEX = false for kernels that have no complex-output instance.
+template <bool COMPLEX = true, typename F>
+static void with_kind(int kind, const F& f) {
+    if constexpr (COMPLEX)
+        if (kind == GCWT_OUT_COMPLEX) return f(IntC<GCWT_OUT_COMPLEX>());
+    if (kind == GCWT_OUT_AMPLITUDE) f(IntC<GCWT_OUT_AMPLITUDE>());
+    else f(IntC<GCWT_OUT_POWER>());
+}
 
 }  // namespace gcwt

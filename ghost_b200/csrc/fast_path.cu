@@ -1668,21 +1668,15 @@ fused_full_kernel(const FusedParams prm) {
 }
 
 // ============================================================================ driver
-template <int V> using IntC = std::integral_constant<int, V>;
-
 // The one place where a run-time output kind and guard flag become template arguments of the fused kernels:
 // calls f(IntC<KIND>(), std::integral_constant<bool, GUARD>()).  COMPLEX = false for the interpolating
 // kernels, which have no complex-output instance.
 template <bool COMPLEX, typename F>
 static void with_kind_guard(int kind, bool guard, const F& f) {
-    const auto with_guard = [&](auto k) {
+    with_kind<COMPLEX>(kind, [&](auto k) {
         if (guard) f(k, std::true_type());
         else f(k, std::false_type());
-    };
-    if constexpr (COMPLEX)
-        if (kind == GCWT_OUT_COMPLEX) return with_guard(IntC<GCWT_OUT_COMPLEX>());
-    if (kind == GCWT_OUT_AMPLITUDE) with_guard(IntC<GCWT_OUT_AMPLITUDE>());
-    else with_guard(IntC<GCWT_OUT_POWER>());
+    });
 }
 
 struct LevelGeom { int64_t lo, hi, len, stride; float* ptr; };
@@ -2024,7 +2018,7 @@ int guard_resolve(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, 
             const int sp = prof_begin(p, 3, st);
             int rc = generic_execute(p, run_ids, (const char*)x + in_el * run_start * x_stride, in_type, c - run_start, n_samples,
                                      x_stride, halo_l, halo_r, d_means + run_start, (char*)out + out_el * run_start * c_stride,
-                                     s_stride, c_stride, st, true);
+                                     s_stride, c_stride, st);
             prof_end(p, sp, st);
             if (rc) return rc;
         }
@@ -2035,29 +2029,27 @@ int guard_resolve(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, 
     return GCWT_OK;
 }
 
-// Once per device: the dynamic shared-memory limit of every fused-kernel instance fast_run can launch, and the
-// filter taps in constant memory (which is per device; the taps do not depend on the plan).
 static std::atomic<bool> g_device_ready[64];
 
-static int prepare_device(int device) {
+int prepare_device(int device) {
     if (g_device_ready[device & 63]) return GCWT_OK;
-    cudaError_t e = cudaSuccess;
-    const auto smem = [&](auto kernel, size_t bytes) {
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    };
+    std::vector<SmemKernel> big = fourstep_kernels();
     for (int kind = GCWT_OUT_COMPLEX; kind <= GCWT_OUT_POWER; ++kind)
         for (bool guard : {false, true})
             with_kind_guard<true>(kind, guard, [&](auto K, auto G) {
-                smem(fused_banded_kernel<K, 0, G>, kBandedSmem);
-                smem(fused_banded_kernel<K, 4, G>, kBandedSmem);
-                smem(fused_full_kernel<float, K, G>, kFullSmem);
-                smem(fused_full_kernel<double, K, G>, kFullSmem);
+                big.push_back({(const void*)fused_banded_kernel<K, 0, G>, kBandedSmem});
+                big.push_back({(const void*)fused_banded_kernel<K, 4, G>, kBandedSmem});
+                big.push_back({(const void*)fused_full_kernel<float, K, G>, kFullSmem});
+                big.push_back({(const void*)fused_full_kernel<double, K, G>, kFullSmem});
                 if constexpr (K != GCWT_OUT_COMPLEX) {
-                    smem(fused_interp_kernel<K, G>, kInterpSmem);
-                    smem(fused_wide2_kernel<K, G>, kWide2Smem);
+                    big.push_back({(const void*)fused_interp_kernel<K, G>, kInterpSmem});
+                    big.push_back({(const void*)fused_wide2_kernel<K, G>, kWide2Smem});
                 }
             });
-    if (e != cudaSuccess) { set_error(std::string("fused kernels: shared-memory limit: ") + cudaGetErrorString(e)); return GCWT_ERR_CUDA; }
+    for (const SmemKernel& k : big) {
+        const cudaError_t e = cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.bytes);
+        if (e != cudaSuccess) { set_error(std::string("shared-memory limit of a kernel: ") + cudaGetErrorString(e)); return GCWT_ERR_CUDA; }
+    }
     int rc = upload_constants();
     if (rc) return rc;
     g_device_ready[device & 63] = true;
@@ -2067,8 +2059,6 @@ static int prepare_device(int device) {
 int fast_execute(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n_samples,
                  int64_t x_stride, int64_t halo_l, int64_t halo_r, const double* d_means, void* out,
                  int64_t s_stride, int64_t c_stride, cudaStream_t st) {
-    int rc = prepare_device(p->device);
-    if (rc) return rc;
     if (in_type == GCWT_F32)
         return fast_run<float>(p, (const float*)x, in_type, n_channels, n_samples, x_stride, halo_l, halo_r,
                                d_means, out, s_stride, c_stride, st);

@@ -1,4 +1,4 @@
-// Batched power-of-two FFT through global memory (radix-16/8/4/2 Stockham autosort passes).
+// Batched power-of-two complex128 FFT through global memory (radix-16/8/4/2 Stockham autosort passes).
 // Shared by the generic CWT path and the sigtools helpers.
 #pragma once
 #include "plan.h"
@@ -9,16 +9,14 @@ namespace gcwt {
 
 // ----------------------------------------------------------------------------- FFT pass
 // One radix-R Stockham autosort pass over `batch` transforms of length n.
-template <typename T, int R, int SIGN>
-__global__ void stockham_pass_kernel(const typename cplx_of<T>::type* __restrict__ in,
-                                     typename cplx_of<T>::type* __restrict__ out, int n, int ns) {
-    typedef typename cplx_of<T>::type C;
+template <int R, int SIGN>
+__global__ void stockham_pass_kernel(const double2* __restrict__ in, double2* __restrict__ out, int n, int ns) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     const int m = n / R;
     if (j >= m) return;
     const int64_t base = (int64_t)blockIdx.y * n;
     const int k = j % ns;
-    C v[R];
+    double2 v[R];
 #pragma unroll
     for (int r = 0; r < R; ++r) v[r] = in[base + j + (int64_t)r * m];
     if (ns > 1) {
@@ -26,20 +24,17 @@ __global__ void stockham_pass_kernel(const typename cplx_of<T>::type* __restrict
 #pragma unroll
         for (int r = 1; r < R; ++r) {
             const int e = (int)(((int64_t)r * k) % span);
-            // the ratio is formed in fp64: e and span are not exact in fp32 once n exceeds 2^24
-            C w = expipi((T)((double)(SIGN * 2) * (double)e / (double)span));
-            v[r] = cmul(v[r], w);
+            v[r] = cmul(v[r], expipi((double)(SIGN * 2) * (double)e / (double)span));
         }
     }
-    small_dft<R, SIGN, C>::run(v);
+    small_dft<R, SIGN, double2>::run(v);
     const int64_t j0 = (int64_t)(j - k) * R + k;
 #pragma unroll
     for (int r = 0; r < R; ++r) out[base + j0 + (int64_t)r * ns] = v[r];
 }
 
-template <typename T, int SIGN>
-static void fft_batched(typename cplx_of<T>::type*& a, typename cplx_of<T>::type*& b, int n, int batch,
-                        cudaStream_t st) {
+template <int SIGN>
+static void fft_batched(double2*& a, double2*& b, int n, int batch, cudaStream_t st) {
     // result ends up in `a` (pointers are swapped as passes go)
     int lg = ilog2_ceil(n);
     int ns = 1;
@@ -48,10 +43,10 @@ static void fft_batched(typename cplx_of<T>::type*& a, typename cplx_of<T>::type
         const int m = n / r;
         dim3 grid((m + 127) / 128, batch);
         switch (r) {
-            case 16: stockham_pass_kernel<T, 16, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
-            case 8:  stockham_pass_kernel<T, 8, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
-            case 4:  stockham_pass_kernel<T, 4, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
-            default: stockham_pass_kernel<T, 2, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
+            case 16: stockham_pass_kernel<16, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
+            case 8:  stockham_pass_kernel<8, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
+            case 4:  stockham_pass_kernel<4, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
+            default: stockham_pass_kernel<2, SIGN><<<grid, 128, 0, st>>>(a, b, n, ns); break;
         }
         count_launch();
         std::swap(a, b);

@@ -11,8 +11,6 @@
 #include "fft_global.cuh"
 #include "fft_fourstep.cuh"
 #include <algorithm>
-#include <cstdlib>
-#include <type_traits>
 
 namespace gcwt {
 
@@ -103,10 +101,10 @@ int means_launch(const void* x, int in_type, int64_t n_channels, int64_t n_sampl
 }
 
 // ----------------------------------------------------------------------------- load
-template <typename TIn, typename T>
+template <typename TIn>
 __global__ void generic_load_kernel(const TIn* __restrict__ x, int64_t x_stride, int64_t n,
                                     int64_t halo_l, int64_t halo_r, const double* __restrict__ means,
-                                    typename cplx_of<T>::type* __restrict__ dst, int nfft,
+                                    double2* __restrict__ dst, int nfft,
                                     int64_t hop, int64_t offset, int64_t item0, int64_t n_chunks) {
     const int64_t item = item0 + blockIdx.y;
     const int64_t c = item / n_chunks, q = item % n_chunks;
@@ -117,38 +115,27 @@ __global__ void generic_load_kernel(const TIn* __restrict__ x, int64_t x_stride,
         const int64_t t = t0 + i;
         double v = 0.0;
         if (t >= -halo_l && t < n + halo_r) v = (double)xc[t] - mu;
-        dst[(int64_t)blockIdx.y * nfft + i] = mk<T>((T)v, (T)0);
+        dst[(int64_t)blockIdx.y * nfft + i] = make_double2(v, 0.0);
     }
 }
 
 // ----------------------------------------------------------------------------- response
 // H_s on the n-point grid, scaled by 1/n.  Kernel (2)'s multiplier, evaluated in registers.
 // p2 >= 0: position j holds bin k1 + 2^p1 * k2 with k1 = j >> p2, k2 = j & (2^p2 - 1) (four-step order)
-template <typename T>
 __global__ void generic_response_kernel(const ScaleInfo* __restrict__ scales,
                                         const double* __restrict__ terms,
                                         const int* __restrict__ ids, int nfft,
-                                        typename cplx_of<T>::type* __restrict__ H, int p1 = -1, int p2 = -1) {
+                                        double2* __restrict__ H, int p1 = -1, int p2 = -1) {
     const int pos = blockIdx.x * blockDim.x + threadIdx.x;
     if (pos >= nfft) return;
     const int j = p2 < 0 ? pos : (pos >> p2) + ((pos & ((1 << p2) - 1)) << p1);
     const ScaleInfo sc = scales[ids ? ids[blockIdx.y] : (int)blockIdx.y];
-    double g = morse_response(j, nfft, sc.L, sc.k_first, sc.n_terms, terms + sc.term_off);
-    g /= (double)nfft;
-    double re = g, im = 0.0;
-    if ((sc.L & 1) == 0) {                       // half-sample delay of the even-L kernel
-        double s, c;
-        sincospi(-(double)j / (double)nfft, &s, &c);
-        re = g * c;
-        im = g * s;
-    }
-    H[(int64_t)blockIdx.y * nfft + pos] = mk<T>((T)re, (T)im);
+    H[(int64_t)blockIdx.y * nfft + pos] = morse_transfer(j, nfft, sc.L, sc.k_first, sc.n_terms, terms + sc.term_off,
+                                                         (double)nfft);
 }
 
-template <typename T>
-__global__ void generic_multiply_kernel(const typename cplx_of<T>::type* __restrict__ Y,
-                                        const typename cplx_of<T>::type* __restrict__ H,
-                                        typename cplx_of<T>::type* __restrict__ Z, int nfft, int sb) {
+__global__ void generic_multiply_kernel(const double2* __restrict__ Y, const double2* __restrict__ H,
+                                        double2* __restrict__ Z, int nfft, int sb) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= nfft) return;
     const int s = blockIdx.y, ib = blockIdx.z;
@@ -156,12 +143,11 @@ __global__ void generic_multiply_kernel(const typename cplx_of<T>::type* __restr
 }
 
 // ----------------------------------------------------------------------------- epilogue
-template <typename T, typename TOut, int KIND>
-__global__ void generic_epilogue_kernel(const typename cplx_of<T>::type* __restrict__ Z, int nfft,
+template <typename TOut, int KIND>
+__global__ void generic_epilogue_kernel(const double2* __restrict__ Z, int nfft,
                                         int64_t item0, int64_t n_chunks, int64_t hop, int64_t offset,
                                         int64_t n, const int* __restrict__ ids, int sb, void* out,
                                         int64_t s_stride, int64_t c_stride) {
-    typedef typename cplx_of<T>::type C;
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= hop) return;
     const int s = blockIdx.y, ib = blockIdx.z;
@@ -169,7 +155,7 @@ __global__ void generic_epilogue_kernel(const typename cplx_of<T>::type* __restr
     const int64_t c = item / n_chunks, q = item % n_chunks;
     const int64_t t = q * hop + i;
     if (t >= n) return;
-    const C v = Z[((int64_t)ib * sb + s) * nfft + offset + i];
+    const double2 v = Z[((int64_t)ib * sb + s) * nfft + offset + i];
     const int64_t o = c * c_stride + (int64_t)ids[s] * s_stride + t;
     typedef typename cplx_of<TOut>::type CO;
     if (KIND == GCWT_OUT_COMPLEX) ((CO*)out)[o] = mk<TOut>((TOut)v.x, (TOut)v.y);
@@ -177,41 +163,43 @@ __global__ void generic_epilogue_kernel(const typename cplx_of<T>::type* __restr
     else ((TOut*)out)[o] = (TOut)(v.x * v.x + v.y * v.y);
 }
 
-// ----------------------------------------------------------------------------- four-step driver (fp64)
-template <typename TOut>
-static void launch_fs_cols(int kind, dim3 grid, cudaStream_t st, const FourStepParams& fp, const double2* T, int sb,
-                           const int* ids, void* out, int64_t s_stride, int64_t c_stride) {
-    static bool attr[3] = {false, false, false};
-    auto set = [&](auto kern, int k) {
-        if (!attr[k]) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFourStepSmem); attr[k] = true; }
-    };
-    if (kind == GCWT_OUT_COMPLEX) {
-        set(fs_inverse_cols_kernel<TOut, GCWT_OUT_COMPLEX>, 0);
-        fs_inverse_cols_kernel<TOut, GCWT_OUT_COMPLEX><<<grid, 256, kFourStepSmem, st>>>(fp, T, sb, ids, out, s_stride, c_stride);
-    } else if (kind == GCWT_OUT_AMPLITUDE) {
-        set(fs_inverse_cols_kernel<TOut, GCWT_OUT_AMPLITUDE>, 1);
-        fs_inverse_cols_kernel<TOut, GCWT_OUT_AMPLITUDE><<<grid, 256, kFourStepSmem, st>>>(fp, T, sb, ids, out, s_stride, c_stride);
-    } else {
-        set(fs_inverse_cols_kernel<TOut, GCWT_OUT_POWER>, 2);
-        fs_inverse_cols_kernel<TOut, GCWT_OUT_POWER><<<grid, 256, kFourStepSmem, st>>>(fp, T, sb, ids, out, s_stride, c_stride);
-    }
+// ----------------------------------------------------------------------------- drivers
+// One generic call: the scales `ids` of every channel, chunked for overlap-save.  Input samples are TIn, the
+// arithmetic is fp64 and the coefficients are stored as TOut (fp32 plans: fp64 arithmetic with an fp32 store).
+struct GenericCall {
+    gcwt_plan* p;
+    const std::vector<int>& ids;
+    const void* x;
+    int64_t n_channels, n, x_stride, halo_l, halo_r;
+    const double* d_means;
+    void* out;
+    int64_t s_stride, c_stride;
+    cudaStream_t st;
+    int64_t nfft, offset, hop, n_chunks, n_items;   // chunk geometry
+};
+
+std::vector<SmemKernel> fourstep_kernels() {
+    std::vector<SmemKernel> k = {{(const void*)fs_forward_cols_kernel<float>, kFourStepSmem},
+                                 {(const void*)fs_forward_cols_kernel<double>, kFourStepSmem},
+                                 {(const void*)fs_forward_rows_kernel, kFourStepSmem},
+                                 {(const void*)fs_inverse_rows_kernel, kFourStepSmem}};
+    for (int kind = GCWT_OUT_COMPLEX; kind <= GCWT_OUT_POWER; ++kind)
+        with_kind(kind, [&](auto K) {
+            k.push_back({(const void*)fs_inverse_cols_kernel<float, K>, kFourStepSmem});
+            k.push_back({(const void*)fs_inverse_cols_kernel<double, K>, kFourStepSmem});
+        });
+    return k;
 }
 
+// 2^11 <= nfft <= 2^20: the four-step FFT with shared-memory sub-transforms (fft_fourstep.cuh)
 template <typename TIn, typename TOut>
-static int generic_run_fourstep(gcwt_plan* p, const std::vector<int>& ids, const TIn* x, int64_t n_channels, int64_t n,
-                                int64_t x_stride, int64_t halo_l, int64_t halo_r, const double* d_means, void* out,
-                                int64_t s_stride, int64_t c_stride, cudaStream_t st, int64_t nfft, int64_t lmax) {
+static int run_fourstep(const GenericCall& g) {
+    gcwt_plan* p = g.p;
+    const std::vector<int>& ids = g.ids;
     const int ns = (int)ids.size();
+    const int64_t nfft = g.nfft;
     const FourStep fs(nfft);
-    const int64_t offset = lmax / 2, hop = nfft - (lmax - 1);
-    const int64_t n_chunks = (n + hop - 1) / hop, n_items = n_channels * n_chunks;
-    static bool attr_done = false;
-    if (!attr_done) {
-        GCWT_CUDA_OK(cudaFuncSetAttribute(fs_forward_cols_kernel<TIn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFourStepSmem));
-        GCWT_CUDA_OK(cudaFuncSetAttribute(fs_forward_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFourStepSmem));
-        GCWT_CUDA_OK(cudaFuncSetAttribute(fs_inverse_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFourStepSmem));
-        attr_done = true;
-    }
+    cudaStream_t st = g.st;
     // ---- tables ------------------------------------------------------------------------------
     if (!p->d_tw1k) {
         std::vector<double2> tw(1024);
@@ -233,9 +221,8 @@ static int generic_run_fourstep(gcwt_plan* p, const std::vector<int>& ids, const
     const size_t row = (size_t)nfft * sizeof(double2);
     // intermediate of one launch pair.  Measured on config 5: 32 ... 96 MB (L2-sized) 21.3 ms, 192 MB 19.9, 512 MB 19.3 --
     // the kernels are bound by shared-memory wavefronts, not by HBM, so fewer and larger launches win
-    size_t t_budget = (size_t)512 << 20;
-    if (const char* e = getenv("GCWT_F64_TBATCH_MB")) t_budget = (size_t)std::max(1, atoi(e)) << 20;
-    const int ib = (int)std::max<int64_t>(1, std::min<int64_t>(n_items, (int64_t)(((size_t)256 << 20) / row)));
+    const size_t t_budget = (size_t)512 << 20;
+    const int ib = (int)std::max<int64_t>(1, std::min<int64_t>(g.n_items, (int64_t)(((size_t)256 << 20) / row)));
     const int sb = (int)std::max<int64_t>(1, std::min<int64_t>(ns, (int64_t)(t_budget / (row * ib))));
     // the responses of a whole plan are cached when they fit (they depend on the scale and nfft only)
     bool contiguous = true;
@@ -244,7 +231,7 @@ static int generic_run_fourstep(gcwt_plan* p, const std::vector<int>& ids, const
     if (cache && p->hcache_n != nfft) {
         if (p->d_hcache) { GCWT_CUDA_OK(cudaStreamSynchronize(st)); cudaFree(p->d_hcache); p->d_hcache = nullptr; p->hcache_n = 0; }
         if (cudaMalloc((void**)&p->d_hcache, (size_t)p->n_scales * row) == cudaSuccess) {
-            generic_response_kernel<double><<<dim3((unsigned)((nfft + 255) / 256), p->n_scales), 256, 0, st>>>(
+            generic_response_kernel<<<dim3((unsigned)((nfft + 255) / 256), p->n_scales), 256, 0, st>>>(
                 p->d_scales, p->d_terms, nullptr, (int)nfft, p->d_hcache, fs.p1, fs.p2);
             count_launch();
             p->hcache_n = nfft;
@@ -267,24 +254,27 @@ static int generic_run_fourstep(gcwt_plan* p, const std::vector<int>& ids, const
 
     FourStepParams fp;
     fp.p = fs.p; fp.p1 = fs.p1; fp.p2 = fs.p2; fp.tw = p->d_tw1k; fp.tw_fine = p->d_tw_fine;
-    fp.n_chunks = n_chunks; fp.hop = hop; fp.offset = offset; fp.n = n; fp.halo_l = halo_l; fp.halo_r = halo_r;
+    fp.n_chunks = g.n_chunks; fp.hop = g.hop; fp.offset = g.offset; fp.n = g.n; fp.halo_l = g.halo_l; fp.halo_r = g.halo_r;
     const unsigned col_blocks = (unsigned)(fs.n2 / fs.cols_per_block), row_blocks = (unsigned)(fs.n1 / fs.rows_per_block);
-    for (int64_t i0 = 0; i0 < n_items; i0 += ib) {
-        const int ibn = (int)std::min<int64_t>(ib, n_items - i0);
+    for (int64_t i0 = 0; i0 < g.n_items; i0 += ib) {
+        const int ibn = (int)std::min<int64_t>(ib, g.n_items - i0);
         fp.item0 = i0; fp.n_items = ibn;
-        fs_forward_cols_kernel<TIn><<<col_blocks * ibn, 256, kFourStepSmem, st>>>(fp, x, x_stride, d_means, U);
+        fs_forward_cols_kernel<TIn><<<col_blocks * ibn, 256, kFourStepSmem, st>>>(fp, (const TIn*)g.x, g.x_stride, g.d_means, U);
         fs_forward_rows_kernel<<<row_blocks * ibn, 256, kFourStepSmem, st>>>(fp, U, Y);
         count_launch(2);
         for (int s0 = 0; s0 < ns; s0 += sb) {
             const int sbn = std::min(sb, ns - s0);
             const double2* H = cached ? p->d_hcache + ((int64_t)ids[s0] << fs.p) : Hb;
             if (!cached) {
-                generic_response_kernel<double><<<dim3((unsigned)((nfft + 255) / 256), sbn), 256, 0, st>>>(
+                generic_response_kernel<<<dim3((unsigned)((nfft + 255) / 256), sbn), 256, 0, st>>>(
                     p->d_scales, p->d_terms, d_ids + s0, (int)nfft, Hb, fs.p1, fs.p2);
                 count_launch();
             }
             fs_inverse_rows_kernel<<<dim3(row_blocks * ibn, sbn), 256, kFourStepSmem, st>>>(fp, Y, H, T, sbn);
-            launch_fs_cols<TOut>(p->out_kind, dim3(col_blocks * ibn, sbn), st, fp, T, sbn, d_ids + s0, out, s_stride, c_stride);
+            with_kind(p->out_kind, [&](auto K) {
+                fs_inverse_cols_kernel<TOut, K><<<dim3(col_blocks * ibn, sbn), 256, kFourStepSmem, st>>>(
+                    fp, T, sbn, d_ids + s0, g.out, g.s_stride, g.c_stride);
+            });
             count_launch(2);
         }
     }
@@ -292,34 +282,17 @@ static int generic_run_fourstep(gcwt_plan* p, const std::vector<int>& ids, const
     return GCWT_OK;
 }
 
-// ----------------------------------------------------------------------------- driver
-template <typename TIn, typename T, typename TOut>
-static int generic_run(gcwt_plan* p, const std::vector<int>& ids, const TIn* x, int64_t n_channels,
-                       int64_t n, int64_t x_stride, int64_t halo_l, int64_t halo_r,
-                       const double* d_means, void* out, int64_t s_stride, int64_t c_stride,
-                       cudaStream_t st) {
-    typedef typename cplx_of<T>::type C;
-    const int ns = (int)ids.size();
-    int64_t lmax = 1;
-    for (int id : ids) lmax = std::max<int64_t>(lmax, p->scales[id].L);
-    // chunk geometry: one chunk when the whole segment fits a 2^20-point transform
-    int64_t nfft;
-    if (n + lmax - 1 <= (int64_t(1) << 20)) nfft = int64_t(1) << ilog2_ceil(n + lmax - 1);
-    else nfft = std::max<int64_t>(int64_t(1) << 17, int64_t(1) << ilog2_ceil(4 * lmax));
-    if (nfft > (int64_t(1) << 26)) { set_error("generic path: kernel too long"); return GCWT_ERR_UNSUPPORTED; }
-    if (nfft < 16) nfft = 16;
-    if (std::is_same<T, double>::value && FourStep::usable(nfft))
-        return generic_run_fourstep<TIn, TOut>(p, ids, x, n_channels, n, x_stride, halo_l, halo_r, d_means, out, s_stride,
-                                               c_stride, st, nfft, lmax);
-    const int64_t offset = lmax / 2;
-    const int64_t hop = nfft - (lmax - 1);
-    const int64_t n_chunks = (n + hop - 1) / hop;
-    const int64_t n_items = n_channels * n_chunks;
-
-    const size_t row = (size_t)nfft * sizeof(C);
+// every other nfft: radix-16/8/4/2 passes through global memory (fft_global.cuh)
+template <typename TIn, typename TOut>
+static int run_stockham(const GenericCall& g) {
+    gcwt_plan* p = g.p;
+    const int ns = (int)g.ids.size();
+    const int64_t nfft = g.nfft;
+    cudaStream_t st = g.st;
+    const size_t row = (size_t)nfft * sizeof(double2);
     const size_t budget = (size_t)1 << 30;
     // few scales (the accuracy guard re-computing a handful of pairs): batch more chunks per launch instead
-    int ib = (int)std::min<int64_t>(n_items, std::max<int64_t>(4, std::min<int64_t>(32, (int64_t)(budget / (6 * row * std::min(ns, 4))))));
+    int ib = (int)std::min<int64_t>(g.n_items, std::max<int64_t>(4, std::min<int64_t>(32, (int64_t)(budget / (6 * row * std::min(ns, 4))))));
     int sb = (int)std::min<int64_t>(ns, std::max<int64_t>(1, (int64_t)(budget / (2 * row * ib))));
     sb = std::min(sb, 1024);
     // layout: Y[ib] | H[sb] | Za[ib*sb] | Zb[ib*sb] | ids[ns] | Yscratch[ib]
@@ -327,47 +300,36 @@ static int generic_run(gcwt_plan* p, const std::vector<int>& ids, const TIn* x, 
     int rc = ensure_workspace(p, need);
     if (rc) return rc;
     char* w = (char*)p->ws.ptr;
-    C* Y = (C*)w;                 w += row * ib;
-    C* Y2 = (C*)w;                w += row * ib;
-    C* H = (C*)w;                 w += row * sb;
-    C* Za = (C*)w;                w += row * (size_t)ib * sb;
-    C* Zb = (C*)w;                w += row * (size_t)ib * sb;
+    double2* Y = (double2*)w;     w += row * ib;
+    double2* Y2 = (double2*)w;    w += row * ib;
+    double2* H = (double2*)w;     w += row * sb;
+    double2* Za = (double2*)w;    w += row * (size_t)ib * sb;
+    double2* Zb = (double2*)w;    w += row * (size_t)ib * sb;
     int* d_ids = (int*)w;
-    GCWT_CUDA_OK(cudaMemcpyAsync(d_ids, ids.data(), sizeof(int) * ns, cudaMemcpyHostToDevice, st));
+    GCWT_CUDA_OK(cudaMemcpyAsync(d_ids, g.ids.data(), sizeof(int) * ns, cudaMemcpyHostToDevice, st));
 
     const int tpb = 256;
     const unsigned gx = (unsigned)((nfft + tpb - 1) / tpb);
     for (int s0 = 0; s0 < ns; s0 += sb) {
         const int sbn = std::min(sb, ns - s0);
-        generic_response_kernel<T><<<dim3(gx, sbn), tpb, 0, st>>>(p->d_scales, p->d_terms, d_ids + s0,
-                                                                  (int)nfft, H);
+        generic_response_kernel<<<dim3(gx, sbn), tpb, 0, st>>>(p->d_scales, p->d_terms, d_ids + s0, (int)nfft, H);
         count_launch();
-        for (int64_t i0 = 0; i0 < n_items; i0 += ib) {
-            const int ibn = (int)std::min<int64_t>(ib, n_items - i0);
-            generic_load_kernel<TIn, T><<<dim3(std::min(gx, 1024u), ibn), tpb, 0, st>>>(
-                x, x_stride, n, halo_l, halo_r, d_means, Y, (int)nfft, hop, offset, i0, n_chunks);
+        for (int64_t i0 = 0; i0 < g.n_items; i0 += ib) {
+            const int ibn = (int)std::min<int64_t>(ib, g.n_items - i0);
+            generic_load_kernel<TIn><<<dim3(std::min(gx, 1024u), ibn), tpb, 0, st>>>(
+                (const TIn*)g.x, g.x_stride, g.n, g.halo_l, g.halo_r, g.d_means, Y, (int)nfft, g.hop, g.offset, i0, g.n_chunks);
             count_launch();
-            C* ya = Y; C* yb = Y2;
-            fft_batched<T, -1>(ya, yb, (int)nfft, ibn, st);
-            generic_multiply_kernel<T><<<dim3(gx, sbn, ibn), tpb, 0, st>>>(ya, H, Za, (int)nfft, sbn);
+            double2* ya = Y; double2* yb = Y2;
+            fft_batched<-1>(ya, yb, (int)nfft, ibn, st);
+            generic_multiply_kernel<<<dim3(gx, sbn, ibn), tpb, 0, st>>>(ya, H, Za, (int)nfft, sbn);
             count_launch();
-            C* za = Za; C* zb = Zb;
-            fft_batched<T, +1>(za, zb, (int)nfft, ibn * sbn, st);
-            dim3 ge((unsigned)((hop + tpb - 1) / tpb), sbn, ibn);
-            switch (p->out_kind) {
-                case GCWT_OUT_COMPLEX:
-                    generic_epilogue_kernel<T, TOut, GCWT_OUT_COMPLEX><<<ge, tpb, 0, st>>>(
-                        za, (int)nfft, i0, n_chunks, hop, offset, n, d_ids + s0, sbn, out, s_stride, c_stride);
-                    break;
-                case GCWT_OUT_AMPLITUDE:
-                    generic_epilogue_kernel<T, TOut, GCWT_OUT_AMPLITUDE><<<ge, tpb, 0, st>>>(
-                        za, (int)nfft, i0, n_chunks, hop, offset, n, d_ids + s0, sbn, out, s_stride, c_stride);
-                    break;
-                default:
-                    generic_epilogue_kernel<T, TOut, GCWT_OUT_POWER><<<ge, tpb, 0, st>>>(
-                        za, (int)nfft, i0, n_chunks, hop, offset, n, d_ids + s0, sbn, out, s_stride, c_stride);
-                    break;
-            }
+            double2* za = Za; double2* zb = Zb;
+            fft_batched<+1>(za, zb, (int)nfft, ibn * sbn, st);
+            const dim3 ge((unsigned)((g.hop + tpb - 1) / tpb), sbn, ibn);
+            with_kind(p->out_kind, [&](auto K) {
+                generic_epilogue_kernel<TOut, K><<<ge, tpb, 0, st>>>(
+                    za, (int)nfft, i0, g.n_chunks, g.hop, g.offset, g.n, d_ids + s0, sbn, g.out, g.s_stride, g.c_stride);
+            });
             count_launch();
         }
     }
@@ -375,29 +337,34 @@ static int generic_run(gcwt_plan* p, const std::vector<int>& ids, const TIn* x, 
     return GCWT_OK;
 }
 
+// fp64 plans, and in fp32 plans the scales the fused kernels cannot take (wavelets whose truncated kernels are
+// genuinely broadband, GCWT_FLAG_FORCE_GENERIC) and the pairs the accuracy guard re-computes.  Always fp64
+// arithmetic: a full-spectrum fp32 transform has no guard of its own against recordings whose energy sits far
+// from a scale's band (errors of 1e-4 ... 1e-3 there), and the fp64 four-step path is the faster one anyway.
 int generic_execute(gcwt_plan* p, const std::vector<int>& ids, const void* x, int in_type,
                     int64_t n_channels, int64_t n_samples, int64_t x_stride, int64_t halo_l,
                     int64_t halo_r, const double* d_means, void* out, int64_t s_stride,
-                    int64_t c_stride, cudaStream_t st, bool fp64_for_fp32_plan) {
+                    int64_t c_stride, cudaStream_t st) {
     if (ids.empty()) return GCWT_OK;
-    if (p->compute_type == GCWT_F64) {
-        if (in_type == GCWT_F32)
-            return generic_run<float, double, double>(p, ids, (const float*)x, n_channels, n_samples, x_stride, halo_l,
-                                                      halo_r, d_means, out, s_stride, c_stride, st);
-        return generic_run<double, double, double>(p, ids, (const double*)x, n_channels, n_samples, x_stride, halo_l,
-                                                   halo_r, d_means, out, s_stride, c_stride, st);
-    }
-    // fp32 plans: the scales the fused kernels cannot take (wavelets whose truncated kernels are genuinely
-    // broadband, GCWT_FLAG_FORCE_GENERIC) and the pairs the accuracy guard re-computes.  Always fp64 arithmetic
-    // with an fp32 store: a full-spectrum fp32 transform has no guard of its own against recordings whose
-    // energy sits far from a scale's band (errors of 1e-4 ... 1e-3 there), and since round 2 the fp64
-    // four-step path is the faster one anyway.
-    (void)fp64_for_fp32_plan;
-    if (in_type == GCWT_F32)
-        return generic_run<float, double, float>(p, ids, (const float*)x, n_channels, n_samples, x_stride, halo_l,
-                                                 halo_r, d_means, out, s_stride, c_stride, st);
-    return generic_run<double, double, float>(p, ids, (const double*)x, n_channels, n_samples, x_stride, halo_l,
-                                              halo_r, d_means, out, s_stride, c_stride, st);
+    int64_t lmax = 1;
+    for (int id : ids) lmax = std::max<int64_t>(lmax, p->scales[id].L);
+    // chunk geometry: one chunk when the whole segment fits a 2^20-point transform
+    int64_t nfft;
+    if (n_samples + lmax - 1 <= (int64_t(1) << 20)) nfft = int64_t(1) << ilog2_ceil(n_samples + lmax - 1);
+    else nfft = std::max<int64_t>(int64_t(1) << 17, int64_t(1) << ilog2_ceil(4 * lmax));
+    if (nfft > (int64_t(1) << 26)) { set_error("generic path: kernel too long"); return GCWT_ERR_UNSUPPORTED; }
+    if (nfft < 16) nfft = 16;
+    const int64_t hop = nfft - (lmax - 1), n_chunks = (n_samples + hop - 1) / hop;
+    const GenericCall g{p, ids, x, n_channels, n_samples, x_stride, halo_l, halo_r, d_means, out, s_stride, c_stride, st,
+                        nfft, lmax / 2, hop, n_chunks, n_channels * n_chunks};
+    const auto by_type = [](int type, auto f) { return type == GCWT_F32 ? f(float()) : f(double()); };
+    return by_type(in_type, [&](auto tin) {
+        return by_type(p->compute_type, [&](auto tout) {
+            using TIn = decltype(tin);
+            using TOut = decltype(tout);
+            return FourStep::usable(nfft) ? run_fourstep<TIn, TOut>(g) : run_stockham<TIn, TOut>(g);
+        });
+    });
 }
 
 // ----------------------------------------------------------------------------- probe
@@ -406,16 +373,7 @@ __global__ void filter_response_kernel(int64_t L, int k_first, int n_terms, cons
                                        double2* __restrict__ out) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_bins) return;
-    const int64_t j = first_bin + i;
-    const double g = morse_response(j, nfft, L, k_first, n_terms, terms);
-    double re = g, im = 0.0;
-    if ((L & 1) == 0) {
-        double s, c;
-        sincospi(-(double)(j % (2 * nfft)) / (double)nfft, &s, &c);
-        re = g * c;
-        im = g * s;
-    }
-    out[i] = make_double2(re, im);
+    out[i] = morse_transfer(first_bin + i, nfft, L, k_first, n_terms, terms, 1.0);
 }
 
 int filter_response_device(int64_t L, int k_first, int n_terms, const double* terms_host, int64_t nfft,

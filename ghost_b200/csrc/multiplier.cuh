@@ -51,4 +51,14 @@ __host__ __device__ inline double morse_response(int64_t j, int64_t n, int64_t L
     return acc;
 }
 
+// H at bin j of an n-point grid, divided by `div`: G with the half-sample delay of an even-L kernel.
+__device__ inline double2 morse_transfer(int64_t j, int64_t n, int64_t L, int k_first, int n_terms, const double* X,
+                                         double div) {
+    const double g = morse_response(j, n, L, k_first, n_terms, X) / div;
+    if (L & 1) return make_double2(g, 0.0);
+    double s, c;
+    sincospi(-(double)(j % (2 * n)) / (double)n, &s, &c);
+    return make_double2(g * c, g * s);
+}
+
 }  // namespace gcwt

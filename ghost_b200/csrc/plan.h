@@ -164,12 +164,18 @@ int64_t launches_so_far();
 int prof_begin(gcwt_plan* p, int kind, cudaStream_t st, int tag = 0);
 void prof_end(gcwt_plan* p, int idx, cudaStream_t st);
 
+// a kernel launched with more dynamic shared memory than the 48 KB default, and the bytes it is launched with
+struct SmemKernel { const void* fn; size_t bytes; };
+std::vector<SmemKernel> fourstep_kernels();   // the four-step FFT kernels of the generic path
+// Once per device, from gcwt_plan_create: the shared-memory limit of every such kernel of both paths, and the
+// fused kernels' filter taps in constant memory.  Both are per device and do not depend on the plan.
+int prepare_device(int device);
+
 // path drivers (each returns a GCWT_* code)
 int generic_execute(gcwt_plan* p, const std::vector<int>& ids, const void* x, int in_type,
                     int64_t n_channels, int64_t n_samples, int64_t x_stride,
                     int64_t halo_l, int64_t halo_r, const double* d_means,
-                    void* out, int64_t s_stride, int64_t c_stride, cudaStream_t st,
-                    bool fp64_for_fp32_plan = false);
+                    void* out, int64_t s_stride, int64_t c_stride, cudaStream_t st);
 int guard_resolve(gcwt_plan* p, const void* x, int in_type, int64_t n_channels, int64_t n_samples,
                   int64_t x_stride, int64_t halo_l, int64_t halo_r, const double* d_means,
                   void* out, int64_t s_stride, int64_t c_stride, cudaStream_t st);

@@ -88,12 +88,17 @@ __global__ void st_hilbert_weights(C* __restrict__ X, int64_t n) {
 
 static inline unsigned nblk(int64_t m) { return (unsigned)((m + 255) / 256); }
 
-// Power-of-two FFT of `m` points: result pointer returned in `res` (one of a / b).
-template <int SIGN>
-static void fft_pow2(C* a, C* b, int64_t m, C*& res) {
-    C* pa = a; C* pb = b;
-    if (m > 1) fft_batched<double, SIGN>(pa, pb, (int)m, 1, 0);
-    res = pa;
+// Cyclic convolution of two m-point buffers (m a power of two): forward transforms of a and b, their product
+// scaled by 1/m, inverse transform.  `t` is a third m-point buffer; all three are overwritten, and the one that
+// holds the result is returned.
+static C* cyclic_conv(C* a, C* b, C* t, int64_t m) {
+    C* spare = t;
+    fft_batched<-1>(a, spare, (int)m, 1, 0);
+    fft_batched<-1>(b, spare, (int)m, 1, 0);
+    st_mul<<<nblk(m), 256>>>(a, b, m, 1.0 / (double)m);
+    count_launch();
+    fft_batched<+1>(a, spare, (int)m, 1, 0);
+    return a;
 }
 
 // DFT of arbitrary length n (device in -> device out), sign = -1 forward / +1 backward (unscaled).
@@ -103,8 +108,9 @@ static int dft_any(const C* d_in, int64_t n, int sign, C* d_out) {
     if (pow2) {
         DevBuf t; int rc = t.alloc(sizeof(C) * n); if (rc) return rc;
         GCWT_CUDA_OK(cudaMemcpy(d_out, d_in, sizeof(C) * n, cudaMemcpyDeviceToDevice));
-        C* res;
-        if (sign < 0) fft_pow2<-1>(d_out, t.c(), n, res); else fft_pow2<+1>(d_out, t.c(), n, res);
+        C* res = d_out;
+        C* spare = t.c();
+        if (sign < 0) fft_batched<-1>(res, spare, (int)n, 1, 0); else fft_batched<+1>(res, spare, (int)n, 1, 0);
         if (res != d_out) GCWT_CUDA_OK(cudaMemcpy(d_out, res, sizeof(C) * n, cudaMemcpyDeviceToDevice));
         return GCWT_OK;
     }
@@ -116,15 +122,8 @@ static int dft_any(const C* d_in, int64_t n, int sign, C* d_out) {
     st_bluestein_pre<<<nblk(m), 256>>>(d_in, n, a.c(), m, sign);
     st_bluestein_kernel<<<nblk(m), 256>>>(b.c(), n, m, sign);
     count_launch(2);
-    C *fa, *fb, *fc;
-    fft_pow2<-1>(a.c(), t.c(), m, fa);
-    C* spare_a = (fa == a.c()) ? t.c() : a.c();
-    fft_pow2<-1>(b.c(), spare_a, m, fb);
-    C* spare_b = (fb == b.c()) ? spare_a : b.c();
-    st_mul<<<nblk(m), 256>>>(fa, fb, m, 1.0 / (double)m);
-    count_launch();
-    fft_pow2<+1>(fa, spare_b, m, fc);
-    st_bluestein_post<<<nblk(n), 256>>>(fc, n, d_out, sign, 1.0);
+    const C* conv = cyclic_conv(a.c(), b.c(), t.c(), m);
+    st_bluestein_post<<<nblk(n), 256>>>(conv, n, d_out, sign, 1.0);
     count_launch();
     GCWT_CUDA_OK(cudaGetLastError());
     GCWT_CUDA_OK(cudaDeviceSynchronize());
@@ -179,16 +178,9 @@ int sig_fastconv_host(const double* sig_host, int sig_complex, int64_t n, const 
     if (ker_complex) st_pad_complex<<<nblk(nfft), 256>>>((const C*)raw_k.p, m, b.c(), nfft);
     else st_pad_real<<<nblk(nfft), 256>>>((const double*)raw_k.p, m, b.c(), nfft);
     count_launch(2);
-    C *fa, *fb, *fc;
-    fft_pow2<-1>(a.c(), t.c(), nfft, fa);
-    C* spare_a = (fa == a.c()) ? t.c() : a.c();
-    fft_pow2<-1>(b.c(), spare_a, nfft, fb);
-    C* spare_b = (fb == b.c()) ? spare_a : b.c();
-    st_mul<<<nblk(nfft), 256>>>(fa, fb, nfft, 1.0 / (double)nfft);
-    count_launch();
-    fft_pow2<+1>(fa, spare_b, nfft, fc);
+    const C* res = cyclic_conv(a.c(), b.c(), t.c(), nfft);
     GCWT_CUDA_OK(cudaGetLastError());
-    GCWT_CUDA_OK(cudaMemcpy(out_host, fc, sizeof(C) * tot, cudaMemcpyDeviceToHost));
+    GCWT_CUDA_OK(cudaMemcpy(out_host, res, sizeof(C) * tot, cudaMemcpyDeviceToHost));
     return GCWT_OK;
 }
 

@@ -10,7 +10,9 @@ and constant-bank-3 operands are written as symbol + offset, so that a __constan
 changing what it holds does not count as a change.  A function that differs is listed with the instructions
 only one side has, counted as multisets with register, predicate and barrier names and operand-reuse flags blanked out: ptxas
 reallocates registers and reorders blocks throughout a function when one branch of it changes, which turns a
-line diff into noise.  A refactor that must leave the kernels alone should report every function `same`.
+line diff into noise.  A function only one tree has is reported as `renamed OLD -> NEW` when its instructions
+are identical to those of exactly one function only the other tree has, and their resource lines are compared
+under that pairing.  A refactor that must leave the kernels alone should report every function `same` or `renamed`.
 """
 import collections
 import concurrent.futures
@@ -99,8 +101,19 @@ def main():
             ptx = {s: j.result() for s, j in jobs.items()}
             fo, fn = sass(cub["old"]), sass(cub["new"])
             print("==", src, "(%d functions old, %d new)" % (len(fo), len(fn)))
+            # a function only one side has is a rename when exactly one function of the other side has its code
+            by_code = collections.defaultdict(lambda: ([], []))
+            for side, funcs, other in ((0, fo, fn), (1, fn, fo)):
+                for f in funcs:
+                    if f not in other:
+                        by_code[tuple(funcs[f])][side].append(f)
+            renamed = {a[0]: b[0] for a, b in by_code.values() if len(a) == 1 and len(b) == 1}
             for f in sorted(set(fo) | set(fn)):
-                if f not in fo or f not in fn:
+                if f in renamed:
+                    print("renamed   %s -> %s" % (f, renamed[f]))
+                elif f in renamed.values():
+                    continue
+                elif f not in fo or f not in fn:
                     print("%-9s %s" % ("new only" if f in fn else "old only", f))
                     changed += 1
                 elif fo[f] == fn[f]:
@@ -115,6 +128,7 @@ def main():
                         print("    " + l)
                     changed += 1
             ro, rn = resources(ptx["old"]), resources(ptx["new"])
+            rn.update({f: rn.pop(g) for f, g in renamed.items() if g in rn})       # compare renamed pairs
             diff = [f for f in sorted(set(ro) | set(rn)) if ro.get(f) != rn.get(f)]
             print("ptxas resources: %s" % ("identical for all %d functions" % len(rn) if not diff else "differ"))
             for f in diff:
