@@ -17,10 +17,11 @@ FLAG_FORCE_GENERIC = 1
 FLAG_NO_INTERP = 2
 FLAG_NO_GUARD = 4
 POOL_MEAN, POOL_MAX = 0, 1
+KERNEL_FULL, KERNEL_BANDED, KERNEL_INTERP, KERNEL_WIDE2 = 0, 1, 2, 3
 
 EXPORTS = (
     "gcwt_version", "gcwt_last_error", "gcwt_launch_count", "gcwt_plan_create",
-    "gcwt_plan_destroy", "gcwt_plan_levels", "gcwt_plan_workspace_bytes",
+    "gcwt_plan_destroy", "gcwt_plan_levels", "gcwt_plan_classes", "gcwt_plan_workspace_bytes",
     "gcwt_channel_means", "gcwt_execute", "gcwt_execute_host", "gcwt_filter_response",
     "gcwt_morse_kernel", "gcwt_profile_enable", "gcwt_profile_read",
     "gcwt_fastconv", "gcwt_dft", "gcwt_analytic_signal", "gcwt_moments", "gcwt_interp_taps",
@@ -49,6 +50,18 @@ class PlanDesc(C.Structure):
     ]
 
 
+class ClassInfo(C.Structure):
+    _fields_ = [
+        ("level", C.c_int32),
+        ("kernel", C.c_int32),
+        ("log2u", C.c_int32),
+        ("n_scales", C.c_int32),
+        ("chunk", C.c_int64),
+        ("offset", C.c_int64),
+        ("hop", C.c_int64),
+    ]
+
+
 _lib = None
 
 
@@ -70,6 +83,7 @@ def load():
     lib.gcwt_plan_create.argtypes = [C.POINTER(vp), C.POINTER(PlanDesc)]
     lib.gcwt_plan_destroy.argtypes = [vp]
     lib.gcwt_plan_levels.argtypes = [vp, C.POINTER(i32)]
+    lib.gcwt_plan_classes.argtypes = [vp, C.POINTER(i32), C.POINTER(ClassInfo), C.POINTER(i32)]
     lib.gcwt_plan_workspace_bytes.restype = C.c_size_t
     lib.gcwt_plan_workspace_bytes.argtypes = [vp]
     lib.gcwt_channel_means.argtypes = [vp, i32, i64, i64, i64, vp, i32, vp]

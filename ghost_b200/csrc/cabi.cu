@@ -263,6 +263,31 @@ int gcwt_plan_levels(const gcwt_plan* p, int32_t* levels_out) {
     return GCWT_OK;
 }
 
+int gcwt_plan_classes(const gcwt_plan* p, int32_t* n_classes, gcwt_class_info* info, int32_t* class_of_scale) {
+    if (!p || !n_classes) { set_error("plan_classes: NULL argument"); return GCWT_ERR_ARG; }
+    const int nc = (int)p->classes.size();
+    *n_classes = nc;
+    if (class_of_scale)
+        for (int s = 0; s < p->n_scales; ++s) class_of_scale[s] = -1;
+    for (int i = 0; i < nc; ++i) {
+        const gcwt::FastClass& fc = p->classes[i];
+        if (info) {
+            gcwt_class_info& ci = info[i];
+            ci.level = fc.level;
+            ci.kernel = fc.level < 0 ? GCWT_KERNEL_FULL
+                      : fc.wide ? GCWT_KERNEL_WIDE2 : (fc.interp ? GCWT_KERNEL_INTERP : GCWT_KERNEL_BANDED);
+            ci.log2u = fc.interp ? fc.log2u : 0;
+            ci.n_scales = (int32_t)fc.scale_ids.size();
+            ci.chunk = fc.wide ? 2 * fc.nc_full : fc.nc_full;
+            ci.offset = fc.wide ? fc.offset2 : fc.offset;
+            ci.hop = fc.wide ? fc.hop2 : fc.hop;
+        }
+        if (class_of_scale)
+            for (int id : fc.scale_ids) class_of_scale[id] = i;
+    }
+    return GCWT_OK;
+}
+
 size_t gcwt_plan_workspace_bytes(const gcwt_plan* p) { return p ? p->ws.bytes : 0; }
 
 int gcwt_guard_stats(const gcwt_plan* p, int64_t* last_pairs, int64_t* total_pairs, int64_t* checked_pairs,

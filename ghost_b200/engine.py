@@ -164,6 +164,21 @@ class CwtPlan:
         _lib.check(self.lib.gcwt_plan_levels(self._h, out.ctypes.data_as(C.POINTER(C.c_int32))))
         return out
 
+    def classes(self):
+        """Scale classes of the fp32 fused kernels (include/ghost_cwt.h, gcwt_plan_classes): a list of dicts
+        (level, kernel as planned: 'full' / 'banded' / 'interp' / 'wide2', log2u, n_scales, and the chunk,
+        offset and hop of the chunk that kernel transforms), and per scale its class index (-1: generic path)."""
+        n = C.c_int32()
+        _lib.check(self.lib.gcwt_plan_classes(self._h, C.byref(n), None, None))
+        info = (_lib.ClassInfo * max(1, n.value))()
+        of_scale = np.empty(self.n_scales, dtype=np.int32)
+        _lib.check(self.lib.gcwt_plan_classes(self._h, C.byref(n), info, of_scale.ctypes.data_as(C.POINTER(C.c_int32))))
+        names = {_lib.KERNEL_FULL: "full", _lib.KERNEL_BANDED: "banded", _lib.KERNEL_INTERP: "interp",
+                 _lib.KERNEL_WIDE2: "wide2"}
+        out = [{"level": c.level, "kernel": names[c.kernel], "log2u": c.log2u, "n_scales": c.n_scales,
+                "chunk": c.chunk, "offset": c.offset, "hop": c.hop} for c in info[:n.value]]
+        return out, of_scale
+
     def guard_stats(self):
         """Accuracy guard of the fp32 paths (include/ghost_cwt.h, gcwt_guard_stats): dict with the
         (channel, scale) pairs re-computed in fp64 by the last execute, in total, the pairs examined

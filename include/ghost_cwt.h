@@ -90,6 +90,31 @@ int gcwt_plan_destroy(gcwt_plan *plan);
  * fast path at 2**level; -1: full-spectrum fused kernel; -2: generic global-memory path). */
 int gcwt_plan_levels(const gcwt_plan *plan, int32_t *levels_out);
 
+/* Introspection: the scale classes of an fp32 plan's fused kernels (one fused launch each; the guard
+ * splits the full-spectrum launch in two on long segments).  The planner forms classes from band widths
+ * it measures on the device, so this is the only way to see them.  kernel is the kernel as planned: at
+ * execute time an interpolated class with log2u == 2 falls back to the banded kernel when the output rows
+ * are not 16-byte aligned.  chunk, offset and hop describe the chunk that kernel transforms (full-rate
+ * samples): a wide-interpolation class runs on chunks of twice its level's 1024 << level samples.
+ *   n_classes       number of classes (0 for fp64 plans and plans of generic scales only)
+ *   info            optional [*n_classes] records
+ *   class_of_scale  optional [n_scales]: index into info, -1 for a scale of the generic path */
+#define GCWT_KERNEL_FULL   0   /* fused_full_kernel: full spectrum at the full rate (level -1)      */
+#define GCWT_KERNEL_BANDED 1   /* fused_banded_kernel: pruned inverse FFT of every output sample   */
+#define GCWT_KERNEL_INTERP 2   /* fused_interp_kernel: |W|^2 on a grid of 2**log2u + interpolator  */
+#define GCWT_KERNEL_WIDE2  3   /* fused_wide2_kernel: levels 2-3, spacing U = 2**level, 2x chunks  */
+typedef struct gcwt_class_info {
+    int32_t level;      /* >= 2: band-limited at decimation 2**level; -1: full spectrum              */
+    int32_t kernel;     /* GCWT_KERNEL_*                                                             */
+    int32_t log2u;      /* coarse spacing of the interpolated kernels (0 for full and banded)         */
+    int32_t n_scales;   /* scales of the class (<= 16; <= 64 for the full-spectrum class)             */
+    int64_t chunk;      /* chunk length in full-rate samples                                          */
+    int64_t offset;     /* first chunk-local sample a chunk owns                                      */
+    int64_t hop;        /* samples owned per chunk: chunk q owns [q hop, (q + 1) hop) of the segment  */
+} gcwt_class_info;
+int gcwt_plan_classes(const gcwt_plan *plan, int32_t *n_classes, gcwt_class_info *info,
+                      int32_t *class_of_scale);
+
 /* Transform one contiguous segment (an epoch, or one rank's time shard) of n_channels
  * channels.  Replaces, for every scale, convfun(x[start:stop], kernel) followed by
  * np.abs (transforms.py:202-204), i.e. a zero-padded 'same' linear convolution.

@@ -37,6 +37,28 @@ def test_constants_match_header():
     assert int(defs["GCWT_OUT_POWER"]) == _lib.OUT_POWER
     assert int(defs["GCWT_FLAG_FORCE_GENERIC"]) == _lib.FLAG_FORCE_GENERIC
     assert int(defs["GCWT_FLAG_NO_INTERP"]) == _lib.FLAG_NO_INTERP
+    assert int(defs["GCWT_FLAG_NO_GUARD"]) == _lib.FLAG_NO_GUARD
+    for name in ("FULL", "BANDED", "INTERP", "WIDE2"):
+        assert int(defs["GCWT_KERNEL_" + name]) == getattr(_lib, "KERNEL_" + name)
+
+
+def test_class_info_layout_matches_header():
+    text = open(os.path.join(ROOT, "include", "ghost_cwt.h")).read()
+    body = re.search(r"typedef struct gcwt_class_info \{(.*?)\} gcwt_class_info;", text, flags=re.S).group(1)
+    body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
+    fields = re.findall(r"(int32_t|int64_t)\s+(\w+);", body)
+    ctypes_of = {"int32_t": C.c_int32, "int64_t": C.c_int64}
+    assert [(n, ctypes_of[t]) for t, n in fields] == list(_lib.ClassInfo._fields_)
+    assert C.sizeof(_lib.ClassInfo) == 40
+
+
+def test_plan_classes_null_arguments():
+    lib = _lib.load()
+    n = C.c_int32(7)
+    assert lib.gcwt_plan_classes(None, C.byref(n), None, None) == -1
+    assert b"NULL" in lib.gcwt_last_error()
+    assert n.value == 7
+    assert lib.gcwt_plan_classes(None, None, None, None) == -1
 
 
 def test_argument_errors_without_device():
